@@ -1,6 +1,7 @@
 """Headline benchmark: 100-step DDIM sampling of 64x64 images (BASELINE.json configs[1]).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--scaling strong|weak]
+                    [--dump-outputs DIR]
 
 One "step" = one complete DDIM-100 sampling pass over the job's batch of synthetic images (InfoDiff a_dim=256, T=100,
 random-init weights, xT and a ~ N(0,1)).  Sampling is per-sample independent, so N GPUs run N batch shards with no
@@ -22,6 +23,10 @@ under "weak_scaling".  --scaling weak makes that the headline instead.
  dp_check     : N > 1 only: N-rank averaged gradients vs rank 0's single-process gradients on the concatenated batch,
                 and sharded sampling vs single-GPU sampling (correctness evidence for the scaling runs)
 --impl reference times the CPU path alone and prints the same line with "impl": "reference".
+--dump-outputs DIR writes the images the last timed step returned as DIR/samples.npy (float32), so that two builds
+can be compared output for output.  Compare only runs with the same arguments: the weights are seeded, xT and a are
+drawn per rank (seed 1000 + rank, so --gpus, --scaling and --batch change them), and the DDIM noise (eta 0.01) comes
+from torch's CUDA generator, seeded once before the warm-up (so --warmup and --steps change it).
 """
 from __future__ import annotations
 
@@ -37,6 +42,7 @@ from pathlib import Path
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True      # the benchmark leaves the tree as it found it (it may be read-only)
 
 import torch  # noqa: E402
 
@@ -66,7 +72,30 @@ def parse():
     ap.add_argument("--no-fuse-adagn", action="store_true", help="stand-alone AdaGN kernels everywhere (A/B comparison)")
     ap.add_argument("--no-train", action="store_true", help="skip the secondary training-throughput measurement")
     ap.add_argument("--train-batch", type=int, default=32)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the samples of the last timed step to DIR/samples.npy; the inputs "
+                    "and noise are the same only for runs with the same --gpus, --scaling, --batch, --warmup and --steps")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours (the reference leg times a bounded sample, not whole sampling passes)")
+    return a
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_samples(out_dir: str, x: torch.Tensor) -> None:
+    """x -> out_dir/samples.npy in float32.  Beyond DUMP_BYTES only a fixed, seeded choice of images is kept (the same
+    images for the same batch size), in batch order."""
+    import numpy as np
+    x = x.detach().float().cpu()
+    keep = DUMP_BYTES // (x[0].numel() * 4)
+    if x.shape[0] > keep:
+        rows = torch.randperm(x.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        x = x[rows]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "samples.npy"), x.numpy())
 
 
 def ncu_traffic(kind: str):
@@ -603,9 +632,9 @@ def run_ours(a):
             if world > 1:
                 if even:
                     dist.all_gather_into_tensor(gathered, x)
-                else:
-                    from infodiffusion_b200.distributed import gather_batch
-                    gather_batch(x, global_batch)
+                    return gathered
+                from infodiffusion_b200.distributed import gather_batch
+                return gather_batch(x, global_batch)
             return x
 
         def job_e2e():
@@ -619,7 +648,7 @@ def run_ours(a):
             l0 = _lib.launches()
             e0.record()
             for _ in range(n):
-                job()
+                out = job()
             e1.record()
             barrier()
             ms = e0.elapsed_time(e1)
@@ -627,15 +656,15 @@ def run_ours(a):
                 t = torch.tensor([ms], device=dev)
                 dist.all_reduce(t, op=dist.ReduceOp.MAX)
                 ms = float(t.item())
-            return ms, _lib.launches() - l0
+            return ms, _lib.launches() - l0, out
 
         for _ in range(warmup):
             job_device()
-        ms, launches = timed(job_device, k)
+        ms, launches, out = timed(job_device, k)
         job_e2e()
-        ms_e2e, _ = timed(job_e2e, k)
+        ms_e2e, _, _ = timed(job_e2e, k)
         return dict(ms=ms, ms_e2e=ms_e2e, launches=launches, B=B, h2d=xT_h.numel() * 4 + a_h.numel() * 4,
-                    d2h=out_h.numel() * 4)
+                    d2h=out_h.numel() * 4, out=out)
 
     strong = a.scaling == "strong"
     global_batch = a.batch if strong else a.batch * world
@@ -644,6 +673,8 @@ def run_ours(a):
         clocks.start()
     m = measure(global_batch, a.steps, max(a.warmup, 3))
     clk = clocks.stop() if rank == 0 else None
+    if a.dump_outputs and rank == 0:
+        dump_samples(a.dump_outputs, m["out"])
     B = m["B"]
     value = global_batch * a.steps / (m["ms"] / 1000.0)
     e2e = global_batch * a.steps / (m["ms_e2e"] / 1000.0)

@@ -24,10 +24,18 @@ DST = Path(__file__).resolve().parent / "_ref"
 FILES = ("modules.py", "models.py", "sampling.py", "utils.py")
 
 
+def _present(d: Path) -> bool:
+    """True when `d` holds the four reference files.  A directory this user may not read counts as absent."""
+    try:
+        return all((d / f).exists() for f in FILES)
+    except OSError:
+        return False
+
+
 def build(verbose: bool = True) -> bool:
     """Returns True when oracle/_ref holds the four reference files (freshly copied or already there)."""
-    if not all((REF / f).exists() for f in FILES):
-        ok = all((DST / f).exists() for f in FILES)
+    if not _present(REF):
+        ok = _present(DST)
         if verbose:
             print(f"[build_ref] {REF} not present; oracle/_ref {'already populated' if ok else 'unavailable'}")
         return ok
