@@ -39,20 +39,15 @@ typedef enum {
 
 int idf_version(void);
 const char* idf_last_error(void);
-/* Checks that the current device is sm_100 and raises dynamic-smem limits. */
+/* Checks that the current device is sm_100, records its SM count and resolves the driver's tensor-map encoder. */
 int idf_init(void);
-/* Implementation switches kept for A/B measurement and tests:
- *   "attn_impl"     = 1 (thread-gathered operands) | 2 (TMA-fed, default)
+/* Switches for tests, measurement and launch behaviour (unknown keys or values: IDF_ERR_ARG):
  *   "conv_force_mt" = 0 (auto) | 1 | 2 | 4   128-row tiles per CTA work unit of the conv kernel
  *   "conv_debug_skip_epilogue" = 0 | 1       plans created while set drain no output (main-loop ceiling)
  *   "pdl" = 0 | 1 (default)                   launch the conv / AdaGN kernels with programmatic dependent launch
  *   "conv_pair" = 0 | 1 (default)             conv plans with block_n >= 64 run as CTA pairs (tcgen05 cta_group::2)
- *   "stats_item" = 0 | 1 (default)            GroupNorm partials per (work item, lane quarter) where an image has at
- *                                             least as many rows as an item (else, or 0: per 32-row window)
  *   "xf_debug" = 0 | 1 | 2 | 5                measurement only: fused-AdaGN transform warps do nothing / skip the SiLU /
- *                                             5: no MMAs are issued (what the transform costs alone)
- *   "adagn_ring" = 1..8 (default 2)          shared-memory stages per CTA of the streaming AdaGN kernel
- *   "adagn_ctas" >= 1 (default 400)          CTAs the streaming AdaGN kernel aims for (slices per image = ceil(v / batch)) */
+ *                                             5: no MMAs are issued (what the transform costs alone) */
 int idf_set_option(const char* key, int32_t value);
 
 /* ------------------------------------------------------------------------------------------

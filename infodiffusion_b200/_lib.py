@@ -183,11 +183,6 @@ def load(build_if_missing: bool = True):
         fn.restype = res
         fn.argtypes = args
     _lib = lib
-    # tuning / measurement switches without code changes: IDF_OPTS="adagn_impl=1,pdl=1" -> idf_set_option per pair
-    for kv in filter(None, os.environ.get("IDF_OPTS", "").split(",")):
-        k, v = kv.split("=")
-        if lib.idf_set_option(k.strip().encode(), int(v)) != 0:
-            raise IdfError(f"IDF_OPTS: bad option {kv!r}")
     return lib
 
 

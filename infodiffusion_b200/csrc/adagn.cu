@@ -16,22 +16,16 @@
 // torch.cat([h, skip]) followed by GroupNorm behaves (models.py:321 -> modules.py:265).
 #include <cooperative_groups.h>
 
-#include <algorithm>
-
 #include "kernels.cuh"
 
 namespace cg = cooperative_groups;
 
 namespace idf {
 
-// tuning knobs (idf_set_option "adagn_ring" / "adagn_ctas").  Measured on B200 (tools/adagn_microbench.py): two
+// ring stages per CTA and CTAs per launch of the streaming kernel.  Measured on B200 (DESIGN.md section 4.1): two
 // stages (five CTAs per SM) beat three or five -- the sweep is bound by resident warps, not by bytes in flight.
-int g_adagn_ring = 2;
-int g_adagn_ctas = 400;
-int g_adagn_ctas2 = 1184;    // streaming variant 2: CTAs aimed for (8 per SM)
-int g_adagn_impl = 1;      // 1 = shared-memory ring kernel (default: 4.6 TB/s on 64ch@64^2), 2 = direct-load kernel (4.1-4.25:
-                           // its per-CTA coefficient prologue is not overlapped with streaming)
-extern int g_pdl;
+constexpr int kAdaRing = 2;
+constexpr int kAdaCtas = 400;
 
 constexpr int kAdaThreads = 256;
 constexpr int kMaxC = 256;
@@ -64,7 +58,6 @@ struct AdaGNParams {
   long long bwin0, bwin1;      // records before the B part of stats0 / stats1
   int block_rows;              // rows per ring stage of the streaming variant
   int ring;                    // ring stages in use
-  int stream_threads;          // streaming variant 2: threads that stream (multiple of C/8)
   unsigned drop_thr16;         // dropout: drop iff 16 random bits < thr16 (0 = off)
   float drop_scale;            // 1 / (1 - p)
   const unsigned long long* drop_seed;
@@ -514,136 +507,14 @@ __global__ void __launch_bounds__(kAdaThreads) adagn_apply_kernel(const AdaGNPar
   }
 }
 
-// ---------------------------------------------------------------------------------------------------
-// Streaming variant 2 (idf_set_option "adagn_impl" = 2; measured slower than the ring, kept for A/B): no ring.  A CTA owns the image rows [y0, y1) of image n and walks the
-// INTERIOR pixels only -- index i over (y, x, 16-byte channel granule) maps to the pad-flat address
-// (y*Wp)*VPR + i % (W*VPR), so there is no pad-row test, no division per element and the pad rows are never
-// touched.  Each thread keeps one channel granule (blockDim % VPR == 0), i.e. its 8 (A, B) pairs live in registers;
-// per 16 bytes: 1 LDG.128 (L1 no-allocate), 8 unpack, 8 FFMA, 8 MUFU.TANH, 8 FFMA, 4 pack, 1 STG.128 -- half the
-// instructions of the ring variant (ncu: that one issued ~100 instructions per 16 bytes at 54 % issue utilisation).
-// Four granules per thread are in flight; bytes in flight per SM = resident threads x 64 B.
-// ---------------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint4 ldg_stream(const void* p) {
-  uint4 v;
-  asm volatile("ld.global.nc.L1::no_allocate.v4.b32 {%0, %1, %2, %3}, [%4];"
-               : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p));
-  return v;
-}
-
-template <bool DROPOUT>
-__global__ void __launch_bounds__(kAdaThreads) adagn_stream_kernel(const AdaGNParams p) {
-  __shared__ CoefShared<kAdaThreads> sh;
-  const int n = blockIdx.y;
-  const int t = threadIdx.x;
-  const int C = p.C;
-  griddep_launch();
-  griddep_wait();                 // the sources, their statistics and the modulation rows come from earlier kernels
-  fold_coefficients<kAdaThreads, kMaxC>(p, n, sh, blockIdx.x == 0);
-
-  const int VPR = C >> 3;                       // 16-byte granules per pixel
-  const int NT = p.stream_threads;              // multiple of VPR (<= blockDim): the threads that stream
-  if (t >= NT) return;
-  const int vl = t % VPR;                       // this thread's channel granule, fixed for the whole kernel
-  const bool do_silu = p.apply_silu != 0;
-  const float cs = do_silu ? 0.5f : 1.0f;       // SiLU(v) = h + h*tanh(h) with h = v/2: the 1/2 is folded into (A, B)
-  float A[8], B[8];
-#pragma unroll
-  for (int j = 0; j < 8; ++j) { const float2 ab = sh.ab[vl * 8 + j]; A[j] = ab.x * cs; B[j] = ab.y * cs; }
-  const int v0 = p.c0 >> 3;
-  const bool from0 = vl < v0;
-  // source / destination columns of this thread; rows advance by whole pixels
-  const bf16* src = from0 ? p.src0 + vl * 8 : p.src1 + (vl - v0) * 8;
-  const int spitch = from0 ? p.c0 : p.c1;       // elements per pixel in the source
-  const long long img_row0 = static_cast<long long>(n) * p.rows_per_img;
-  const int tp = t / VPR;                       // this thread's pixel slot; PPI pixels per pass
-  const int PPI = NT / VPR;
-  const float inv_w = 1.0f / static_cast<float>(p.W);
-  const int y0 = blockIdx.x * p.slice_rows, y1 = min(p.H, y0 + p.slice_rows);     // slice_rows = IMAGE rows here
-  const int total = (y1 - y0) * p.W;            // interior pixels of the slice
-  const int row_y0 = static_cast<int>(img_row0) + y0 * p.Wp;         // pad-flat rows fit 22 bits (checked at launch)
-  const unsigned long long drop_seed = (DROPOUT && p.drop_seed != nullptr) ? *p.drop_seed : 0ull;
-
-  auto locate = [&](int q) -> int {              // interior pixel index in the slice -> pad-flat pixel row
-    const int yy = __float2int_rd((static_cast<float>(q) + 0.5f) * inv_w);      // exact: q < 2^23
-    return row_y0 + yy + q;                      // = row_y0 + yy*Wp + (q - yy*W) with Wp = W + 1
-  };
-  auto xform = [&](const uint4& u, int pix) -> uint4 {
-    const float2 a0 = unpack_bf16x2(u.x), a1 = unpack_bf16x2(u.y), a2 = unpack_bf16x2(u.z), a3 = unpack_bf16x2(u.w);
-    float f[8] = {a0.x, a0.y, a1.x, a1.y, a2.x, a2.y, a3.x, a3.y};
-    if (do_silu) {
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        const float h = fmaf(f[j], A[j], B[j]);
-        float th;
-        asm("tanh.approx.f32 %0, %1;" : "=f"(th) : "f"(h));
-        f[j] = fmaf(h, th, h);
-      }
-    } else {
-#pragma unroll
-      for (int j = 0; j < 8; ++j) f[j] = fmaf(f[j], A[j], B[j]);
-    }
-    if (DROPOUT) {
-      const uint32_t keep = dropout_keep8(drop_seed, p.drop_layer, static_cast<uint64_t>(pix) * VPR + vl, p.drop_thr16);
-#pragma unroll
-      for (int j = 0; j < 8; ++j) f[j] = ((keep >> j) & 1u) ? f[j] * p.drop_scale : 0.f;
-    }
-    uint4 o;
-    o.x = pack_bf16x2(f[0], f[1]); o.y = pack_bf16x2(f[2], f[3]);
-    o.z = pack_bf16x2(f[4], f[5]); o.w = pack_bf16x2(f[6], f[7]);
-    return o;
-  };
-  bf16* const out = p.out + vl * 8;
-  int q = tp;
-  for (; q + 3 * PPI < total; q += 4 * PPI) {
-    int pix[4];
-    uint4 u[4];
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      pix[k] = locate(q + k * PPI);
-      u[k] = ldg_stream(src + static_cast<uint32_t>(pix[k] * spitch));          // element offsets fit 31 bits
-    }
-#pragma unroll
-    for (int k = 0; k < 4; ++k) *reinterpret_cast<uint4*>(out + static_cast<uint32_t>(pix[k] * C)) = xform(u[k], pix[k]);
-  }
-  for (; q < total; q += PPI) {
-    const int pix = locate(q);
-    *reinterpret_cast<uint4*>(out + static_cast<uint32_t>(pix * C)) = xform(ldg_stream(src + static_cast<uint32_t>(pix * spitch)), pix);
-  }
-}
-
-static cudaError_t fill_params(const idf_adagn_args& a, AdaGNParams& p);
-
-cudaError_t launch_adagn_coef(const idf_adagn_args& a, float* coef_out, cudaStream_t stream) {
-  AdaGNParams p;
-  cudaError_t e = fill_params(a, p);
-  if (e != cudaSuccess) return e;
-  if (p.stats0 == nullptr || (p.c1 != 0 && p.stats1 == nullptr) || a.dropout_p > 0.f) return cudaErrorInvalidValue;
-  p.save_coef = nullptr;
-  if (!g_pdl) {
-    if (p.C <= kMaxC) adagn_coef_kernel<kMaxC><<<a.batch, kCoefThreads, 0, stream>>>(p, reinterpret_cast<float2*>(coef_out));
-    else              adagn_coef_kernel<kMaxCWide><<<a.batch, kCoefThreads, 0, stream>>>(p, reinterpret_cast<float2*>(coef_out));
-    return cudaGetLastError();
-  }
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(a.batch, 1, 1);
-  cfg.blockDim = dim3(kCoefThreads, 1, 1);
-  cfg.dynamicSmemBytes = 0;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  if (p.C <= kMaxC) return cudaLaunchKernelEx(&cfg, adagn_coef_kernel<kMaxC>, p, reinterpret_cast<float2*>(coef_out));
-  return cudaLaunchKernelEx(&cfg, adagn_coef_kernel<kMaxCWide>, p, reinterpret_cast<float2*>(coef_out));
-}
-
-static cudaError_t fill_params(const idf_adagn_args& a, AdaGNParams& p) {
+// c1: channels of the second source.  The coefficient kernel counts them whenever their statistics are given (the
+// consumer conv reads the second source itself); the apply kernels only when there is a second source to read.
+static cudaError_t fill_params(const idf_adagn_args& a, int c1, AdaGNParams& p) {
   p.src0 = static_cast<const bf16*>(a.src0);
   p.src1 = static_cast<const bf16*>(a.src1);
   p.out = static_cast<bf16*>(a.out);
   p.c0 = a.c0;
-  p.c1 = (a.src1 || a.stats1) ? a.c1 : 0;
+  p.c1 = c1;
   p.C = p.c0 + p.c1;
   p.H = a.H; p.W = a.W; p.Hp = a.H + 1; p.Wp = a.W + 1;
   p.rows_per_img = p.Hp * p.Wp;
@@ -672,111 +543,50 @@ static cudaError_t fill_params(const idf_adagn_args& a, AdaGNParams& p) {
   return cudaSuccess;
 }
 
+cudaError_t launch_adagn_coef(const idf_adagn_args& a, float* coef_out, cudaStream_t stream) {
+  AdaGNParams p;
+  cudaError_t e = fill_params(a, (a.src1 || a.stats1) ? a.c1 : 0, p);
+  if (e != cudaSuccess) return e;
+  if (p.stats0 == nullptr || (p.c1 != 0 && p.stats1 == nullptr) || a.dropout_p > 0.f) return cudaErrorInvalidValue;
+  p.save_coef = nullptr;
+  return launch_kernel(p.C <= kMaxC ? adagn_coef_kernel<kMaxC> : adagn_coef_kernel<kMaxCWide>, dim3(a.batch),
+                       dim3(kCoefThreads), 0, stream, g_pdl != 0, 0, p, reinterpret_cast<float2*>(coef_out));
+}
+
 cudaError_t launch_adagn(const idf_adagn_args& a, cudaStream_t stream) {
   AdaGNParams p;
-  p.src0 = static_cast<const bf16*>(a.src0);
-  p.src1 = static_cast<const bf16*>(a.src1);
-  p.out = static_cast<bf16*>(a.out);
-  p.c0 = a.c0;
-  p.c1 = a.src1 ? a.c1 : 0;
-  p.C = p.c0 + p.c1;
-  p.H = a.H; p.W = a.W; p.Hp = a.H + 1; p.Wp = a.W + 1;
-  p.rows_per_img = p.Hp * p.Wp;
-  p.gamma = a.gamma; p.beta = a.beta; p.eps = a.eps;
-  p.mod_t = a.mod_t; p.mod_t_step_stride = a.mod_t_step_stride; p.mod_t_batch_stride = a.mod_t_batch_stride;
-  p.mod_z = a.mod_z; p.mod_z_step_stride = a.mod_z_step_stride; p.mod_z_batch_stride = a.mod_z_batch_stride;
-  p.step_ptr = a.step_ptr;
-  p.apply_silu = a.apply_silu;
-  if (p.C > kMaxCWide || p.C % 32 != 0 || p.c0 % 8 != 0 || p.c1 % 8 != 0 || a.batch <= 0) return cudaErrorInvalidValue;
-  p.stats0 = a.stats0;
-  p.stats1 = a.stats1;
-  p.slice_rows = 0;
-  p.drop_thr16 = 0; p.drop_scale = 1.f; p.drop_seed = reinterpret_cast<const unsigned long long*>(a.dropout_seed);
-  p.drop_layer = a.dropout_layer;
-  p.save_coef = a.save_coef;
+  cudaError_t e = fill_params(a, a.src1 ? a.c1 : 0, p);
+  if (e != cudaSuccess) return e;
   if (a.dropout_p > 0.f) {
     if (a.stats0 == nullptr) return cudaErrorInvalidValue;     // dropout lives in the streaming variant only
     p.drop_thr16 = static_cast<unsigned>(a.dropout_p * 65536.f + 0.5f);
     p.drop_scale = 65536.f / (65536.f - static_cast<float>(p.drop_thr16));
-  }
-  p.stats_b_windows = (static_cast<long long>(a.batch) * p.rows_per_img + kBM - 1) / kBM * 4;
-  p.unit0 = a.stats_unit0 > 0 ? a.stats_unit0 : 32;
-  p.unit1 = a.stats_unit1 > 0 ? a.stats_unit1 : 32;
-  p.planes0 = a.stats_planes0 > 0 ? a.stats_planes0 : 1;
-  p.planes1 = a.stats_planes1 > 0 ? a.stats_planes1 : 1;
-  p.rsrc0 = a.stats_rows0 > 0 ? a.stats_rows0 : p.rows_per_img;
-  p.rsrc1 = a.stats_rows1 > 0 ? a.stats_rows1 : p.rows_per_img;
-  p.bwin0 = (static_cast<long long>(a.batch) * p.rsrc0 + kBM - 1) / kBM * 4;
-  p.bwin1 = (static_cast<long long>(a.batch) * p.rsrc1 + kBM - 1) / kBM * 4;
-  if ((p.unit0 > 32 && p.unit0 > p.rsrc0) || (p.unit1 > 32 && p.unit1 > p.rsrc1)) return cudaErrorInvalidValue;   // a unit spans <= 2 images
-  if (g_adagn_impl == 2 && p.C <= kMaxC && p.stats0 != nullptr && (p.c1 == 0 || p.stats1 != nullptr)) {
-    // streaming variant 2: a CTA owns whole image rows; enough CTAs for >= 4 per SM, each with >= 16 KB to stream
-    const int VPR = p.C / 8;
-    if (static_cast<long long>(a.batch) * p.rows_per_img * p.C >= (1ll << 31)) return cudaErrorInvalidValue;   // 32-bit element offsets
-    p.stream_threads = kAdaThreads / VPR * VPR;
-    const long long row_bytes = static_cast<long long>(p.W) * p.C * 2;
-    int slices = (g_adagn_ctas2 + a.batch - 1) / a.batch;
-    const int max_slices = static_cast<int>(std::max<long long>(1, static_cast<long long>(p.H) * row_bytes / 16384));
-    if (slices > max_slices) slices = max_slices;
-    if (slices > p.H) slices = p.H;
-    if (slices < 1) slices = 1;
-    p.slice_rows = (p.H + slices - 1) / slices;
-    slices = (p.H + p.slice_rows - 1) / p.slice_rows;
-    p.block_rows = 0; p.ring = 0;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(slices, a.batch, 1);
-    cfg.blockDim = dim3(kAdaThreads, 1, 1);
-    cfg.dynamicSmemBytes = 0;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = g_pdl ? 1 : 0;
-    if (p.drop_thr16 != 0) return cudaLaunchKernelEx(&cfg, adagn_stream_kernel<true>, p);
-    return cudaLaunchKernelEx(&cfg, adagn_stream_kernel<false>, p);
   }
   if (p.stats0 != nullptr && (p.c1 == 0 || p.stats1 != nullptr)) {
     // streaming variant: bytes in flight come from the per-CTA ring, not from occupancy, so a few hundred
     // CTAs suffice; large slices amortise the per-CTA coefficient prologue
     const long long bytes_s = static_cast<long long>(p.rows_per_img) * p.C * 2;
     const int max_slices = static_cast<int>((bytes_s + 32767) / 32768);
-    int slices = (g_adagn_ctas + a.batch - 1) / a.batch;
+    int slices = (kAdaCtas + a.batch - 1) / a.batch;
     if (slices > max_slices) slices = max_slices;
     if (slices < 1) slices = 1;
     p.slice_rows = (p.rows_per_img + slices - 1) / slices;
     slices = (p.rows_per_img + p.slice_rows - 1) / p.slice_rows;
     p.block_rows = 4 * (kAdaThreads / (p.C / 8));            // four rows per thread and stage (<= 16 KB)
-    p.ring = g_adagn_ring;
+    p.ring = kAdaRing;
     const size_t ring_bytes = static_cast<size_t>(p.ring) * p.block_rows * p.C * 2;
     static bool attr_set = false;
     if (!attr_set) {
-      cudaError_t e = cudaFuncSetAttribute(adagn_apply_kernel<kMaxC>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                           kRingMax * kRingStageBytes);
+      e = cudaFuncSetAttribute(adagn_apply_kernel<kMaxC>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                               kRingMax * kRingStageBytes);
       if (e == cudaSuccess)
         e = cudaFuncSetAttribute(adagn_apply_kernel<kMaxCWide>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  kRingMax * kRingStageBytes);
       if (e != cudaSuccess) return e;
       attr_set = true;
     }
-    const bool wide = p.C > kMaxC;
-    if (!g_pdl) {
-      if (wide) adagn_apply_kernel<kMaxCWide><<<dim3(slices, a.batch, 1), kAdaThreads, ring_bytes, stream>>>(p);
-      else      adagn_apply_kernel<kMaxC><<<dim3(slices, a.batch, 1), kAdaThreads, ring_bytes, stream>>>(p);
-      return cudaGetLastError();
-    }
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(slices, a.batch, 1);
-    cfg.blockDim = dim3(kAdaThreads, 1, 1);
-    cfg.dynamicSmemBytes = ring_bytes;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    if (wide) return cudaLaunchKernelEx(&cfg, adagn_apply_kernel<kMaxCWide>, p);
-    return cudaLaunchKernelEx(&cfg, adagn_apply_kernel<kMaxC>, p);
+    return launch_kernel(p.C > kMaxC ? adagn_apply_kernel<kMaxCWide> : adagn_apply_kernel<kMaxC>,
+                         dim3(slices, a.batch, 1), dim3(kAdaThreads), ring_bytes, stream, g_pdl != 0, 0, p);
   }
 
   if (p.C > kMaxC) return cudaErrorInvalidValue;       // the two-sweep fallback (no producer statistics) serves <= 256 channels
@@ -789,24 +599,11 @@ cudaError_t launch_adagn(const idf_adagn_args& a, cudaStream_t stream) {
   if (smem > 200 * 1024) return cudaErrorInvalidValue;
   static size_t attr_smem = 0;
   if (smem > attr_smem) {
-    cudaError_t e = cudaFuncSetAttribute(adagn_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
+    e = cudaFuncSetAttribute(adagn_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
     if (e != cudaSuccess) return e;
     attr_smem = smem;
   }
-
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(CL, a.batch, 1);
-  cfg.blockDim = dim3(kAdaThreads, 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CL;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, adagn_kernel, p);
+  return launch_kernel(adagn_kernel, dim3(CL, a.batch, 1), dim3(kAdaThreads), smem, stream, false, CL, p);
 }
 
 }  // namespace idf

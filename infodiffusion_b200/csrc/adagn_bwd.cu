@@ -13,8 +13,6 @@
 
 namespace idf {
 
-extern int g_pdl;
-
 constexpr int kBT = 256;       // threads
 constexpr int kBMaxC = 256;
 constexpr int kBSlices = 16;   // max row slices per sample (the launcher uses fewer for large batches / small maps)
@@ -357,26 +355,9 @@ cudaError_t launch_adagn_bwd(const idf_adagn_bwd_args& b, int num_sms, cudaStrea
   p.slice_rows = (p.R + ns - 1) / ns;
   p.n_slices = (p.R + p.slice_rows - 1) / p.slice_rows;
   const dim3 grid(p.n_slices, a.batch, 1);
-  if (!g_pdl) {
-    adagn_bwd_stats_kernel<<<grid, kBT, 0, stream>>>(p);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return e;
-    adagn_bwd_apply_kernel<<<grid, kBT, 0, stream>>>(p);
-    return cudaGetLastError();
-  }
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid;
-  cfg.blockDim = dim3(kBT, 1, 1);
-  cfg.dynamicSmemBytes = 0;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, adagn_bwd_stats_kernel, p);
+  cudaError_t e = launch_kernel(adagn_bwd_stats_kernel, grid, dim3(kBT), 0, stream, g_pdl != 0, 0, p);
   if (e != cudaSuccess) return e;
-  return cudaLaunchKernelEx(&cfg, adagn_bwd_apply_kernel, p);
+  return launch_kernel(adagn_bwd_apply_kernel, grid, dim3(kBT), 0, stream, g_pdl != 0, 0, p);
 }
 
 }  // namespace idf

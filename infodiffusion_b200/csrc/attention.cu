@@ -4,9 +4,10 @@
 //   S = Q K^T   : tcgen05.mma  M=128, N=S,   K=128   -> TMEM columns [0, S)       (fp32)
 //   P = softmax : one thread per query row, straight out of TMEM (exp2, fp32), bf16 P -> shared memory
 //   O = P V     : tcgen05.mma  M=128, N=128, K=S     -> TMEM columns [256, 384)   (fp32)
-// Q, K are gathered from the pad-flat [rows, 3d] qkv matrix into the K-major 128B-swizzled layout by
-// the CTA's threads (tokens skip the pad rows, so this is a gather, not a TMA box); V is transposed
-// on the way in (V^T rows = d, contiguous along keys) so that both GEMMs use K-major operands.
+// Tokens of one image row are W consecutive rows of the pad-flat [rows, 3d] qkv matrix, so Q, K and V
+// arrive as [W x 64] TMA boxes (one per image row and 64-wide d-chunk) straight into the K-major
+// 128B-swizzled layout -- no gather instructions.  V is not transposed: it is the MN-major B operand
+// of O = P V (N = d contiguous).
 // Scores never leave the SM (the reference materialises [B,S,S] fp32 in HBM, modules.py:154-156).
 #include "kernels.cuh"
 
@@ -20,206 +21,8 @@ __device__ __forceinline__ uint32_t sw128_off(int r, int g) {
   return static_cast<uint32_t>((r >> 3) * 1024 + (r & 7) * 128 + ((g ^ (r & 7)) << 4));
 }
 
-template <int S>
-__global__ void __launch_bounds__(kAttnThreads, 1)
-attn_gather_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ out, int Hp, int Wp, int W, float scale_log2e) {
-  // shared-memory map (all tiles are [rows x 64 elem] SW128 blocks, 1024-aligned):
-  //   Q  : 2 d-chunks   x [128 x 128B]          = 32 KB
-  //   K  : 2 d-chunks   x [S   x 128B]          = S/4 KB   (re-used for P: S/64 key-chunks x [128 x 128B])
-  //   VT : S/64 chunks  x [128 x 128B]          = S/4 KB
-  constexpr int KCH = S / 64;                      // key chunks
-  constexpr uint32_t Q_BYTES = 2 * 128 * 128;
-  constexpr uint32_t K_BYTES = (2 * S * 128 > KCH * 128 * 128) ? 2 * S * 128 : KCH * 128 * 128;
-  constexpr uint32_t VT_BYTES = KCH * 128 * 128;
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* smQ = smem;
-  uint8_t* smK = smQ + Q_BYTES;                    // later: P
-  uint8_t* smVT = smK + K_BYTES;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smVT + VT_BYTES);   // [0]: S ready, [1]: O ready
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2);
-
-  const int t = threadIdx.x;
-  const int warp = t >> 5, lane = t & 31;
-  const int n = blockIdx.y;
-  const int q0 = blockIdx.x * 128;                 // first query token of this tile
-  const long long img_row0 = static_cast<long long>(n) * Hp * Wp;
-  const int ld = 3 * kD;
-
-  if (t == 0) {
-    mbar_init(bars + 0, 1);
-    mbar_init(bars + 1, 1);
-    fence_mbar_init();
-  }
-  if (warp == 0) {
-    tmem_alloc(tmem_slot, 512);
-    tmem_relinquish();
-  }
-
-  auto tok_row = [&](int tok) -> long long { return img_row0 + (tok / W) * Wp + (tok % W); };
-
-  // ---- gather Q (rows >= S are zero-filled) and K into swizzled K-major tiles
-  for (int i = t; i < 128 * 16; i += kAttnThreads) {      // 16 granules of 16B per 256-byte row
-    const int r = i >> 4, g = i & 15;
-    const int tok = q0 + r;
-    uint4 v = make_uint4(0, 0, 0, 0);
-    if (tok < S) v = __ldg(reinterpret_cast<const uint4*>(qkv + tok_row(tok) * ld + g * 8));
-    *reinterpret_cast<uint4*>(smQ + (g >> 3) * (128 * 128) + sw128_off(r, g & 7)) = v;
-  }
-  for (int i = t; i < S * 16; i += kAttnThreads) {
-    const int r = i >> 4, g = i & 15;
-    const uint4 v = __ldg(reinterpret_cast<const uint4*>(qkv + tok_row(r) * ld + kD + g * 8));
-    *reinterpret_cast<uint4*>(smK + (g >> 3) * (S * 128) + sw128_off(r, g & 7)) = v;
-  }
-  // ---- V^T: lane -> key (so the 2-byte transposed stores of a warp are contiguous along keys)
-  for (int i = t; i < S * 16; i += kAttnThreads) {
-    const int key = (i & 31) + ((i >> 9) << 5);            // 32 keys per warp-step, 16 granules each
-    const int g = (i >> 5) & 15;
-    const uint4 v = __ldg(reinterpret_cast<const uint4*>(qkv + tok_row(key) * ld + 2 * kD + g * 8));
-    const uint32_t w[4] = {v.x, v.y, v.z, v.w};
-    uint8_t* chunk = smVT + (key >> 6) * (128 * 128);
-    const int kk = key & 63;
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      const int dd = g * 8 + j;                            // row of V^T
-      const uint16_t h = static_cast<uint16_t>((j & 1) ? (w[j >> 1] >> 16) : (w[j >> 1] & 0xffffu));
-      *reinterpret_cast<uint16_t*>(chunk + sw128_off(dd, kk >> 3) + (kk & 7) * 2) = h;
-    }
-  }
-  fence_async_smem();
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  const uint32_t tmem_S = tmem_base;
-  const uint32_t tmem_O = tmem_base + 256;
-
-  // ---- S = Q K^T
-  if (t == 0) {
-    constexpr uint32_t idesc = umma_idesc_f16(128, S, kFmtBF16);
-#pragma unroll
-    for (int c = 0; c < 2; ++c) {
-      const uint64_t da = umma_desc_k_sw128(smem_u32(smQ + c * (128 * 128)));
-      const uint64_t db = umma_desc_k_sw128(smem_u32(smK + c * (S * 128)));
-#pragma unroll
-      for (int k = 0; k < 4; ++k) umma_f16(tmem_S, da + 2 * k, db + 2 * k, idesc, (c | k) != 0 ? 1u : 0u);
-    }
-    umma_commit(bars + 0);
-  }
-  mbar_wait(bars + 0, 0);
-  tc_fence_after();
-
-  // ---- softmax: thread owns query row (warp*32 + lane) == TMEM lane
-  const int row = warp * 32 + lane;
-  const uint32_t lane_addr = static_cast<uint32_t>(warp * 32) << 16;
-  float mx = -INFINITY;
-#pragma unroll 1
-  for (int c = 0; c < S / 32; ++c) {
-    uint32_t v[32];
-    tmem_ld_32x32(tmem_S + lane_addr + c * 32, v);
-    tmem_ld_wait();
-#pragma unroll
-    for (int j = 0; j < 32; ++j) mx = fmaxf(mx, __uint_as_float(v[j]));
-  }
-  float sum = 0.f;
-  const float mxs = mx * scale_log2e;
-#pragma unroll 1
-  for (int c = 0; c < S / 32; ++c) {
-    uint32_t v[32];
-    tmem_ld_32x32(tmem_S + lane_addr + c * 32, v);
-    tmem_ld_wait();
-    uint8_t* chunk = smK + (c >> 1) * (128 * 128);         // P tile for keys [64*(c/2), +64)
-#pragma unroll
-    for (int g = 0; g < 4; ++g) {
-      float e[8];
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        e[j] = exp2f(fmaf(__uint_as_float(v[g * 8 + j]), scale_log2e, -mxs));
-        sum += e[j];
-      }
-      uint4 o;
-      o.x = pack_bf16x2(e[0], e[1]);
-      o.y = pack_bf16x2(e[2], e[3]);
-      o.z = pack_bf16x2(e[4], e[5]);
-      o.w = pack_bf16x2(e[6], e[7]);
-      *reinterpret_cast<uint4*>(chunk + sw128_off(row, (c & 1) * 4 + g)) = o;
-    }
-  }
-  fence_async_smem();
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-
-  // ---- O = P V
-  if (t == 0) {
-    constexpr uint32_t idesc = umma_idesc_f16(128, kD, kFmtBF16);
-#pragma unroll
-    for (int c = 0; c < KCH; ++c) {
-      const uint64_t da = umma_desc_k_sw128(smem_u32(smK + c * (128 * 128)));
-      const uint64_t db = umma_desc_k_sw128(smem_u32(smVT + c * (128 * 128)));
-#pragma unroll
-      for (int k = 0; k < 4; ++k) umma_f16(tmem_O, da + 2 * k, db + 2 * k, idesc, (c | k) != 0 ? 1u : 0u);
-    }
-    umma_commit(bars + 1);
-  }
-  mbar_wait(bars + 1, 0);
-  tc_fence_after();
-
-  const float inv = 1.0f / sum;
-  const int tok = q0 + row;
-  const bool valid = tok < S;
-  bf16* orow = out + (valid ? tok_row(tok) : 0) * kD;
-#pragma unroll 1
-  for (int c = 0; c < kD / 32; ++c) {
-    uint32_t v[32];
-    tmem_ld_32x32(tmem_O + lane_addr + c * 32, v);
-    tmem_ld_wait();
-    if (valid) {
-#pragma unroll
-      for (int g = 0; g < 4; ++g) {
-        uint4 o;
-        o.x = pack_bf16x2(__uint_as_float(v[g * 8 + 0]) * inv, __uint_as_float(v[g * 8 + 1]) * inv);
-        o.y = pack_bf16x2(__uint_as_float(v[g * 8 + 2]) * inv, __uint_as_float(v[g * 8 + 3]) * inv);
-        o.z = pack_bf16x2(__uint_as_float(v[g * 8 + 4]) * inv, __uint_as_float(v[g * 8 + 5]) * inv);
-        o.w = pack_bf16x2(__uint_as_float(v[g * 8 + 6]) * inv, __uint_as_float(v[g * 8 + 7]) * inv);
-        *reinterpret_cast<uint4*>(orow + c * 32 + g * 8) = o;
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, 512);
-  }
-}
-
-template <int S>
-static cudaError_t launch_attn_gather(const bf16* qkv, bf16* out, int batch, int H, int W, float scale,
-                                 cudaStream_t stream) {
-  constexpr int KCH = S / 64;
-  constexpr uint32_t K_BYTES = (2 * S * 128 > KCH * 128 * 128) ? 2 * S * 128 : KCH * 128 * 128;
-  constexpr uint32_t SMEM = 2 * 128 * 128 + K_BYTES + KCH * 128 * 128 + 64 + 1024;
-  static bool attr_set = false;
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(attn_gather_kernel<S>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         static_cast<int>(SMEM));
-    if (e != cudaSuccess) return e;
-    attr_set = true;
-  }
-  dim3 grid((S + 127) / 128, batch, 1);
-  attn_gather_kernel<S><<<grid, kAttnThreads, SMEM, stream>>>(qkv, out, H + 1, W + 1, W, scale * 1.4426950408889634f);
-  return cudaGetLastError();
-}
-
-
-// ---------------------------------------------------------------------------------------------------
-// v2: TMA-fed.  Tokens of one image row are W consecutive pad-flat rows, so Q, K and V arrive as
-// [W x 64] TMA boxes (one per image row and 64-wide d-chunk) straight into the swizzled K-major
-// layout -- no gather instructions.  V is NOT transposed: it is used as an MN-major B operand
-// (N = d contiguous), described by LBO = distance between the two 64-wide d-chunks and
-// SBO = 1024 B (8 keys); the K loop of O = P V advances 16 keys = 2048 B per MMA.
-// ---------------------------------------------------------------------------------------------------
+// MN-major SW128 operand descriptor of V: LBO = distance between the two 64-wide d-chunks, SBO = 1024 B
+// (8 keys); the K loop of O = P V advances 16 keys = 2048 B per MMA.
 __device__ __forceinline__ uint64_t umma_desc_mn_sw128(uint32_t smem_addr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
   uint64_t d = 0;
   d |= static_cast<uint64_t>((smem_addr >> 4) & 0x3fffu);
@@ -571,15 +374,6 @@ cudaError_t launch_attn_generic(const bf16* qkv, bf16* out, int batch, int H, in
   }
   attn_generic_kernel<<<dim3((S + kGenQ - 1) / kGenQ, batch, 1), 256, smem, stream>>>(qkv, out, H, W, d, scale);
   return cudaGetLastError();
-}
-
-cudaError_t launch_attn(const bf16* qkv, bf16* out, int batch, int H, int W, int d, float scale,
-                        cudaStream_t stream) {
-  if (d != kD) return cudaErrorInvalidValue;
-  const int S = H * W;
-  if (S == 256) return launch_attn_gather<256>(qkv, out, batch, H, W, scale, stream);
-  if (S == 64) return launch_attn_gather<64>(qkv, out, batch, H, W, scale, stream);
-  return cudaErrorInvalidValue;
 }
 
 }  // namespace idf

@@ -11,7 +11,6 @@
 
 #include "kernels.cuh"
 
-namespace idf { extern int g_adagn_ring, g_adagn_ctas, g_adagn_ctas2, g_adagn_impl, g_pdl, g_xf_debug; }
 using namespace idf;
 
 namespace {
@@ -32,10 +31,8 @@ int cuda_fail(cudaError_t e, const char* what) {
 
 PFN_cuTensorMapEncodeTiled_v12000 g_encode = nullptr;
 int g_num_sms = 0;
-int g_attn_impl = 2;
 int g_force_mt = 0;   // 0 = choose automatically
 int g_skip_epilogue = 0;
-int g_stats_item = 1;  // GroupNorm partials per work item instead of per 32-row window (idf_set_option "stats_item")
 int g_conv_pair = 1;  // conv kernels with N >= 64 run as CTA pairs (idf_set_option "conv_pair", 0 = single CTAs)
 
 int ensure_init() {
@@ -110,10 +107,6 @@ const char* idf_last_error(void) { return g_err; }
 int idf_init(void) { return ensure_init(); }
 
 int idf_set_option(const char* key, int32_t value) {
-  if (key != nullptr && std::strcmp(key, "attn_impl") == 0 && (value == 1 || value == 2)) {
-    g_attn_impl = value;
-    return IDF_OK;
-  }
   if (key != nullptr && std::strcmp(key, "conv_force_mt") == 0 && (value == 0 || value == 1 || value == 2 || value == 4)) {
     g_force_mt = value;
     return IDF_OK;
@@ -122,14 +115,9 @@ int idf_set_option(const char* key, int32_t value) {
     g_skip_epilogue = value ? 1 : 0;
     return IDF_OK;
   }
-  if (key != nullptr && std::strcmp(key, "stats_item") == 0 && (value == 0 || value == 1)) { g_stats_item = value; return IDF_OK; }
   if (key != nullptr && std::strcmp(key, "conv_pair") == 0 && (value == 0 || value == 1)) { g_conv_pair = value; return IDF_OK; }
   if (key != nullptr && std::strcmp(key, "pdl") == 0) { g_pdl = value ? 1 : 0; return IDF_OK; }
   if (key != nullptr && std::strcmp(key, "xf_debug") == 0 && value >= 0 && value <= 5) { g_xf_debug = value; return IDF_OK; }
-  if (key != nullptr && std::strcmp(key, "adagn_ring") == 0 && value >= 1 && value <= 8) { g_adagn_ring = static_cast<int>(value); return IDF_OK; }
-  if (key != nullptr && std::strcmp(key, "adagn_ctas") == 0 && value >= 1) { g_adagn_ctas = static_cast<int>(value); return IDF_OK; }
-  if (key != nullptr && std::strcmp(key, "adagn_ctas2") == 0 && value >= 1) { g_adagn_ctas2 = static_cast<int>(value); return IDF_OK; }
-  if (key != nullptr && std::strcmp(key, "adagn_impl") == 0 && (value == 1 || value == 2)) { g_adagn_impl = static_cast<int>(value); return IDF_OK; }
   return fail(IDF_ERR_ARG, "unknown option or value");
 }
 
@@ -271,7 +259,7 @@ int idf_conv_plan_create(const idf_conv_desc* d, idf_conv_plan** out_plan) {
   p.stats_ld = d->up2 != 0 ? d->cout_pad : d->out_ld;
   p.stats_b_off = static_cast<int64_t>(m_tiles) * 4 * p.stats_ld * 2;
   // item-level records when a work item spans at most two images
-  p.stats_item = (p.stats != nullptr && g_stats_item != 0 && d->block_n >= 64 &&
+  p.stats_item = (p.stats != nullptr && d->block_n >= 64 &&
                   static_cast<int64_t>(p.Hp) * p.Wp >= static_cast<int64_t>(mt) * kBM) ? 1 : 0;
   pl->stats_unit = p.stats_item ? mt * kBM : 32;
   if (p.stats != nullptr && d->out_ld != d->cout) { delete pl; return fail(IDF_ERR_ARG, "stats_out needs out_ld == cout"); }
@@ -447,15 +435,10 @@ int idf_attn_fwd(const void* qkv, void* out, int32_t batch, int32_t H, int32_t W
     if (e != cudaSuccess) return cuda_fail(e, "attention launch (tensor-core kernel: d=128 with H*W in {64,256}; otherwise d % 8 == 0, H*W <= 1024)");
     return IDF_OK;
   }
-  if (g_attn_impl == 1) {   // v1: thread-gathered operands, V transposed in shared memory
-    e = launch_attn(static_cast<const bf16*>(qkv), static_cast<bf16*>(out), batch, H, W, d, scale,
-                    reinterpret_cast<cudaStream_t>(stream));
-  } else {                  // v2: TMA boxes per image row, V as MN-major operand
-    CUtensorMap tm;
-    rc = encode_2d(&tm, qkv, static_cast<int64_t>(batch) * (H + 1) * (W + 1), 3 * d, W);
-    if (rc != IDF_OK) return rc;
-    e = launch_attn_v2(tm, static_cast<bf16*>(out), batch, H, W, d, scale, reinterpret_cast<cudaStream_t>(stream));
-  }
+  CUtensorMap tm;   // TMA boxes per image row
+  rc = encode_2d(&tm, qkv, static_cast<int64_t>(batch) * (H + 1) * (W + 1), 3 * d, W);
+  if (rc != IDF_OK) return rc;
+  e = launch_attn_v2(tm, static_cast<bf16*>(out), batch, H, W, d, scale, reinterpret_cast<cudaStream_t>(stream));
   if (e != cudaSuccess) return cuda_fail(e, "attention launch (supported: d=128, H*W in {64,256})");
   return IDF_OK;
 }

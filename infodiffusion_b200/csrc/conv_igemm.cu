@@ -905,32 +905,8 @@ static cudaError_t launch_cfg(const ConvKernelParams& p, int grid, cudaStream_t 
     if (e != cudaSuccess) return e;
     attr_smem = smem;
   }
-  if (!g_pdl && !PAIR) {
-    conv_halo_kernel<BN, MT, XF, PAIR><<<grid, conv_threads(XF), smem, stream>>>(p);
-    return cudaGetLastError();
-  }
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(grid, 1, 1);
-  cfg.blockDim = dim3(conv_threads(XF), 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
-  int na = 0;
-  if (g_pdl) {
-    attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[na].val.programmaticStreamSerializationAllowed = 1;
-    ++na;
-  }
-  if (PAIR) {
-    attr[na].id = cudaLaunchAttributeClusterDimension;
-    attr[na].val.clusterDim.x = 2;
-    attr[na].val.clusterDim.y = 1;
-    attr[na].val.clusterDim.z = 1;
-    ++na;
-  }
-  cfg.attrs = attr;
-  cfg.numAttrs = na;
-  return cudaLaunchKernelEx(&cfg, conv_halo_kernel<BN, MT, XF, PAIR>, p);
+  return launch_kernel(conv_halo_kernel<BN, MT, XF, PAIR>, dim3(grid), dim3(conv_threads(XF)), smem, stream, g_pdl != 0,
+                       PAIR ? 2 : 0, p);
 }
 
 template <bool XF, bool PAIR>

@@ -75,13 +75,48 @@ struct alignas(64) WgradKernelParams {
 cudaError_t launch_wgrad(const WgradKernelParams& p, int grid, cudaStream_t stream);
 
 static_assert(sizeof(ConvKernelParams) <= 4000, "kernel parameters are limited to 4 KB");
+
+// library-wide options (idf_set_option), defined in conv_igemm.cu
+extern int g_pdl;
+extern int g_xf_debug;
+
+// kernel<<<grid, block, smem, stream>>>(args...), with programmatic dependent launch when `pdl` is set (the kernel's
+// prologue may overlap its predecessor's tail; it orders its dependent reads with griddepcontrol.wait) and as clusters
+// of `cluster` CTAs along x when `cluster` > 0.  The arguments are converted to the kernel's parameter types, as by
+// cudaLaunchKernelEx, not deduced against them.
+template <typename... KernelParams, typename... Args>
+cudaError_t launch_kernel(void (*kernel)(KernelParams...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
+                          bool pdl, int cluster, const Args&... args) {
+  cudaLaunchAttribute attr[2];
+  unsigned na = 0;
+  if (pdl) {
+    attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[na].val.programmaticStreamSerializationAllowed = 1;
+    ++na;
+  }
+  if (cluster > 0) {
+    attr[na].id = cudaLaunchAttributeClusterDimension;
+    attr[na].val.clusterDim.x = cluster;
+    attr[na].val.clusterDim.y = 1;
+    attr[na].val.clusterDim.z = 1;
+    ++na;
+  }
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = grid;
+  cfg.blockDim = block;
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = stream;
+  cfg.attrs = attr;
+  cfg.numAttrs = na;
+  return cudaLaunchKernelEx(&cfg, kernel, args...);
+}
+
 cudaError_t launch_conv_igemm(const ConvKernelParams& p, int block_n, int mt, bool xform, bool pair, int grid, cudaStream_t stream);
 cudaError_t launch_adagn_coef(const idf_adagn_args& a, float* coef_out, cudaStream_t stream);
 uint32_t conv_config_smem(int block_n, int mt, int a_stage_bytes, bool pair, bool xf);
 cudaError_t launch_adagn(const idf_adagn_args& a, cudaStream_t stream);
 cudaError_t launch_adagn_bwd(const idf_adagn_bwd_args& b, int num_sms, cudaStream_t stream);
 int64_t adagn_bwd_ws_floats(int batch, int C);
-cudaError_t launch_attn(const bf16* qkv, bf16* out, int batch, int H, int W, int d, float scale, cudaStream_t stream);
 cudaError_t launch_attn_small(const bf16* qkv, bf16* out, int batch, int H, int W, int d, float scale, cudaStream_t stream);
 cudaError_t launch_attn_generic(const bf16* qkv, bf16* out, int batch, int H, int W, int d, float scale, cudaStream_t stream);
 cudaError_t launch_attn_v2(const CUtensorMap& tm, bf16* out, int batch, int H, int W, int d, float scale,

@@ -91,12 +91,10 @@ class VAct:
 # the AdaGN launch it replaces.  FUSE_ADAGN = True fuses every layer (bench.py --fuse-adagn all); FUSE_ADAGN_MIN_H fuses
 # the maps of at least that size when the batch is large enough to fill the machine (the default: 64x64 maps).
 FUSE_ADAGN = False
-FUSE_ADAGN_MIN_H = int(__import__("os").environ.get("IDF_FUSE_MIN_H", "64"))
+FUSE_ADAGN_MIN_H = 64
 FUSE_ADAGN_MIN_ROWS = 128 * 65 * 65      # ... and only from this many pad-flat rows (batch 128 at 64x64)
 MAX_GN_CHANNELS = 1024       # widest GroupNorm the AdaGN forward kernels take (csrc/adagn.cu kMaxCWide)
 MAX_TRAIN_GN_CHANNELS = 256  # ... and their backward kernels (csrc/adagn_bwd.cu); wgrad plans stop at 64 work units
-UPSAMPLE_FOLD = __import__("os").environ.get("IDF_UPSAMPLE_FOLD", "1") != "0"   # inference: nearest x2 folded into the following conv (see Plan.upsample)
-TRAIN_PDL = True       # programmatic dependent launch once a training plan exists (library-wide switch)
 
 
 class Workspace:
@@ -179,7 +177,7 @@ class Plan:
         self.B = batch
         self.device = device
         self.training = training
-        if training and TRAIN_PDL:
+        if training:
             # the training step is a chain of ~1000 small dependent kernels: let each conv / AdaGN kernel run its
             # prologue (barriers, TMEM, bias, weight tiles) while its predecessor drains (+2.5 % step rate, bitwise
             # neutral: tests/test_gpu_network.py::test_programmatic_dependent_launch_is_bitwise_neutral)
@@ -541,7 +539,7 @@ class Plan:
         (idf_conv_desc.up2: the GEMM runs on the input grid, four taps per output parity, pre-summed weights, the
         epilogue scatters the parities: 4/9 of the FLOPs and no upsampled tensor); training plans materialise it."""
         cout = conv.out_channels
-        if UPSAMPLE_FOLD and not self.training and cout in (64, 128) and src.C % 64 == 0:
+        if not self.training and cout in (64, 128) and src.C % 64 == 0:
             H = src.H
             out = self.ws.alloc(2 * H, cout)
             wp = self.weight(lambda: pack_conv3x3_up2(pv(conv.weight)))

@@ -28,11 +28,6 @@ def timeit(fn, n=20):
     return e0.elapsed_time(e1) / n * 1e3     # us
 
 
-import os
-for knob in ("adagn_ring", "adagn_ctas"):
-    if os.environ.get(knob.upper()):
-        _lib.check(lib.idf_set_option(knob.encode(), int(os.environ[knob.upper()])))
-        print(knob, "=", os.environ[knob.upper()])
 SHAPES = [(256, 64, 64), (256, 32, 128), (256, 16, 128), (256, 8, 128), (256, 16, 256), (256, 8, 256), (32, 64, 64), (32, 32, 128)]
 for (B, H, Cc) in SHAPES:
     rows = B * (H + 1) * (H + 1)
