@@ -230,9 +230,12 @@ int idf_attn_fwd(const void* qkv, void* out, int32_t batch, int32_t H, int32_t W
                  idf_stream_t stream);
 
 /* Backward of idf_attn_fwd (autograd of modules.py:145-164): dqkv [rows, 3*d] (dq | dk | dv, interior rows only) from the
- * saved qkv and dout = dL/dO [rows, d].  Two tcgen05 kernels per call (scores: P and dS rows -> workspace; gradients:
- * dQ = dS K, dK = dS^T Q, dV = P^T dO); ws = idf_attn_bwd_ws_bytes(batch, H, W) bytes of device memory, 1024-aligned
- * (unused for the small-map fallback H*W <= 64, H*W*d <= 8192). */
+ * saved qkv and dout = dL/dO [rows, d].  Supported shapes:
+ *   H*W in {64, 256} with d in {128, 256, 512}: two tcgen05 kernels per call (scores: P and dS rows -> workspace;
+ *     gradients: dQ = dS K, dK = dS^T Q, dV = P^T dO); ws = idf_attn_bwd_ws_bytes(batch, H, W) bytes of device memory,
+ *     1024-aligned (the same for every d);
+ *   otherwise H*W <= 64 with H*W*d <= 8192: a small-map kernel (ws unused).
+ * Other shapes return IDF_ERR_CUDA with a message naming these. */
 int idf_attn_bwd(const void* qkv, const void* dout, void* dqkv, void* ws, int32_t batch, int32_t H, int32_t W, int32_t d,
                  float scale, idf_stream_t stream);
 int64_t idf_attn_bwd_ws_bytes(int32_t batch, int32_t H, int32_t W);

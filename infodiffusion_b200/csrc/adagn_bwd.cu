@@ -14,7 +14,8 @@
 namespace idf {
 
 constexpr int kBT = 256;       // threads
-constexpr int kBMaxC = 256;
+constexpr int kBMaxC = 256;       // every InfoDiff layer
+constexpr int kBMaxCWide = 1024;  // the vanilla Diff UNet (ch_mult [1,2,4,8]): 512 channels, concatenations of 768 / 1024
 constexpr int kBSlices = 16;   // max row slices per sample (the launcher uses fewer for large batches / small maps)
 
 struct AdaGNBwdParams {
@@ -37,16 +38,23 @@ struct AdaGNBwdParams {
 };
 
 constexpr int kUn = 2;            // rows in flight per thread (more would cost occupancy: 4 CTAs/SM at <= 64 registers)
+// resident CTAs per SM the register budget is sized for: 3 at <= 256 channels (80 registers, a few bytes of spills), 2 for
+// the wide instantiation, which then needs no spills (its layers are the few 8x8 / 16x16 maps of the vanilla UNet)
+template <int kMaxC> constexpr int kBwdMinCtas = kMaxC > kBMaxC ? 2 : 3;
 
+// Above kBT channels the prologue sweeps the channels once (nsub == 1), so the wide instantiation keeps one row of
+// `sub` and its shared state stays static (stats kernel: 24 KB here + 17 KB of s_part at 1024 channels).
+template <int kMaxC>
 struct BwdShared {
-  float2 sub[4][kBMaxC];
-  float tot[2 * kBMaxC];
+  float2 sub[kMaxC > kBT ? 1 : 4][kMaxC];
+  float tot[2 * kMaxC];
   float mean[32], rstd[32];
-  float2 ab[kBMaxC];
+  float2 ab[kMaxC];
 };
 
 // Forward statistics + folded coefficients for sample n (same arithmetic, same order as adagn_apply_kernel).
-__device__ void bwd_prologue(const AdaGNBwdParams& p, int n, BwdShared& sh) {
+template <int kMaxC>
+__device__ void bwd_prologue(const AdaGNBwdParams& p, int n, BwdShared<kMaxC>& sh) {
   const int t = threadIdx.x, C = p.C, R = p.R;
   if (p.save_coef != nullptr) {               // coefficients saved by the forward kernel
     const int cpg = C / 32;
@@ -142,14 +150,15 @@ __device__ __forceinline__ void granule_dv(const AdaGNBwdParams& p, const uint4&
   }
 }
 
-__global__ void __launch_bounds__(kBT, 3) adagn_bwd_stats_kernel(const AdaGNBwdParams p) {
-  __shared__ BwdShared sh;
+template <int kMaxC>
+__global__ void __launch_bounds__(kBT, kBwdMinCtas<kMaxC>) adagn_bwd_stats_kernel(const AdaGNBwdParams p) {
+  __shared__ BwdShared<kMaxC> sh;
   __shared__ float s_part[kBT][17];
   const int n = blockIdx.y, t = threadIdx.x, C = p.C, R = p.R;
   griddep_launch();
   griddep_wait();                 // programmatic dependent launch: all inputs come from earlier kernels
   bwd_prologue(p, n, sh);
-  const int VPR = C >> 3, rpp = kBT / VPR;
+  const int VPR = C >> 3, rpp = kBT / VPR;    // 768 channels: 2 rows per pass, threads 192..255 idle
   const bool active = t < rpp * VPR;
   const int vl = t % VPR, rsub = t / VPR, v0 = p.c0 >> 3, cpg = C / 32;
   float A[8], B[8], s1[8], s2[8];          // s2 accumulates sum dv*x; the (x - mean)*rstd form is applied at the end
@@ -209,9 +218,10 @@ __global__ void __launch_bounds__(kBT, 3) adagn_bwd_stats_kernel(const AdaGNBwdP
   }
 }
 
-__global__ void __launch_bounds__(kBT, 3) adagn_bwd_apply_kernel(const AdaGNBwdParams p) {
-  __shared__ BwdShared sh;
-  __shared__ float s_S[2 * kBMaxC];
+template <int kMaxC>
+__global__ void __launch_bounds__(kBT, kBwdMinCtas<kMaxC>) adagn_bwd_apply_kernel(const AdaGNBwdParams p) {
+  __shared__ BwdShared<kMaxC> sh;
+  __shared__ float s_S[2 * kMaxC];
   __shared__ float s_G[64];
   const int n = blockIdx.y, t = threadIdx.x, C = p.C, R = p.R;
   griddep_launch();
@@ -343,7 +353,7 @@ cudaError_t launch_adagn_bwd(const idf_adagn_bwd_args& b, int num_sms, cudaStrea
   p.dx0 = static_cast<bf16*>(b.dx0); p.dx1 = static_cast<bf16*>(b.dx1); p.acc0 = b.acc0; p.acc1 = b.acc1;
   p.sums = b.sums; p.ws = b.ws; p.save_coef = a.save_coef;
   p.d_mod_t = b.d_mod_t; p.d_mod_z = b.d_mod_z; p.dgamma = b.dgamma; p.dbeta = b.dbeta;
-  if (p.C > kBMaxC || p.C % 32 != 0 || p.c0 % 8 != 0 || p.c1 % 8 != 0 || a.batch <= 0) return cudaErrorInvalidValue;
+  if (p.C > kBMaxCWide || p.C % 32 != 0 || p.c0 % 8 != 0 || p.c1 % 8 != 0 || a.batch <= 0) return cudaErrorInvalidValue;
   if (p.stats0 == nullptr || (p.c1 != 0 && (p.stats1 == nullptr || p.dx1 == nullptr)) || p.dx0 == nullptr ||
       p.dy == nullptr || p.sums == nullptr || p.ws == nullptr)
     return cudaErrorInvalidValue;
@@ -355,9 +365,12 @@ cudaError_t launch_adagn_bwd(const idf_adagn_bwd_args& b, int num_sms, cudaStrea
   p.slice_rows = (p.R + ns - 1) / ns;
   p.n_slices = (p.R + p.slice_rows - 1) / p.slice_rows;
   const dim3 grid(p.n_slices, a.batch, 1);
-  cudaError_t e = launch_kernel(adagn_bwd_stats_kernel, grid, dim3(kBT), 0, stream, g_pdl != 0, 0, p);
+  const bool wide = p.C > kBMaxC;
+  cudaError_t e = launch_kernel(wide ? adagn_bwd_stats_kernel<kBMaxCWide> : adagn_bwd_stats_kernel<kBMaxC>, grid, dim3(kBT),
+                                0, stream, g_pdl != 0, 0, p);
   if (e != cudaSuccess) return e;
-  return launch_kernel(adagn_bwd_apply_kernel, grid, dim3(kBT), 0, stream, g_pdl != 0, 0, p);
+  return launch_kernel(wide ? adagn_bwd_apply_kernel<kBMaxCWide> : adagn_bwd_apply_kernel<kBMaxC>, grid, dim3(kBT), 0,
+                       stream, g_pdl != 0, 0, p);
 }
 
 }  // namespace idf

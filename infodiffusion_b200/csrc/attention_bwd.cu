@@ -16,6 +16,13 @@
 //      and one thread per token writes the bf16 row (dq | dk | dv) of the pad-flat gradient matrix.
 // Splitting at the [S, S] matrices keeps every CTA's operands in shared memory (<= 192 KB) without cross-CTA
 // reductions: dK / dV sum over ALL queries, which a query-tile CTA cannot do alone.
+//
+// Wider heads (D = 256, 512: the vanilla Diff UNet's 16x16 and 8x8 levels) reuse the D = 128 machinery:
+//   * scores: S and dP reduce over d, so the kernel walks d in 128-wide chunks through the same shared-memory buffers
+//     and accumulates into the same two TMEM accumulators; the next chunk's Q | K load overlaps the dP MMAs of this one;
+//   * grads: grid (ceil(S/128), batch, D/128), CTA z owns the 128-wide column slice z of dQ, dK and dV (the B operands
+//     K / Q / dO are read at that slice), so each CTA is the D = 128 kernel at a column offset.
+// The P / dS workspace does not depend on D.
 #include "kernels.cuh"
 
 namespace idf {
@@ -41,20 +48,23 @@ __device__ __forceinline__ uint64_t desc_mn(uint32_t smem_addr, uint32_t lbo_byt
 // ---------------------------------------------------------------------------------------------------
 // kernel 1: P and dS rows of one 128-query tile
 // ---------------------------------------------------------------------------------------------------
-template <int S>
+template <int S, int D>
 __global__ void __launch_bounds__(kT, 1)
 attn_bwd_scores_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant__ CUtensorMap tmDO,
                        bf16* __restrict__ Pbuf, bf16* __restrict__ dSbuf, int Hp, int Wp, int W, float scale) {
   constexpr uint32_t QT = 2 * 128 * 128;          // a 128-row tile, two 64-wide d-chunks
   constexpr uint32_t KV_CHUNK = S * 128;          // one 64-wide d-chunk of K or V: [S x 128 B]
+  constexpr int NCH = D / kDh;                    // 128-wide d chunks, one after the other through the same buffers
+  constexpr int NBAR = NCH > 1 ? 5 : 3;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* smQ = smem;
   uint8_t* smDO = smQ + QT;
   uint8_t* smK = smDO + QT;
   uint8_t* smV = smK + 2 * KV_CHUNK;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smV + 2 * KV_CHUNK);    // 0: Q, K landed  1: dO, V landed  2: S, dP ready
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 3);
+  // 0: Q, K landed  1: dO, V landed  2: S, dP ready  (D > 128) 3: a chunk's S MMAs have read smQ / smK, 4: its dP MMAs smDO / smV
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smV + 2 * KV_CHUNK);
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + NBAR);
 
   const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
   const int n = blockIdx.y;
@@ -65,7 +75,7 @@ attn_bwd_scores_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_c
   const int qy0 = q0 / W, q_imgrows = q_rows / W;
 
   if (t == 0) {
-    for (int i = 0; i < 3; ++i) mbar_init(bars + i, 1);
+    for (int i = 0; i < NBAR; ++i) mbar_init(bars + i, 1);
     fence_mbar_init();
   }
   if (warp == 0) {
@@ -89,38 +99,46 @@ attn_bwd_scores_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_c
 
   if (t == 0) {
     const uint32_t box = static_cast<uint32_t>(W) * 128u;
-    mbar_arrive_expect_tx(bars + 0, box * 2u * static_cast<uint32_t>(q_imgrows + H));
-    for (int c = 0; c < 2; ++c)
-      for (int y = 0; y < q_imgrows; ++y)
-        tma_load_2d(smQ + c * (128 * 128) + y * box, &tmQKV, bars + 0, c * 64, img_row0 + (qy0 + y) * Wp);
-    for (int c = 0; c < 2; ++c)
-      for (int y = 0; y < H; ++y)
-        tma_load_2d(smK + c * KV_CHUNK + y * box, &tmQKV, bars + 0, kDh + c * 64, img_row0 + y * Wp);
-    mbar_arrive_expect_tx(bars + 1, box * 2u * static_cast<uint32_t>(q_imgrows + H));
-    for (int c = 0; c < 2; ++c)
-      for (int y = 0; y < q_imgrows; ++y)
-        tma_load_2d(smDO + c * (128 * 128) + y * box, &tmDO, bars + 1, c * 64, img_row0 + (qy0 + y) * Wp);
-    for (int c = 0; c < 2; ++c)
-      for (int y = 0; y < H; ++y)
-        tma_load_2d(smV + c * KV_CHUNK + y * box, &tmQKV, bars + 1, 2 * kDh + c * 64, img_row0 + y * Wp);
     constexpr uint32_t idesc = umma_idesc_f16(128, S, kFmtBF16);
-    mbar_wait(bars + 0, 0);
-    tc_fence_after();
 #pragma unroll
-    for (int c = 0; c < 2; ++c) {                 // S = Q K^T
-      const uint64_t da = umma_desc_k_sw128(smem_u32(smQ + c * (128 * 128)));
-      const uint64_t db = umma_desc_k_sw128(smem_u32(smK + c * KV_CHUNK));
+    for (int ch = 0; ch < NCH; ++ch) {
+      const int dc = ch * kDh;                    // first column of this d chunk
+      if (ch > 0) mbar_wait(bars + 3, (ch - 1) & 1);
+      mbar_arrive_expect_tx(bars + 0, box * 2u * static_cast<uint32_t>(q_imgrows + H));
+      for (int c = 0; c < 2; ++c)
+        for (int y = 0; y < q_imgrows; ++y)
+          tma_load_2d(smQ + c * (128 * 128) + y * box, &tmQKV, bars + 0, dc + c * 64, img_row0 + (qy0 + y) * Wp);
+      for (int c = 0; c < 2; ++c)
+        for (int y = 0; y < H; ++y)
+          tma_load_2d(smK + c * KV_CHUNK + y * box, &tmQKV, bars + 0, D + dc + c * 64, img_row0 + y * Wp);
+      if (ch > 0) mbar_wait(bars + 4, (ch - 1) & 1);
+      mbar_arrive_expect_tx(bars + 1, box * 2u * static_cast<uint32_t>(q_imgrows + H));
+      for (int c = 0; c < 2; ++c)
+        for (int y = 0; y < q_imgrows; ++y)
+          tma_load_2d(smDO + c * (128 * 128) + y * box, &tmDO, bars + 1, dc + c * 64, img_row0 + (qy0 + y) * Wp);
+      for (int c = 0; c < 2; ++c)
+        for (int y = 0; y < H; ++y)
+          tma_load_2d(smV + c * KV_CHUNK + y * box, &tmQKV, bars + 1, 2 * D + dc + c * 64, img_row0 + y * Wp);
+      mbar_wait(bars + 0, ch & 1);
+      tc_fence_after();
 #pragma unroll
-      for (int k = 0; k < 4; ++k) umma_f16(tmem_S, da + 2 * k, db + 2 * k, idesc, (c | k) != 0 ? 1u : 0u);
-    }
-    mbar_wait(bars + 1, 0);
-    tc_fence_after();
+      for (int c = 0; c < 2; ++c) {               // S = Q K^T
+        const uint64_t da = umma_desc_k_sw128(smem_u32(smQ + c * (128 * 128)));
+        const uint64_t db = umma_desc_k_sw128(smem_u32(smK + c * KV_CHUNK));
 #pragma unroll
-    for (int c = 0; c < 2; ++c) {                 // dP = dO V^T
-      const uint64_t da = umma_desc_k_sw128(smem_u32(smDO + c * (128 * 128)));
-      const uint64_t db = umma_desc_k_sw128(smem_u32(smV + c * KV_CHUNK));
+        for (int k = 0; k < 4; ++k) umma_f16(tmem_S, da + 2 * k, db + 2 * k, idesc, (ch | c | k) != 0 ? 1u : 0u);
+      }
+      if (ch + 1 < NCH) umma_commit(bars + 3);
+      mbar_wait(bars + 1, ch & 1);
+      tc_fence_after();
 #pragma unroll
-      for (int k = 0; k < 4; ++k) umma_f16(tmem_dP, da + 2 * k, db + 2 * k, idesc, (c | k) != 0 ? 1u : 0u);
+      for (int c = 0; c < 2; ++c) {               // dP = dO V^T
+        const uint64_t da = umma_desc_k_sw128(smem_u32(smDO + c * (128 * 128)));
+        const uint64_t db = umma_desc_k_sw128(smem_u32(smV + c * KV_CHUNK));
+#pragma unroll
+        for (int k = 0; k < 4; ++k) umma_f16(tmem_dP, da + 2 * k, db + 2 * k, idesc, (ch | c | k) != 0 ? 1u : 0u);
+      }
+      if (ch + 1 < NCH) umma_commit(bars + 4);
     }
     umma_commit(bars + 2);
   }
@@ -195,7 +213,7 @@ attn_bwd_scores_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_c
 // ---------------------------------------------------------------------------------------------------
 // kernel 2: dQ, dK, dV rows of one 128-token tile
 // ---------------------------------------------------------------------------------------------------
-template <int S>
+template <int S, int D>
 __global__ void __launch_bounds__(kT, 1)
 attn_bwd_grads_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant__ CUtensorMap tmDO,
                       const __grid_constant__ CUtensorMap tmPr, const __grid_constant__ CUtensorMap tmDSr,
@@ -217,6 +235,7 @@ attn_bwd_grads_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_co
   const int h0 = blockIdx.x * 128;                // first token of this tile
   const int img_row0 = n * Hp * Wp;
   const int H = S / W;
+  const int dc = (D == kDh) ? 0 : blockIdx.z * kDh;   // this CTA's 128-wide column slice of dQ, dK, dV
 
   if (t == 0) {
     for (int i = 0; i < 6; ++i) mbar_init(bars + i, 1);
@@ -240,7 +259,7 @@ attn_bwd_grads_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_co
     // ---- phase 1: dQ_h = dS[h, :] K
     mbar_arrive_expect_tx(bars + 0, KCH * 128u * 128u + 2u * ATOM);
     for (int kc = 0; kc < KCH; ++kc) tma_load_2d(smA + kc * (128 * 128), &tmDSr, bars + 0, kc * 64, n * S + h0);
-    load_tokens(&tmQKV, kDh, bars + 0);
+    load_tokens(&tmQKV, D + dc, bars + 0);
     mbar_wait(bars + 0, 0);
     tc_fence_after();
     {
@@ -262,8 +281,8 @@ attn_bwd_grads_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_co
       mbar_arrive_expect_tx(bars + 1 + ph, 4u * ATOM);
       for (int j = 0; j < 2; ++j)                 // columns beyond S (S = 64) are zero-filled by the TMA
         tma_load_2d(smA + j * ATOM, ph == 0 ? &tmDSc : &tmPr, bars + 1 + ph, h0 + 64 * j, n * S);
-      if (ph == 0) load_tokens(&tmQKV, 0, bars + 1 + ph);
-      else         load_tokens(&tmDO, 0, bars + 1 + ph);
+      if (ph == 0) load_tokens(&tmQKV, dc, bars + 1 + ph);
+      else         load_tokens(&tmDO, dc, bars + 1 + ph);
       mbar_wait(bars + 1 + ph, 0);
       tc_fence_after();
       constexpr uint32_t idesc = umma_idesc_f16(128, kDh, kFmtBF16) | (1u << 15) | (1u << 16);
@@ -283,9 +302,10 @@ attn_bwd_grads_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_co
   const uint32_t lane_addr = static_cast<uint32_t>(warp * 32) << 16;
   const int tok = h0 + row;
   const bool valid = tok < S;
-  bf16* orow = dqkv + (valid ? (static_cast<long long>(img_row0) + (tok / W) * Wp + (tok % W)) : 0) * (3 * kDh);
+  bf16* orow = dqkv + (valid ? (static_cast<long long>(img_row0) + (tok / W) * Wp + (tok % W)) : 0) * (3 * D);
 #pragma unroll 1
-  for (int c = 0; c < 3 * kDh / 32; ++c) {        // TMEM columns [0, 384) = dq | dk | dv, the row's layout in dqkv
+  for (int c = 0; c < 3 * kDh / 32; ++c) {        // TMEM columns [0, 384) = dq | dk | dv slices, at q / k / v + dc in dqkv
+    const int col = (D == kDh) ? c * 32 : (c >> 2) * D + dc + (c & 3) * 32;
     uint32_t v[32];
     tmem_ld_32x32(tmem_base + lane_addr + c * 32, v);
     tmem_ld_wait();
@@ -297,7 +317,7 @@ attn_bwd_grads_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_co
         o.y = pack_bf16x2(__uint_as_float(v[g * 8 + 2]), __uint_as_float(v[g * 8 + 3]));
         o.z = pack_bf16x2(__uint_as_float(v[g * 8 + 4]), __uint_as_float(v[g * 8 + 5]));
         o.w = pack_bf16x2(__uint_as_float(v[g * 8 + 6]), __uint_as_float(v[g * 8 + 7]));
-        *reinterpret_cast<uint4*>(orow + c * 32 + g * 8) = o;
+        *reinterpret_cast<uint4*>(orow + col + g * 8) = o;
       }
     }
   }
@@ -309,7 +329,7 @@ attn_bwd_grads_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_co
   }
 }
 
-template <int S>
+template <int S, int D>
 static cudaError_t launch_bwd_s(const CUtensorMap& tmQKV, const CUtensorMap& tmDO, const CUtensorMap& tmPr,
                                 const CUtensorMap& tmDSr, const CUtensorMap& tmDSc, bf16* P, bf16* dS, bf16* dqkv,
                                 int batch, int H, int W, float scale, cudaStream_t stream) {
@@ -320,27 +340,37 @@ static cudaError_t launch_bwd_s(const CUtensorMap& tmQKV, const CUtensorMap& tmD
   constexpr uint32_t SM2 = A_BYTES + 2 * ATOM + 64 + 1024;
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(attn_bwd_scores_kernel<S>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(SM1));
+    cudaError_t e = cudaFuncSetAttribute(attn_bwd_scores_kernel<S, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(SM1));
     if (e == cudaSuccess)
-      e = cudaFuncSetAttribute(attn_bwd_grads_kernel<S>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(SM2));
+      e = cudaFuncSetAttribute(attn_bwd_grads_kernel<S, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(SM2));
     if (e != cudaSuccess) return e;
     attr_set = true;
   }
   dim3 grid((S + 127) / 128, batch, 1);
-  attn_bwd_scores_kernel<S><<<grid, kT, SM1, stream>>>(tmQKV, tmDO, P, dS, H + 1, W + 1, W, scale);
+  attn_bwd_scores_kernel<S, D><<<grid, kT, SM1, stream>>>(tmQKV, tmDO, P, dS, H + 1, W + 1, W, scale);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return e;
-  attn_bwd_grads_kernel<S><<<grid, kT, SM2, stream>>>(tmQKV, tmDO, tmPr, tmDSr, tmDSc, dqkv, H + 1, W + 1, W);
+  grid.z = D / kDh;
+  attn_bwd_grads_kernel<S, D><<<grid, kT, SM2, stream>>>(tmQKV, tmDO, tmPr, tmDSr, tmDSc, dqkv, H + 1, W + 1, W);
   return cudaGetLastError();
+}
+
+template <int S>
+static cudaError_t launch_bwd_d(const CUtensorMap& tmQKV, const CUtensorMap& tmDO, const CUtensorMap& tmPr,
+                                const CUtensorMap& tmDSr, const CUtensorMap& tmDSc, bf16* P, bf16* dS, bf16* dqkv,
+                                int batch, int H, int W, int d, float scale, cudaStream_t stream) {
+  if (d == 128) return launch_bwd_s<S, 128>(tmQKV, tmDO, tmPr, tmDSr, tmDSc, P, dS, dqkv, batch, H, W, scale, stream);
+  if (d == 256) return launch_bwd_s<S, 256>(tmQKV, tmDO, tmPr, tmDSr, tmDSc, P, dS, dqkv, batch, H, W, scale, stream);
+  if (d == 512) return launch_bwd_s<S, 512>(tmQKV, tmDO, tmPr, tmDSr, tmDSc, P, dS, dqkv, batch, H, W, scale, stream);
+  return cudaErrorInvalidValue;
 }
 
 cudaError_t launch_attn_bwd(const CUtensorMap& tmQKV, const CUtensorMap& tmDO, const CUtensorMap& tmPr,
                             const CUtensorMap& tmDSr, const CUtensorMap& tmDSc, bf16* P, bf16* dS, bf16* dqkv, int batch,
                             int H, int W, int d, float scale, cudaStream_t stream) {
-  if (d != kDh) return cudaErrorInvalidValue;
   const int S = H * W;
-  if (S == 256) return launch_bwd_s<256>(tmQKV, tmDO, tmPr, tmDSr, tmDSc, P, dS, dqkv, batch, H, W, scale, stream);
-  if (S == 64) return launch_bwd_s<64>(tmQKV, tmDO, tmPr, tmDSr, tmDSc, P, dS, dqkv, batch, H, W, scale, stream);
+  if (S == 256) return launch_bwd_d<256>(tmQKV, tmDO, tmPr, tmDSr, tmDSc, P, dS, dqkv, batch, H, W, d, scale, stream);
+  if (S == 64) return launch_bwd_d<64>(tmQKV, tmDO, tmPr, tmDSr, tmDSc, P, dS, dqkv, batch, H, W, d, scale, stream);
   return cudaErrorInvalidValue;
 }
 

@@ -358,16 +358,14 @@ int idf_wgrad_plan_create(const idf_wgrad_desc* d, idf_wgrad_plan** out_plan) {
     }
   }
   const int ci_step = d->cin >= 128 ? 128 : 64;
-  p.n_units = 0;
-  for (int co0 = 0; co0 < d->cout; co0 += 128)
-    for (int ci0 = 0; ci0 < d->cin; ci0 += ci_step)
-      for (auto& c : cls) {
-        if (p.n_units == kWgMaxUnits) { delete pl; return fail(IDF_ERR_ARG, "too many wgrad units"); }
-        const int u = p.n_units++;
-        p.u_co0[u] = co0; p.u_ci0[u] = ci0; p.u_cin[u] = std::min(ci_step, d->cin - ci0);
-        p.u_ntap[u] = c.n; p.u_base[u] = c.base;
-        for (int k = 0; k < c.n; ++k) { p.u_rel[u * 3 + k] = c.rel[k]; p.u_tap[u * 3 + k] = c.id[k]; }
-      }
+  p.n_cl = static_cast<int32_t>(cls.size());
+  for (int c = 0; c < p.n_cl; ++c) {
+    p.c_ntap[c] = cls[c].n; p.c_base[c] = cls[c].base;
+    for (int k = 0; k < cls[c].n; ++k) { p.c_rel[c * 3 + k] = cls[c].rel[k]; p.c_tap[c * 3 + k] = cls[c].id[k]; }
+  }
+  p.ci_step = ci_step;
+  p.n_ci = (d->cin + ci_step - 1) / ci_step;
+  p.n_units = (d->cout + 127) / 128 * p.n_ci * p.n_cl;     // the kernel derives (co tile, ci chunk, cluster) from the index
   p.n_kb = static_cast<int32_t>((d->rows + 127) / 128);
   int slabs = (g_num_sms + p.n_units - 1) / p.n_units;   // one wave of CTAs: split-K only as far as needed
   if (slabs > p.n_kb) slabs = p.n_kb;
@@ -414,7 +412,7 @@ int64_t idf_adagn_bwd_ws_floats(int32_t batch, int32_t C) { return adagn_bwd_ws_
 int idf_adagn_silu_bwd(const idf_adagn_bwd_args* b, idf_stream_t stream) {
   if (b == nullptr) return fail(IDF_ERR_ARG, "null argument");
   cudaError_t e = launch_adagn_bwd(*b, g_num_sms, reinterpret_cast<cudaStream_t>(stream));
-  if (e != cudaSuccess) return cuda_fail(e, "adagn backward launch (needs stats0/stats1, dy, dx, sums, ws)");
+  if (e != cudaSuccess) return cuda_fail(e, "adagn backward launch (needs stats0/stats1, dy, dx, sums, ws; C <= 1024, C % 32 == 0)");
   return IDF_OK;
 }
 
@@ -450,10 +448,12 @@ int idf_attn_bwd(const void* qkv, const void* dout, void* dqkv, void* ws, int32_
   if (rc != IDF_OK) return rc;
   cudaError_t e;
   const int S_tok = H * W;
-  if (d != 128 || (S_tok != 64 && S_tok != 256)) {
+  if ((d != 128 && d != 256 && d != 512) || (S_tok != 64 && S_tok != 256)) {
     e = launch_attn_small_bwd(static_cast<const bf16*>(qkv), static_cast<const bf16*>(dout), static_cast<bf16*>(dqkv), batch,
                               H, W, d, scale, reinterpret_cast<cudaStream_t>(stream));
-    if (e != cudaSuccess) return cuda_fail(e, "attention backward launch (supported: d=128 with H*W in {64,256}; or H*W <= 64 with H*W*d <= 8192)");
+    if (e != cudaSuccess)
+      return cuda_fail(e, "attention backward launch (supported: d in {128,256,512} with H*W in {64,256}; "
+                          "or H*W <= 64 with H*W*d <= 8192)");
     return IDF_OK;
   }
   if (ws == nullptr) return fail(IDF_ERR_ARG, "attention backward needs a workspace of idf_attn_bwd_ws_bytes()");

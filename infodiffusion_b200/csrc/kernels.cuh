@@ -61,13 +61,14 @@ struct alignas(64) ConvKernelParams {
   int32_t xf_debug;                     // measurement only (idf_set_option "xf_debug")
 };
 
-constexpr int kWgMaxUnits = 64;
+constexpr int kWgMaxClusters = 9;
 struct alignas(64) WgradKernelParams {
   CUtensorMap tmDY;                 // dY [rows, Cout]  box {64, 128}
   CUtensorMap tmX;                  // X  [rowsX, Cin]  box {64, 136}
-  int32_t n_units;
-  int32_t u_co0[kWgMaxUnits], u_ci0[kWgMaxUnits], u_cin[kWgMaxUnits], u_ntap[kWgMaxUnits], u_base[kWgMaxUnits];
-  int32_t u_rel[kWgMaxUnits * 3], u_tap[kWgMaxUnits * 3];
+  // work unit u = (128-wide co tile u / (n_ci * n_cl), ci chunk (u / n_cl) % n_ci of ci_step channels, tap cluster u % n_cl)
+  int32_t n_units, n_cl, n_ci, ci_step;
+  int32_t c_ntap[kWgMaxClusters], c_base[kWgMaxClusters];           // per tap cluster: taps, X row offset of the halo
+  int32_t c_rel[kWgMaxClusters * 3], c_tap[kWgMaxClusters * 3];     // ... each tap's row shift within it and its index
   int32_t n_kb, kb_per_slab;
   int32_t cout, cin, ntaps;
   float* dw;                        // fp32 [Cout, ntaps, Cin], accumulated with atomics

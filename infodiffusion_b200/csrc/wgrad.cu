@@ -46,7 +46,9 @@ __global__ void __launch_bounds__(192, 1) wgrad_kernel(const __grid_constant__ W
   const int slab = blockIdx.x / p.n_units;
   const int kb_begin = slab * p.kb_per_slab;
   const int kb_end = min(p.n_kb, kb_begin + p.kb_per_slab);
-  const int co0 = p.u_co0[unit], ci0 = p.u_ci0[unit], ci_n = p.u_cin[unit], ntap = p.u_ntap[unit];
+  const int cl = unit % p.n_cl;
+  const int co0 = unit / (p.n_cl * p.n_ci) * 128, ci0 = (unit / p.n_cl) % p.n_ci * p.ci_step;
+  const int ci_n = min(p.ci_step, p.cin - ci0), ntap = p.c_ntap[cl];
   const int n_ci_atoms = ci_n >> 6;
 
   if (warp == 0 && lane == 0) {
@@ -78,7 +80,7 @@ __global__ void __launch_bounds__(192, 1) wgrad_kernel(const __grid_constant__ W
           tma_load_2d(a, &p.tmDY, full + st, co0, r0);                       // channels >= Cout are zero-filled
           tma_load_2d(a + kWgKB * 128, &p.tmDY, full + st, co0 + 64, r0);
           for (int j = 0; j < n_ci_atoms; ++j)
-            tma_load_2d(b + j * B_ATOM, &p.tmX, full + st, ci0 + 64 * j, r0 + p.u_base[unit]);
+            tma_load_2d(b + j * B_ATOM, &p.tmX, full + st, ci0 + 64 * j, r0 + p.c_base[cl]);
           if (++st == kWgStages) { st = 0; ph ^= 1u; }
         }
       }
@@ -96,7 +98,7 @@ __global__ void __launch_bounds__(192, 1) wgrad_kernel(const __grid_constant__ W
         const uint32_t b_addr = a_addr + A_BYTES;
         for (int t = 0; t < ntap; ++t) {
           // (shuffles from lane 0 tell the compiler these are warp-uniform)
-          const uint32_t brow = __shfl_sync(0xffffffffu, b_addr + static_cast<uint32_t>(p.u_rel[unit * 3 + t]) * 128u, 0);
+          const uint32_t brow = __shfl_sync(0xffffffffu, b_addr + static_cast<uint32_t>(p.c_rel[cl * 3 + t]) * 128u, 0);
           const uint32_t a_u = __shfl_sync(0xffffffffu, a_addr, 0);
           const uint32_t d = __shfl_sync(0xffffffffu, tmem_u + static_cast<uint32_t>(t * ci_n), 0);
           const uint32_t acc0 = kb > kb_begin ? 1u : 0u;
@@ -124,7 +126,7 @@ __global__ void __launch_bounds__(192, 1) wgrad_kernel(const __grid_constant__ W
       const int co = co0 + q * 32 + lane;
       const uint32_t lane_addr = static_cast<uint32_t>(q * 32) << 16;
       for (int t = 0; t < ntap; ++t) {
-        const int tap = p.u_tap[unit * 3 + t];
+        const int tap = p.c_tap[cl * 3 + t];
         for (int c = 0; c < ci_n; c += 32) {
           uint32_t v[32];
           tmem_ld_32x32(tmem + lane_addr + static_cast<uint32_t>(t * ci_n + c), v);

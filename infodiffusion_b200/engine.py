@@ -93,8 +93,7 @@ class VAct:
 FUSE_ADAGN = False
 FUSE_ADAGN_MIN_H = 64
 FUSE_ADAGN_MIN_ROWS = 128 * 65 * 65      # ... and only from this many pad-flat rows (batch 128 at 64x64)
-MAX_GN_CHANNELS = 1024       # widest GroupNorm the AdaGN forward kernels take (csrc/adagn.cu kMaxCWide)
-MAX_TRAIN_GN_CHANNELS = 256  # ... and their backward kernels (csrc/adagn_bwd.cu); wgrad plans stop at 64 work units
+MAX_GN_CHANNELS = 1024       # widest GroupNorm the AdaGN kernels take, forward and backward (kMaxCWide, kBMaxCWide)
 
 
 class Workspace:

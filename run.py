@@ -7,7 +7,12 @@ What differs, on purpose:
     of scope (SURVEY section 2), so images come from --data_npz (array `images`: N x H x W x C uint8 or N x C x H x W
     float in [-1, 1], optional `labels`) or are synthetic U[-1, 1] (--synthetic_size images);
   * shapes: the kernels cover the 64x64 / 64-channel configuration (celeba, ffhq, chairs-sized data with
-    --unets_channels 64); other dataset names raise;
+    --unets_channels 64) and the 32x32 cifar10 one; other dataset names raise.  The vanilla Diff model (UNet
+    ch_mult [1,2,4,8], GroupNorms over up to 1024 channels) trains and samples at these widths; wider ones raise early;
+  * eval_fid without --is_latent is the reference's two-phase sampler and, like the reference, loads the vanilla model
+    from ./models/diff/{dataset}_{a_dim}d/model-{epochs}.pth.  `--model vanilla --mode train` saves under
+    {model_folder}/diff/<experiment string>, which carries `_0.1mmd` unless --mmd_weight is 0 (reference naming, kept):
+    train the vanilla model with --mmd_weight 0 to write the file eval_fid reads;
   * torchrun: under WORLD_SIZE > 1 training is data parallel (--batch_size per GPU, like BASELINE configs[2]);
     sampling / encoding shard every round of --batch_size images over the ranks, all ranks drawing the round's full
     batch from the same seed, so the written images do not depend on the number of GPUs (checked by
@@ -259,16 +264,15 @@ def train_latent_ddim(args):
 
 def _check_widths(args, vanilla: bool = None) -> None:
     """Fail EARLY and clearly for configurations the kernels do not cover (instead of deep inside plan creation)."""
-    from infodiffusion_b200.engine import MAX_GN_CHANNELS, MAX_TRAIN_GN_CHANNELS
+    from infodiffusion_b200.engine import MAX_GN_CHANNELS
     vanilla = (args.model == 'vanilla') if vanilla is None else vanilla
     if vanilla and not args.is_latent and args.mode != 'train_latent_ddim':
         widest = 8 * args.unets_channels                      # Diff hard-wires ch_mult = [1, 2, 4, 8] (models.py:746)
-        limit = MAX_TRAIN_GN_CHANNELS if args.mode == 'train' else MAX_GN_CHANNELS
-        if 2 * widest > limit:
+        if 2 * widest > MAX_GN_CHANNELS:
             raise NotImplementedError(
                 f"the vanilla image model (Diff over UNet, ch_mult [1,2,4,8], {widest} channels, GroupNorm over "
-                f"{2 * widest}) exceeds the kernels' limit of {limit} GroupNorm channels for --mode {args.mode} "
-                "(inference covers 1024, the backward kernels 256); see DESIGN.md section 7")
+                f"{2 * widest}) exceeds the kernels' limit of {MAX_GN_CHANNELS} GroupNorm channels "
+                f"(--mode {args.mode}; training and inference alike); see DESIGN.md section 7")
 
 
 def _load(args, device, shape):
