@@ -34,8 +34,8 @@ import torch.nn as nn
 from . import _lib
 from ._lib import EPI_BF16, EPI_F32_NCHW, EPI_SAMPLER, AdaGNArgs, ConvDesc
 from .layout import (ParamIndex, pack_conv1x1, pack_conv3x3, pack_conv3x3_up2, pad_cols as _pad_cols, pad_rows as _pad_rows,
-                     probing, pv, taps3x3, taps_stride2, taps_up2)
-from .modules import AttnBlock, AuxResBlock, DownSample, ResBlock, UpSample
+                     probing, pv, tap_offsets3x3, taps_stride2, taps_up2)
+from .modules import AttnBlock, AuxResBlock, DownSample, ResBlock, UpSample, timestep_embedding
 
 BF16 = torch.bfloat16
 
@@ -358,22 +358,7 @@ class Plan:
                                    and src0.rows >= FUSE_ADAGN_MIN_ROWS)
         if fuse and src0.has_stats and (src1 is None or src1.has_stats):
             Cc = src0.C + (src1.C if src1 is not None else 0)
-            a = AdaGNArgs()
-            a.c0 = src0.C
-            a.stats0, a.stats_unit0 = src0.stats.data_ptr(), src0.stats_unit
-            a.stats_planes0, a.stats_rows0 = src0.stats_planes, src0.stats_rows
-            if src1 is not None:
-                a.c1, a.stats1, a.stats_unit1 = src1.C, src1.stats.data_ptr(), src1.stats_unit
-                a.stats_planes1, a.stats_rows1 = src1.stats_planes, src1.stats_rows
-            a.batch, a.H, a.W = self.B, src0.H, src0.H
-            gamma, beta = self.f32(lambda: pv(gn.weight)), self.f32(lambda: pv(gn.bias))
-            a.gamma, a.beta, a.eps = gamma.data_ptr(), beta.data_ptr(), float(gn.eps)
-            if mod_t is not None:
-                a.mod_t, a.mod_t_step_stride, a.mod_t_batch_stride = mod_t
-            if mod_z is not None:
-                a.mod_z, a.mod_z_step_stride, a.mod_z_batch_stride = mod_z
-            a.step_ptr = _ptr(step)
-            a.apply_silu = 1 if silu else 0
+            a, _, _ = self._adagn_args(src0, src1, gn, silu, mod_t, mod_z, step)
             ctab = torch.zeros(self.B, Cc, 2, dtype=torch.float32, device=self.device)
             self.keep += [a, ctab]
             self._emit("adagn_coef", self.lib.idf_adagn_coef, (C.byref(a), ctab.data_ptr()))
@@ -403,19 +388,17 @@ class Plan:
         xf = (src.coef, src.silu, kx) if isinstance(src, VAct) else None
         return list(parts), kb, xf
 
-    def adagn(self, src0: Act, src1: Optional[Act], out: Act, gn: nn.GroupNorm, silu: bool, mod_t=None, mod_z=None,
-              step=None, dropout: bool = False, mod_cols: Optional[int] = None) -> None:
-        """Fused AdaGN.  mod_t / mod_z = (pointer, step stride, batch stride) of this block's (scale | shift)
-        columns; `dropout` applies inverted dropout after the SiLU (training plans only)."""
+    def _adagn_args(self, src0: Act, src1: Optional[Act], gn: nn.GroupNorm, silu: bool, mod_t, mod_z, step):
+        """(AdaGNArgs, gamma, beta) shared by the stand-alone and the conv-fused AdaGN: shapes, GroupNorm affine,
+        modulation, SiLU, and the sources' statistics records when their producers wrote them.  The caller sets the
+        activation pointers and what only it needs."""
         a = AdaGNArgs()
-        a.src0, a.c0 = src0.t.data_ptr(), src0.C
+        a.c0 = src0.C
         if src1 is not None:
-            a.src1, a.c1 = src1.t.data_ptr(), src1.C
-        a.out = out.t.data_ptr()
+            a.c1 = src1.C
         a.batch, a.H, a.W = self.B, src0.H, src0.H
         gamma, beta = self.f32(lambda: pv(gn.weight)), self.f32(lambda: pv(gn.bias))
-        a.gamma, a.beta = gamma.data_ptr(), beta.data_ptr()
-        a.eps = float(gn.eps)
+        a.gamma, a.beta, a.eps = gamma.data_ptr(), beta.data_ptr(), float(gn.eps)
         if mod_t is not None:
             a.mod_t, a.mod_t_step_stride, a.mod_t_batch_stride = mod_t
         if mod_z is not None:
@@ -428,6 +411,16 @@ class Plan:
             if src1 is not None:
                 a.stats1, a.stats_unit1 = src1.stats.data_ptr(), src1.stats_unit
                 a.stats_planes1, a.stats_rows1 = src1.stats_planes, src1.stats_rows
+        return a, gamma, beta
+
+    def adagn(self, src0: Act, src1: Optional[Act], out: Act, gn: nn.GroupNorm, silu: bool, mod_t=None, mod_z=None,
+              step=None, dropout: bool = False, mod_cols: Optional[int] = None) -> None:
+        """Fused AdaGN.  mod_t / mod_z = (pointer, step stride, batch stride) of this block's (scale | shift)
+        columns; `dropout` applies inverted dropout after the SiLU (training plans only)."""
+        a, gamma, beta = self._adagn_args(src0, src1, gn, silu, mod_t, mod_z, step)
+        a.src0, a.out = src0.t.data_ptr(), out.t.data_ptr()
+        if src1 is not None:
+            a.src1 = src1.t.data_ptr()
         if dropout and self.training and self.dropout_p > 0:
             self._drop_layers += 1
             a.dropout_p, a.dropout_seed, a.dropout_layer = self.dropout_p, self.dropout_seed.data_ptr(), self._drop_layers
@@ -459,10 +452,6 @@ class Plan:
 
     # ---- composite emitters ----------------------------------------------------------------------
     @staticmethod
-    def taps3x3(cin: int, H: int, src: int = 0):
-        return taps3x3(cin, H, H, src)
-
-    @staticmethod
     def _bn(cout: int) -> int:
         return 128 if cout % 128 == 0 else 64
 
@@ -471,7 +460,6 @@ class Plan:
         """3x3 / stride 1 / pad 1 conv (+ residual, or + 1x1 shortcut conv over raw sources as extra K-blocks)."""
         cin, cout, H = src.C, conv.out_channels, src.H
         assert conv.in_channels == cin and cout % 64 == 0
-        from .layout import tap_offsets3x3
         srcs, kb, xf = self._operand(src, tap_offsets3x3(H, H))
         if shortcut is None:
             wp = lambda: pack_conv3x3(pv(conv.weight))
@@ -623,7 +611,6 @@ class Plan:
 
     def tail(self, h: Act, gn: nn.GroupNorm, tconv: nn.Conv2d, H: int, cout: int, epilogue: int, out_f32, **extra) -> None:
         """tail: AdaGN + 3x3 conv to `cout` (<= 16) channels, fp32 NCHW out or fused sampler update."""
-        from .layout import tap_offsets3x3
         ta = self.norm(h, None, gn, silu=True)
         srcs, kb, xf = self._operand(ta, tap_offsets3x3(H, H))
         self.conv(srcs, kb, self.weight(lambda: _pad_rows(pack_conv3x3(pv(tconv.weight)), 16)),
@@ -635,34 +622,88 @@ class Plan:
         self.done(ta)
         self.ws.free(h)
 
+    def unet_body(self, net, x_src: torch.Tensor, Cimg: int, H: int, mods=None) -> Act:
+        """head -> down path (every output kept as a skip) -> middle -> up path (skips popped, upsampling folded) of
+        a UNet-shaped `net`; returns the activation its tail reads.  `mods(blk)`: the modulation keyword arguments of
+        res_block for a conditioned block."""
+        kw = mods if mods is not None else (lambda blk: {})
+        h = self.head(x_src, net.head, Cimg, H)
+        skips = [h]
+        for layer in net.downblocks:
+            if isinstance(layer, DownSample):
+                h = self.downsample(h, layer.main)
+            else:
+                h = self.res_block([h], layer, free_inputs=False, **kw(layer))
+            skips.append(h)
+        for i, layer in enumerate(net.middleblocks):
+            # the first middle block reads the last skip tensor, which must stay alive for the up path
+            h = self.res_block([h], layer, free_inputs=i > 0, **kw(layer))
+        for layer in net.upblocks:
+            if isinstance(layer, UpSample):
+                h2 = self.upsample(h, layer.main)
+                self.ws.free(h)
+                h = h2
+            else:
+                h = self.res_block([h, skips.pop()], layer, free_inputs=True, **kw(layer))
+        assert not skips
+        return h
+
+    # modulation MLPs ------------------------------------------------------------------------------
+    def _emit_time_mlp(self, net, pack: "ModulationPack", t_idx: torch.Tensor, out: torch.Tensor) -> None:
+        """out[m] = concat_blocks temb_proj(SiLU(time_embedding(t_idx[m])))  (modules.py:36-38, 249, 312)."""
+        te = net.time_embedding.timembedding
+        M = t_idx.shape[0]
+        f32 = dict(dtype=torch.float32, device=self.device)
+        e0 = torch.zeros(M, te[0].weight.shape[1], **f32)
+        e1 = torch.zeros(M, te[1].out_features, **f32)
+        e2 = torch.zeros(M, te[3].out_features, **f32)
+        self.keep += [e0, e1, e2]
+        table = self.f32(te[0].weight)
+        self._emit("gather_rows", self.lib.idf_gather_rows_f32, (table.data_ptr(), t_idx.data_ptr(), e0.data_ptr(), M,
+                                                                 e0.shape[1]))
+        self.linear(e0, self.f32(te[1].weight), self.f32(te[1].bias), e1, silu_in=False)
+        self.linear(e1, self.f32(te[3].weight), self.f32(te[3].bias), e2, silu_in=True)
+        self.linear(e2, pack.w_t, pack.b_t, out, silu_in=True)
+
+    def _emit_latent_mlp(self, net, pack: "ModulationPack", a_in: torch.Tensor, out: torch.Tensor) -> None:
+        """out[n] = concat_blocks aemb_proj(SiLU(fc_a(a[n])))  (models.py:298; modules.py:316)."""
+        fc = net.fc_a
+        pre_silu = isinstance(fc, nn.Sequential)      # BottleneckAuxUNet: fc_a = SiLU -> Linear (models.py:336-339)
+        if pre_silu:
+            fc = fc[1]
+        aemb = torch.zeros(a_in.shape[0], fc.out_features, dtype=torch.float32, device=self.device)
+        self.keep.append(aemb)
+        self.linear(a_in, self.f32(fc.weight), self.f32(fc.bias), aemb, silu_in=pre_silu)
+        self.linear(aemb, pack.w_z, pack.b_z, out, silu_in=True)
+
 
 # ------------------------------------------------------------------------------------------------
 # modulation (temb_proj / aemb_proj of every block, batched)
 # ------------------------------------------------------------------------------------------------
+def modulation_weights(blocks: Sequence[nn.Module]) -> Tuple[torch.Tensor, ...]:
+    """(w_t, b_t, w_z, b_z): the temb_proj and aemb_proj Linears of `blocks` concatenated along their outputs in
+    block order, with zero rows for a block without aemb_proj.  Not detached, so training can differentiate
+    through them."""
+    lin_t = [b.temb_proj[1] for b in blocks]
+    lin_z = [b.aemb_proj[1] if hasattr(b, "aemb_proj") else None for b in blocks]
+    w_z = [z.weight if z is not None else torch.zeros_like(t.weight) for t, z in zip(lin_t, lin_z)]
+    b_z = [z.bias if z is not None else torch.zeros_like(t.bias) for t, z in zip(lin_t, lin_z)]
+    return (torch.cat([t.weight for t in lin_t], 0), torch.cat([t.bias for t in lin_t], 0), torch.cat(w_z, 0),
+            torch.cat(b_z, 0))
+
+
 class ModulationPack:
     """Column layout of the concatenated per-block (scale | shift) projections."""
 
     def __init__(self, blocks: Sequence[nn.Module], device):
         self.offsets: Dict[int, int] = {}
-        wt, bt, wz, bz = [], [], [], []
         off = 0
-        self.has_z = False
         for blk in blocks:
             self.offsets[id(blk)] = off
-            lin_t = blk.temb_proj[1]
-            wt.append(lin_t.weight.detach())
-            bt.append(lin_t.bias.detach())
-            if hasattr(blk, "aemb_proj"):
-                self.has_z = True
-                wz.append(blk.aemb_proj[1].weight.detach())
-                bz.append(blk.aemb_proj[1].bias.detach())
-            else:
-                wz.append(torch.zeros_like(lin_t.weight))
-                bz.append(torch.zeros_like(lin_t.bias))
-            off += lin_t.out_features
+            off += blk.temb_proj[1].out_features
         self.ncol = off
-        f = lambda xs: torch.cat(xs, 0).to(device=device, dtype=torch.float32).contiguous()
-        self.w_t, self.b_t, self.w_z, self.b_z = f(wt), f(bt), f(wz), f(bz)
+        self.w_t, self.b_t, self.w_z, self.b_z = (x.detach().to(device=device, dtype=torch.float32).contiguous()
+                                                  for x in modulation_weights(blocks))
 
 
 def conditioned_blocks(net) -> List[nn.Module]:
@@ -716,10 +757,10 @@ class BackbonePlan(Plan):
             self.mod_z = torch.zeros(B, ncol, **f32)
             if mode == "eps":
                 self.t_idx = torch.zeros(B, dtype=torch.long, device=device)
-                self._emit_time_mlp(self.t_idx, self.mod_t)
+                self._emit_time_mlp(net, self.pack, self.t_idx, self.mod_t)
                 if hasattr(net, "fc_a"):                      # UNet (models.py:7) has no latent input
                     self.a_in = torch.zeros(B, net.a_dim, **f32)
-                    self._emit_latent_mlp(self.a_in, self.mod_z)
+                    self._emit_latent_mlp(net, self.pack, self.a_in, self.mod_z)
             else:
                 self.d_mod_t = torch.zeros(B, ncol, **f32)
                 self.d_mod_z = torch.zeros(B, ncol, **f32)
@@ -737,69 +778,15 @@ class BackbonePlan(Plan):
         def mods(blk):
             col = self.pack.offsets[id(blk)]
             off = col * 4
-            mt = (mod_t_arg[0] + off, mod_t_arg[1], mod_t_arg[2])
             mz = (mod_z_arg[0] + off, mod_z_arg[1], mod_z_arg[2]) if hasattr(blk, "aemb_proj") else None
-            return mt, mz, col
+            return dict(mod_t=(mod_t_arg[0] + off, mod_t_arg[1], mod_t_arg[2]), mod_z=mz, step=self.step, mod_cols=col)
 
-        ws = self.ws
-        h = self.head(x_src, net.head, Cimg, H)
-        skips = [h]
-        for layer in net.downblocks:
-            if isinstance(layer, DownSample):
-                h = self.downsample(h, layer.main)
-            else:
-                mt, mz, col = mods(layer)
-                h = self.res_block([h], layer, mod_t=mt, mod_z=mz, step=self.step, free_inputs=False, mod_cols=col)
-            skips.append(h)
-        first = True
-        for layer in net.middleblocks:
-            mt, mz, col = mods(layer)
-            # the first middle block reads the last skip tensor, which must stay alive for the up path
-            h = self.res_block([h], layer, mod_t=mt, mod_z=mz, step=self.step, free_inputs=not first, mod_cols=col)
-            first = False
-        for layer in net.upblocks:
-            if isinstance(layer, UpSample):
-                h2 = self.upsample(h, layer.main)
-                ws.free(h)
-                h = h2
-            else:
-                mt, mz, col = mods(layer)
-                h = self.res_block([h, skips.pop()], layer, mod_t=mt, mod_z=mz, step=self.step, free_inputs=True,
-                                   mod_cols=col)
-        assert not skips
+        h = self.unet_body(net, x_src, Cimg, H, mods)
         if mode in ("eps", "train"):
             self.tail(h, net.tail[0], net.tail[-1], H, Cimg, EPI_F32_NCHW, self.eps_out)
         else:
             self.tail(h, net.tail[0], net.tail[-1], H, Cimg, EPI_SAMPLER, self.eps_out, x_io=x_io, noise=noise,
                       coef=coef, step=step)
-
-    # modulation MLPs ------------------------------------------------------------------------------
-    def _emit_time_mlp(self, t_idx: torch.Tensor, out: torch.Tensor) -> None:
-        """out[m] = concat_blocks temb_proj(SiLU(time_embedding(t_idx[m])))  (modules.py:36-38, 249, 312)."""
-        te = self.net.time_embedding.timembedding
-        M = t_idx.shape[0]
-        f32 = dict(dtype=torch.float32, device=self.device)
-        e0 = torch.zeros(M, te[0].weight.shape[1], **f32)
-        e1 = torch.zeros(M, te[1].out_features, **f32)
-        e2 = torch.zeros(M, te[3].out_features, **f32)
-        self.keep += [e0, e1, e2]
-        table = self.f32(te[0].weight)
-        self._emit("gather_rows", self.lib.idf_gather_rows_f32, (table.data_ptr(), t_idx.data_ptr(), e0.data_ptr(), M,
-                                                                 e0.shape[1]))
-        self.linear(e0, self.f32(te[1].weight), self.f32(te[1].bias), e1, silu_in=False)
-        self.linear(e1, self.f32(te[3].weight), self.f32(te[3].bias), e2, silu_in=True)
-        self.linear(e2, self.pack.w_t, self.pack.b_t, out, silu_in=True)
-
-    def _emit_latent_mlp(self, a_in: torch.Tensor, out: torch.Tensor) -> None:
-        """out[n] = concat_blocks aemb_proj(SiLU(fc_a(a[n])))  (models.py:298; modules.py:316)."""
-        fc = self.net.fc_a
-        pre_silu = isinstance(fc, nn.Sequential)      # BottleneckAuxUNet: fc_a = SiLU -> Linear (models.py:336-339)
-        if pre_silu:
-            fc = fc[1]
-        aemb = torch.zeros(a_in.shape[0], fc.out_features, dtype=torch.float32, device=self.device)
-        self.keep.append(aemb)
-        self.linear(a_in, self.f32(fc.weight), self.f32(fc.bias), aemb, silu_in=pre_silu)
-        self.linear(aemb, self.pack.w_z, self.pack.b_z, out, silu_in=True)
 
 
 class ModulationTables(Plan):
@@ -810,14 +797,13 @@ class ModulationTables(Plan):
         self.net, self.pack = net, pack
         self.t_all = torch.arange(T, dtype=torch.long, device=device)
         self.table = torch.zeros(T, pack.ncol, dtype=torch.float32, device=device)
-        BackbonePlan._emit_time_mlp(self, self.t_all, self.table)
+        self._emit_time_mlp(net, pack, self.t_all, self.table)
 
     def latent_rows(self, a: torch.Tensor, out: torch.Tensor) -> None:
         if not hasattr(self.net, "fc_a"):
             return
         p = Plan(1, self.device)
-        p.net, p.pack = self.net, self.pack
-        BackbonePlan._emit_latent_mlp(p, a, out)
+        p._emit_latent_mlp(self.net, self.pack, a, out)
         p.run()
         torch.cuda.current_stream(self.device).synchronize()  # p's temporaries die with it
 
@@ -848,27 +834,7 @@ class EncoderPlan(Plan):
         self.a = torch.zeros(B, net.a_dim, **f32)
         self.mu = torch.zeros(B, net.a_dim, **f32)
         self.log_var = torch.zeros(B, net.a_dim, **f32)
-        ws = self.ws
-        h = self.head(self.x_in, net.head, Cimg, H)
-        skips = [h]
-        for layer in net.downblocks:
-            if isinstance(layer, DownSample):
-                h = self.downsample(h, layer.main)
-            else:
-                h = self.res_block([h], layer, free_inputs=False)
-            skips.append(h)
-        first = True
-        for layer in net.middleblocks:
-            h = self.res_block([h], layer, free_inputs=not first)
-            first = False
-        for layer in net.upblocks:
-            if isinstance(layer, UpSample):
-                h2 = self.upsample(h, layer.main)
-                ws.free(h)
-                h = h2
-            else:
-                h = self.res_block([h, skips.pop()], layer, free_inputs=True)
-        assert not skips
+        h = self.unet_body(net, self.x_in, Cimg, H)
         self.tail(h, net.tail[0], net.tail[-1], H, 1, EPI_F32_NCHW, self.map_out)
         if not training:
             flat = self.map_out.view(B, H * W)
@@ -925,6 +891,17 @@ def encoder_forward(net, x: torch.Tensor):
 # ------------------------------------------------------------------------------------------------
 # latent eps-network (LatentUNet, reference models.py:166-234)
 # ------------------------------------------------------------------------------------------------
+def _emit_latent_time_chain(plan: Plan, te: nn.Sequential, e0: torch.Tensor, w_cond: torch.Tensor,
+                            b_cond: torch.Tensor, out: torch.Tensor) -> None:
+    """out = concat_layers linear_emb(SiLU(te[2](SiLU(te[0](e0)))))  for the rows of the sinusoid embeddings e0."""
+    e1 = torch.zeros(e0.shape[0], te[0].out_features, dtype=torch.float32, device=plan.device)
+    e2 = torch.zeros(e0.shape[0], te[2].out_features, dtype=torch.float32, device=plan.device)
+    plan.keep += [e1, e2]
+    plan.linear(e0, plan.f32(te[0].weight), plan.f32(te[0].bias), e1, silu_in=False)
+    plan.linear(e1, plan.f32(te[2].weight), plan.f32(te[2].bias), e2, silu_in=True)
+    plan.linear(e2, w_cond, b_cond, out, silu_in=True)                 # cond_layers = act -> linear_emb
+
+
 class LatentPlan(Plan):
     """eps = LatentUNet(z, t) for a fixed batch: per layer one fp32 GEMM (idf_linear_f32) and one fused
     (1 + cond) scale -> LayerNorm -> SiLU kernel that writes straight into the [h | z] concatenation buffer the
@@ -955,31 +932,22 @@ class LatentPlan(Plan):
         self.ybuf = torch.zeros(B, Hd, **f32)
         w_cond = self.f32(torch.cat([l.linear_emb.weight for l in layers[:-1]], 0))
         b_cond = self.f32(torch.cat([l.linear_emb.bias for l in layers[:-1]], 0))
-        te = net.time_embed
         C_t = net.num_time_emb_channels
+        assert T is not None, "LatentPlan needs the number of diffusion steps for its sinusoid table"
+        table = timestep_embedding(torch.arange(T, device=device), C_t).contiguous()          # modules.py:41-60
         if mode == "eps":
-            assert T is not None, "LatentPlan needs the number of diffusion steps for its sinusoid table"
-            from .modules import timestep_embedding
             self.t_idx = torch.zeros(B, dtype=torch.long, device=device)
-            table = timestep_embedding(torch.arange(T, device=device), C_t).contiguous()      # modules.py:41-60
-            e0, e1, e2 = torch.zeros(B, C_t, **f32), torch.zeros(B, D, **f32), torch.zeros(B, D, **f32)
+            e0 = torch.zeros(B, C_t, **f32)
             self.cond = torch.zeros(B, n_cond * Hd, **f32)
-            self.keep += [table, e0, e1, e2]
+            self.keep += [table, e0]
             self._emit("gather_rows", self.lib.idf_gather_rows_f32, (table.data_ptr(), self.t_idx.data_ptr(), e0.data_ptr(), B, C_t))
-            self.linear(e0, self.f32(te[0].weight), self.f32(te[0].bias), e1, silu_in=False)
-            self.linear(e1, self.f32(te[2].weight), self.f32(te[2].bias), e2, silu_in=True)
-            self.linear(e2, w_cond, b_cond, self.cond, silu_in=True)           # cond_layers = act -> linear_emb
+            _emit_latent_time_chain(self, net.time_embed, e0, w_cond, b_cond, self.cond)
             cond_arg = lambda i: (self.cond.data_ptr() + 4 * i * Hd, n_cond * Hd, 0, None)
         else:
-            assert z_io is not None and coef is not None and step is not None and T is not None
-            from .modules import timestep_embedding
+            assert z_io is not None and coef is not None and step is not None
             tp = Plan(1, device)                                               # one-off: the [T, n_cond * Hd] table
-            e0 = timestep_embedding(torch.arange(T, device=device), C_t).contiguous()
-            e1, e2 = torch.zeros(T, D, **f32), torch.zeros(T, D, **f32)
             self.cond = torch.zeros(T, n_cond * Hd, **f32)
-            tp.linear(e0, tp.f32(te[0].weight), tp.f32(te[0].bias), e1, silu_in=False)
-            tp.linear(e1, tp.f32(te[2].weight), tp.f32(te[2].bias), e2, silu_in=True)
-            tp.linear(e2, w_cond, b_cond, self.cond, silu_in=True)
+            _emit_latent_time_chain(tp, net.time_embed, table, w_cond, b_cond, self.cond)
             tp.run()
             torch.cuda.current_stream(device).synchronize()
             cond_arg = lambda i: (self.cond.data_ptr() + 4 * i * Hd, 0, n_cond * Hd, step.data_ptr())

@@ -66,6 +66,26 @@ def step_coefficients(kind: str, betas, alphas, alpha_bars, alpha_prev_bars) -> 
     return out.float()
 
 
+def _capture_step(enqueue, x: torch.Tensor, step: torch.Tensor, idx: int) -> torch.cuda.CUDAGraph:
+    """CUDA graph of one sampler step.  `enqueue` runs once on a side stream first (kernel attributes are set outside
+    the capture); that warm-up updates the live buffer x in place, so x is restored and the step counter refilled."""
+    dev = x.device
+    keep = x.clone()
+    torch.cuda.synchronize(dev)
+    side = torch.cuda.Stream(dev)
+    side.wait_stream(torch.cuda.current_stream(dev))
+    with torch.cuda.stream(side):
+        enqueue()
+    torch.cuda.current_stream(dev).wait_stream(side)
+    torch.cuda.synchronize(dev)
+    g = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(g):
+        enqueue()
+    x.copy_(keep)
+    step.fill_(idx)
+    return g
+
+
 class _FusedSampler:
     """Graph-captured step for an InfoDiff model: UNet forward + fused x update, for a fixed batch."""
 
@@ -111,8 +131,7 @@ class _FusedSampler:
                     raise NotImplementedError("re-encoding reverse DDIM with a sampled latent (kld_weight != 0)")
                 ep = EncoderPlan(model.encoder, chunk, dev, ws=self.ws, x_in=self.x[sl])
                 zp = Plan(chunk, dev, ws=self.ws)
-                zp.net, zp.pack = net, self.pack
-                BackbonePlan._emit_latent_mlp(zp, ep.a, self.mod_z[sl])
+                zp._emit_latent_mlp(net, self.pack, ep.a, self.mod_z[sl])
                 self.plans += [ep, zp]
             bp = BackbonePlan(net, chunk, dev, mode="sampler", ws=self.ws, x_io=self.x[sl],
                               noise=None if self.noise is None else self.noise[sl], coef=self.coef, step=self.step,
@@ -142,31 +161,15 @@ class _FusedSampler:
         for st in self.lane_streams[1:]:                 # join
             cur.wait_stream(st)
 
-    def capture(self) -> None:
-        torch.cuda.synchronize(self.x.device)
-        s = torch.cuda.Stream(self.x.device)
-        s.wait_stream(torch.cuda.current_stream(self.x.device))
-        with torch.cuda.stream(s):
-            self._enqueue()          # warm-up (also sets func attributes outside capture)
-        torch.cuda.current_stream(self.x.device).wait_stream(s)
-        torch.cuda.synchronize(self.x.device)
-        g = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(g):
-            self._enqueue()
-        self.graph = g
-
     def run_step(self, idx: int, use_graph: bool = True) -> None:
         self.step.fill_(idx)
-        if use_graph:
-            if self.graph is None:
-                x_save = self.x.clone()
-                self.capture()
-                self.x.copy_(x_save)
-                self.step.fill_(idx)
-            self.graph.replay()
-            _lib.count_launch(self.n_launch)
-        else:
+        if not use_graph:
             self._enqueue()
+            return
+        if self.graph is None:
+            self.graph = _capture_step(self._enqueue, self.x, self.step, idx)
+        self.graph.replay()
+        _lib.count_launch(self.n_launch)
 
 
 class DiffusionProcess():
@@ -388,20 +391,7 @@ class LatentDiffusionProcess():
             s.plan.run()
             return
         if s.graph is None:
-            keep = s.x.clone()
-            torch.cuda.synchronize(self.device)
-            side = torch.cuda.Stream(self.device)
-            side.wait_stream(torch.cuda.current_stream(self.device))
-            with torch.cuda.stream(side):
-                s.plan.run()                         # warm-up outside capture
-            torch.cuda.current_stream(self.device).wait_stream(side)
-            torch.cuda.synchronize(self.device)
-            g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g):
-                s.plan.run()
-            s.graph = g
-            s.x.copy_(keep)
-            s.step.fill_(idx)
+            s.graph = _capture_step(s.plan.run, s.x, s.step, idx)
         s.graph.replay()
         _lib.count_launch(len(s.plan.ops))
 

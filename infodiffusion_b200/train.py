@@ -485,14 +485,7 @@ class GradSync:
         self.covered.update(id(p) for p in params)
 
     def finish(self, params: Sequence[nn.Parameter]) -> None:
-        import torch.distributed as dist
-        rest = [p.grad for p in params if p.grad is not None and id(p) not in self.covered]
-        if rest:
-            buf = torch._utils._flatten_dense_tensors(rest)
-            dist.all_reduce(buf, op=dist.ReduceOp.SUM)
-            buf.div_(self.world)
-            for g, f in zip(rest, torch._utils._unflatten_dense_tensors(buf, rest)):
-                g.copy_(f)
+        allreduce_gradients([p for p in params if id(p) not in self.covered], self.world)
         for work, flat, pv_pairs in self.pending:
             work.wait()
             if not self.avg:
@@ -617,7 +610,7 @@ def stack_params(net) -> List[nn.Parameter]:
 def backbone_train_forward(net, x_t: torch.Tensor, t: torch.Tensor, a: torch.Tensor, seed: int,
                            dropout_p: float) -> torch.Tensor:
     """eps = AuxiliaryUNet(x_t, t, a) with autograd through the sm_100a kernels (reference models.py:296-326)."""
-    from .engine import BackbonePlan, conditioned_blocks
+    from .engine import BackbonePlan, conditioned_blocks, modulation_weights
     B = x_t.shape[0]
     plans = net._plans()
     key = ("train", B, x_t.device.index, float(dropout_p))
@@ -629,17 +622,11 @@ def backbone_train_forward(net, x_t: torch.Tensor, t: torch.Tensor, a: torch.Ten
     silu = torch.nn.functional.silu
     te = net.time_embedding.timembedding
     temb = L.apply(te[3], silu(L.apply(te[1], te[0].weight[t])))
-    blocks = conditioned_blocks(net)
-    w_t = torch.cat([b.temb_proj[1].weight for b in blocks], 0)
-    b_t = torch.cat([b.temb_proj[1].bias for b in blocks], 0)
+    w_t, b_t, w_z, b_z = modulation_weights(conditioned_blocks(net))
     mod_t = L.linear(silu(temb), w_t, b_t)
     if hasattr(net, "fc_a"):
         # Linear (AuxiliaryUNet) or SiLU -> Linear (BottleneckAuxUNet)
         aemb = L.apply(net.fc_a[1], silu(a)) if isinstance(net.fc_a, nn.Sequential) else L.apply(net.fc_a, a)
-        w_z = torch.cat([b.aemb_proj[1].weight if hasattr(b, "aemb_proj") else torch.zeros_like(b.temb_proj[1].weight)
-                         for b in blocks], 0)
-        b_z = torch.cat([b.aemb_proj[1].bias if hasattr(b, "aemb_proj") else torch.zeros_like(b.temb_proj[1].bias)
-                         for b in blocks], 0)
         mod_z = L.linear(silu(aemb), w_z, b_z)
     else:
         mod_z = torch.zeros_like(mod_t)          # UNet: no block reads it
