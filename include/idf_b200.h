@@ -11,6 +11,11 @@
  *  - every launcher is asynchronous on `stream`, allocates nothing, keeps no global state
  *    besides the plan objects the caller owns, and is CUDA-graph capturable.
  *  - return value: 0 on success, negative idf_status on error; idf_last_error() gives text.
+ *  - reductions whose order depends on arrival (split-K weight gradients, bias / GroupNorm-affine gradients, split-K
+ *    fp32 GEMM, MMD) have ORDERED variants: partials go to a caller-owned fp32 workspace and are combined in a fixed
+ *    index order (slab, block, sample, warp), so training is bitwise reproducible run to run.  Partition sizes follow the
+ *    SM count: results repeat on one GPU model, not across models.  Where a variant combines in the last-arriving CTA
+ *    it takes a ticket from caller-zeroed uint32 counters and leaves them zero again (CUDA-graph replays need no reset).
  *  - activations live in the "pad-flat" NHWC layout: image n, pixel (y,x), channel c of an
  *    H x W x C map is element ((n*(H+1) + y)*(W+1) + x)*C + c; row y==H and column x==W of every
  *    image are zero padding shared with the neighbouring row/image, so a 3x3 tap is a constant
@@ -142,7 +147,7 @@ int64_t idf_conv_plan_tiles(const idf_conv_plan* plan);
 int32_t idf_conv_plan_stats_unit(const idf_conv_plan* plan);
 
 /* ------------------------------------------------------------------------------------------
- * Convolution weight gradient (autograd of nn.Conv2d w.r.t. weight), tcgen05, split-K with atomics:
+ * Convolution weight gradient (autograd of nn.Conv2d w.r.t. weight), tcgen05, split-K with atomics (or ordered):
  *   dW[co, t, ci] += sum_r dY[r, co] * X[r + tap_off[t], ci]       dW fp32 [cout, n_taps, cin]
  * dY: bf16 pad-flat [rows, cout] (pad rows zero), X: bf16 [x_rows, cin] (cin multiple of 64).
  * The data gradient needs no kernel of its own: it is idf_conv_run over dY with transposed weights.
@@ -152,9 +157,14 @@ typedef struct {
   const void* x; int64_t x_rows; int32_t cin;
   int32_t n_taps; int32_t tap_off[9];
   float* dw;
+  /* optional: fp32 workspace of idf_wgrad_plan_partials_floats(plan) floats.  When set, every split-K slab stores its
+   * partial dW and a second launch adds the slabs to dw in slab order (bitwise reproducible); NULL = atomics.  Plans
+   * with one slab need none and add directly either way.  The pointer is captured by idf_wgrad_plan_create. */
+  float* partials;
 } idf_wgrad_desc;
 typedef struct idf_wgrad_plan idf_wgrad_plan;
 int idf_wgrad_plan_create(const idf_wgrad_desc* desc, idf_wgrad_plan** plan);
+int64_t idf_wgrad_plan_partials_floats(const idf_wgrad_plan* plan);   /* 0 for single-slab plans */
 int idf_wgrad_plan_destroy(idf_wgrad_plan* plan);
 int idf_wgrad_run(const idf_wgrad_plan* plan, idf_stream_t stream);
 
@@ -217,6 +227,9 @@ typedef struct {
    *   d_mod_t / d_mod_z : fp32 rows laid out like mod_t / mod_z of the forward args (same strides), receive
    *                       (d scale | d shift) of this op;  dgamma / dbeta : fp32 [C], accumulated (atomics) */
   float* d_mod_t; float* d_mod_z; float* dgamma; float* dbeta;
+  /* optional, ordered dgamma / dbeta: fp32 [batch, C, 2] workspace and one caller-zeroed uint32 ticket; the per-sample
+   * contributions are added in sample order instead of with atomics.  NULL = atomics. */
+  float* dparam_ws; uint32_t* dparam_ticket;
 } idf_adagn_bwd_args;
 int64_t idf_adagn_bwd_ws_floats(int32_t batch, int32_t C);
 int idf_adagn_silu_bwd(const idf_adagn_bwd_args* args, idf_stream_t stream);
@@ -252,6 +265,12 @@ int idf_linear_f32(const float* x, int64_t ldx, const float* w, const float* b, 
  * in the autograd graph of modules.py:24-27, 211, 271-275 and models.py:147-163, 223-234, 470-472. */
 int idf_gemm_f32(const float* A, int64_t lda, int32_t transA, const float* B, int64_t ldb, int32_t transB, float* C,
                  int64_t ldc, int32_t M, int32_t N, int32_t K, int32_t accumulate, idf_stream_t stream);
+/* Same result with split-K partial tiles combined in split order (bitwise reproducible): ws holds
+ * idf_gemm_f32_ws_floats(M, N, K) floats (0: no split, ws and tickets unused), tickets 64 caller-zeroed uint32. */
+int idf_gemm_f32_ordered(const float* A, int64_t lda, int32_t transA, const float* B, int64_t ldb, int32_t transB, float* C,
+                         int64_t ldc, int32_t M, int32_t N, int32_t K, int32_t accumulate, float* ws, uint32_t* tickets,
+                         idf_stream_t stream);
+int64_t idf_gemm_f32_ws_floats(int32_t M, int32_t N, int32_t K);
 
 /* y[m, :] = table[idx[m], :]  (nn.Embedding lookup, modules.py:23,37) */
 int idf_gather_rows_f32(const float* table, const int64_t* idx, float* y, int32_t M, int32_t N, idf_stream_t stream);
@@ -320,6 +339,11 @@ int idf_depth_to_space(const void* dphases, void* din, int32_t batch, int32_t H,
                        idf_stream_t stream);   /* H, W: full resolution; inverse of idf_space_to_depth */
 /* out[c] += sum_r m[r, c]  (bias gradient of a conv: column sums of dY), fp32 atomics */
 int idf_colsum_bf16(const void* m, float* out, int64_t rows, int32_t C, idf_stream_t stream);
+/* the same sum with the block partials added in block order: ws = idf_colsum_ws_floats(rows, C) floats, tickets = one
+ * caller-zeroed uint32 */
+int idf_colsum_bf16_ordered(const void* m, float* out, int64_t rows, int32_t C, float* ws, uint32_t* tickets,
+                            idf_stream_t stream);
+int64_t idf_colsum_ws_floats(int64_t rows, int32_t C);
 
 /* ------------------------------------------------------------------------------------------
  * Stand-alone sampler update (the unfused variant of IDF_EPI_SAMPLER):
@@ -335,6 +359,11 @@ int idf_sampler_update(float* x, const float* eps, const float* noise, const flo
  * ------------------------------------------------------------------------------------------ */
 int idf_mmd_fwd_bwd(const float* x, const float* y, float* loss, float* grad_y, int32_t B, int32_t D,
                     idf_stream_t stream);
+/* the same with grad_y summed per warp and the per-row loss partials summed in row order: ws = idf_mmd_ws_floats(B)
+ * floats, tickets = one caller-zeroed uint32 */
+int idf_mmd_fwd_bwd_ordered(const float* x, const float* y, float* loss, float* grad_y, int32_t B, int32_t D, float* ws,
+                            uint32_t* tickets, idf_stream_t stream);
+int64_t idf_mmd_ws_floats(int32_t B);
 
 #ifdef __cplusplus
 }

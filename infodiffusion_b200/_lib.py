@@ -54,6 +54,7 @@ class WgradDesc(C.Structure):
         ("x", C.c_void_p), ("x_rows", C.c_int64), ("cin", C.c_int32),
         ("n_taps", C.c_int32), ("tap_off", C.c_int32 * 9),
         ("dw", C.c_void_p),
+        ("partials", C.c_void_p),
     ]
 
 
@@ -98,6 +99,7 @@ class AdaGNBwdArgs(C.Structure):
         ("sums", C.c_void_p),
         ("ws", C.c_void_p),
         ("d_mod_t", C.c_void_p), ("d_mod_z", C.c_void_p), ("dgamma", C.c_void_p), ("dbeta", C.c_void_p),
+        ("dparam_ws", C.c_void_p), ("dparam_ticket", C.c_void_p),
     ]
 
 
@@ -115,6 +117,7 @@ SIGNATURES = {
     "idf_wgrad_plan_create": (C.c_int, [C.POINTER(WgradDesc), C.POINTER(C.c_void_p)]),
     "idf_wgrad_plan_destroy": (C.c_int, [C.c_void_p]),
     "idf_wgrad_run": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "idf_wgrad_plan_partials_floats": (C.c_int64, [C.c_void_p]),
     "idf_adagn_coef": (C.c_int, [C.POINTER(AdaGNArgs), C.c_void_p, C.c_void_p]),
     "idf_adagn_silu_fwd": (C.c_int, [C.POINTER(AdaGNArgs), C.c_void_p]),
     "idf_adagn_bwd_ws_floats": (C.c_int64, [C.c_int32, C.c_int32]),
@@ -128,6 +131,10 @@ SIGNATURES = {
                                  C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
     "idf_gemm_f32": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_int64,
                                C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
+    "idf_gemm_f32_ordered": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p,
+                                       C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
+                                       C.c_void_p]),
+    "idf_gemm_f32_ws_floats": (C.c_int64, [C.c_int32, C.c_int32, C.c_int32]),
     "idf_scale_layernorm_silu": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p,
                                            C.c_void_p, C.c_float, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_int32,
                                            C.c_void_p]),
@@ -151,10 +158,16 @@ SIGNATURES = {
     "idf_depth_to_space": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                      C.c_void_p]),
     "idf_colsum_bf16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p]),
+    "idf_colsum_bf16_ordered": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p,
+                                          C.c_void_p]),
+    "idf_colsum_ws_floats": (C.c_int64, [C.c_int64, C.c_int32]),
     "idf_sampler_update": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
                                      C.c_void_p]),
     "idf_mmd_fwd_bwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32,
                                   C.c_void_p]),
+    "idf_mmd_fwd_bwd_ordered": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32,
+                                          C.c_void_p, C.c_void_p, C.c_void_p]),
+    "idf_mmd_ws_floats": (C.c_int64, [C.c_int32]),
 }
 
 _lib = None

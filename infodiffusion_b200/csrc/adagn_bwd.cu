@@ -7,7 +7,9 @@
 //     dx = A_c dv - rstd_g / cnt * ( G1_g + xhat * G2_g ),   G1_g = sum_{c in g} g_c S1,  G2_g = sum g_c S2
 // and every parameter / modulation gradient of the op is a closed form of (S1, S2) (done by the host
 // side on [B, C] tensors).  Two sweeps: `stats` accumulates per-slice (S1, S2) partials, `apply` folds them
-// in a fixed order (deterministic) and writes dx (optionally accumulating into an existing gradient).
+// in a fixed order (deterministic) and writes dx (optionally accumulating into an existing gradient).  The fused
+// dgamma / dbeta sums over the batch are atomics, or (ordered variant, dparam_ws given) per-sample rows that the last
+// sample's CTA adds in sample order.
 // The forward statistics come from the producing conv's window records, as in the forward kernel.
 #include "kernels.cuh"
 
@@ -35,6 +37,7 @@ struct AdaGNBwdParams {
   float* d_mod_t; float* d_mod_z; float* dgamma; float* dbeta;
   int slice_rows;
   int n_slices;
+  float* dparam_ws; unsigned* dparam_ticket;   // ordered dgamma / dbeta: per-sample rows summed in sample order
 };
 
 constexpr int kUn = 2;            // rows in flight per thread (more would cost occupancy: 4 CTAs/SM at <= 64 registers)
@@ -218,7 +221,7 @@ __global__ void __launch_bounds__(kBT, kBwdMinCtas<kMaxC>) adagn_bwd_stats_kerne
   }
 }
 
-template <int kMaxC>
+template <int kMaxC, bool kOrdered>
 __global__ void __launch_bounds__(kBT, kBwdMinCtas<kMaxC>) adagn_bwd_apply_kernel(const AdaGNBwdParams p) {
   __shared__ BwdShared<kMaxC> sh;
   __shared__ float s_S[2 * kMaxC];
@@ -257,8 +260,33 @@ __global__ void __launch_bounds__(kBT, kBwdMinCtas<kMaxC>) adagn_bwd_apply_kerne
       if (p.mod_z != nullptr) Z = 1.f + p.mod_z[off_z + ch];
       if (p.d_mod_t != nullptr) { p.d_mod_t[off_t + ch] = Z * q; p.d_mod_t[off_t + C + ch] = Z * S1; }
       if (p.d_mod_z != nullptr) { p.d_mod_z[off_z + ch] = T * q + bt * S1; p.d_mod_z[off_z + C + ch] = S1; }
-      if (p.dgamma != nullptr) atomicAdd(p.dgamma + ch, T * Z * S2);
-      if (p.dbeta != nullptr) atomicAdd(p.dbeta + ch, T * Z * S1);
+      if constexpr (kOrdered) {
+        p.dparam_ws[(static_cast<long long>(n) * C + ch) * 2] = T * Z * S2;
+        p.dparam_ws[(static_cast<long long>(n) * C + ch) * 2 + 1] = T * Z * S1;
+      } else {
+        if (p.dgamma != nullptr) atomicAdd(p.dgamma + ch, T * Z * S2);
+        if (p.dbeta != nullptr) atomicAdd(p.dbeta + ch, T * Z * S1);
+      }
+    }
+    if constexpr (kOrdered) {               // the last of the batch's slice-0 CTAs adds the rows in sample order
+      __shared__ bool last;
+      __threadfence();
+      __syncthreads();
+      if (t == 0) last = atomicAdd(p.dparam_ticket, 1u) == gridDim.y - 1;
+      __syncthreads();
+      if (last) {
+        __threadfence();
+        for (int ch = t; ch < C; ch += kBT) {
+          float sg = 0.f, sb = 0.f;
+          for (unsigned b = 0; b < gridDim.y; ++b) {
+            const float2 v = __ldcg(reinterpret_cast<const float2*>(p.dparam_ws) + static_cast<long long>(b) * C + ch);
+            sg += v.x; sb += v.y;
+          }
+          if (p.dgamma != nullptr) p.dgamma[ch] += sg;
+          if (p.dbeta != nullptr) p.dbeta[ch] += sb;
+        }
+        if (t == 0) *p.dparam_ticket = 0u;
+      }
     }
   }
   if (t < 32) {
@@ -353,6 +381,9 @@ cudaError_t launch_adagn_bwd(const idf_adagn_bwd_args& b, int num_sms, cudaStrea
   p.dx0 = static_cast<bf16*>(b.dx0); p.dx1 = static_cast<bf16*>(b.dx1); p.acc0 = b.acc0; p.acc1 = b.acc1;
   p.sums = b.sums; p.ws = b.ws; p.save_coef = a.save_coef;
   p.d_mod_t = b.d_mod_t; p.d_mod_z = b.d_mod_z; p.dgamma = b.dgamma; p.dbeta = b.dbeta;
+  p.dparam_ws = b.dparam_ws; p.dparam_ticket = b.dparam_ticket;
+  const bool ordered = p.dparam_ws != nullptr && (p.dgamma != nullptr || p.dbeta != nullptr);
+  if (p.dparam_ws != nullptr && p.dparam_ticket == nullptr) return cudaErrorInvalidValue;
   if (p.C > kBMaxCWide || p.C % 32 != 0 || p.c0 % 8 != 0 || p.c1 % 8 != 0 || a.batch <= 0) return cudaErrorInvalidValue;
   if (p.stats0 == nullptr || (p.c1 != 0 && (p.stats1 == nullptr || p.dx1 == nullptr)) || p.dx0 == nullptr ||
       p.dy == nullptr || p.sums == nullptr || p.ws == nullptr)
@@ -369,8 +400,11 @@ cudaError_t launch_adagn_bwd(const idf_adagn_bwd_args& b, int num_sms, cudaStrea
   cudaError_t e = launch_kernel(wide ? adagn_bwd_stats_kernel<kBMaxCWide> : adagn_bwd_stats_kernel<kBMaxC>, grid, dim3(kBT),
                                 0, stream, g_pdl != 0, 0, p);
   if (e != cudaSuccess) return e;
-  return launch_kernel(wide ? adagn_bwd_apply_kernel<kBMaxCWide> : adagn_bwd_apply_kernel<kBMaxC>, grid, dim3(kBT), 0,
-                       stream, g_pdl != 0, 0, p);
+  if (ordered)
+    return launch_kernel(wide ? adagn_bwd_apply_kernel<kBMaxCWide, true> : adagn_bwd_apply_kernel<kBMaxC, true>, grid,
+                         dim3(kBT), 0, stream, g_pdl != 0, 0, p);
+  return launch_kernel(wide ? adagn_bwd_apply_kernel<kBMaxCWide, false> : adagn_bwd_apply_kernel<kBMaxC, false>, grid,
+                       dim3(kBT), 0, stream, g_pdl != 0, 0, p);
 }
 
 }  // namespace idf

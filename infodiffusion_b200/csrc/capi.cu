@@ -330,6 +330,7 @@ int idf_conv_run(const idf_conv_plan* plan, idf_stream_t stream) {
 struct idf_wgrad_plan {
   WgradKernelParams params;
   int grid;
+  int slabs;
 };
 
 int idf_wgrad_plan_create(const idf_wgrad_desc* d, idf_wgrad_plan** out_plan) {
@@ -372,13 +373,19 @@ int idf_wgrad_plan_create(const idf_wgrad_desc* d, idf_wgrad_plan** out_plan) {
   if (slabs < 1) slabs = 1;
   p.kb_per_slab = (p.n_kb + slabs - 1) / slabs;
   slabs = (p.n_kb + p.kb_per_slab - 1) / p.kb_per_slab;
-  p.cout = d->cout; p.cin = d->cin; p.ntaps = d->n_taps; p.dw = d->dw;
+  p.cout = d->cout; p.cin = d->cin; p.ntaps = d->n_taps; p.dw = d->dw; p.partials = d->partials;
   rc = encode_2d(&p.tmDY, d->dy, d->rows, d->cout, 128);
   if (rc == IDF_OK) rc = encode_2d(&p.tmX, d->x, d->x_rows, d->cin, 136);
   if (rc != IDF_OK) { delete pl; return rc; }
   pl->grid = p.n_units * slabs;
+  pl->slabs = slabs;
   *out_plan = pl;
   return IDF_OK;
+}
+
+int64_t idf_wgrad_plan_partials_floats(const idf_wgrad_plan* plan) {
+  if (plan == nullptr || plan->slabs < 2) return 0;
+  return static_cast<int64_t>(plan->slabs) * plan->params.cout * plan->params.ntaps * plan->params.cin;
 }
 
 int idf_wgrad_plan_destroy(idf_wgrad_plan* plan) {
@@ -388,7 +395,7 @@ int idf_wgrad_plan_destroy(idf_wgrad_plan* plan) {
 
 int idf_wgrad_run(const idf_wgrad_plan* plan, idf_stream_t stream) {
   if (plan == nullptr) return fail(IDF_ERR_ARG, "null plan");
-  cudaError_t e = launch_wgrad(plan->params, plan->grid, reinterpret_cast<cudaStream_t>(stream));
+  cudaError_t e = launch_wgrad(plan->params, plan->grid, plan->slabs, g_num_sms, reinterpret_cast<cudaStream_t>(stream));
   if (e != cudaSuccess) return cuda_fail(e, "wgrad launch");
   return IDF_OK;
 }
@@ -492,6 +499,20 @@ int idf_gemm_f32(const float* A, int64_t lda, int32_t transA, const float* B, in
   cudaError_t e = launch_gemm_f32(A, lda, transA, B, ldb, transB, Cm, ldc, M, N, K, accumulate, reinterpret_cast<cudaStream_t>(stream));
   if (e != cudaSuccess) return cuda_fail(e, "gemm_f32 launch");
   return IDF_OK;
+}
+
+int idf_gemm_f32_ordered(const float* A, int64_t lda, int32_t transA, const float* B, int64_t ldb, int32_t transB, float* Cm,
+                         int64_t ldc, int32_t M, int32_t N, int32_t K, int32_t accumulate, float* ws, uint32_t* tickets,
+                         idf_stream_t stream) {
+  if (A == nullptr || B == nullptr || Cm == nullptr || M <= 0 || N <= 0 || K <= 0) return fail(IDF_ERR_ARG, "bad gemm arguments");
+  cudaError_t e = launch_gemm_f32_ordered(A, lda, transA, B, ldb, transB, Cm, ldc, M, N, K, accumulate, ws, tickets,
+                                          reinterpret_cast<cudaStream_t>(stream));
+  if (e != cudaSuccess) return cuda_fail(e, "gemm_f32 (ordered) launch (split-K shapes need ws and tickets)");
+  return IDF_OK;
+}
+
+int64_t idf_gemm_f32_ws_floats(int32_t M, int32_t N, int32_t K) {
+  return (M <= 0 || N <= 0 || K <= 0) ? 0 : gemm_f32_ws_floats(M, N, K);
 }
 
 int idf_gather_rows_f32(const float* table, const int64_t* idx, float* y, int32_t M, int32_t N, idf_stream_t stream) {
@@ -613,6 +634,21 @@ int idf_colsum_bf16(const void* m, float* out, int64_t rows, int32_t C, idf_stre
   return IDF_OK;
 }
 
+int idf_colsum_bf16_ordered(const void* m, float* out, int64_t rows, int32_t C, float* ws, uint32_t* tickets,
+                            idf_stream_t stream) {
+  int rc = ensure_init();
+  if (rc != IDF_OK) return rc;
+  cudaError_t e = launch_colsum_ordered(static_cast<const bf16*>(m), out, rows, C, g_num_sms, ws, tickets,
+                                        reinterpret_cast<cudaStream_t>(stream));
+  if (e != cudaSuccess) return cuda_fail(e, "colsum (ordered) launch");
+  return IDF_OK;
+}
+
+int64_t idf_colsum_ws_floats(int64_t rows, int32_t C) {
+  if (ensure_init() != IDF_OK) return 0;
+  return colsum_ws_floats(rows, C, g_num_sms);
+}
+
 int idf_padflat_to_nchw(const void* in, float* y, int32_t batch, int32_t C, int32_t H, int32_t W,
                         idf_stream_t stream) {
   cudaError_t e = launch_padflat_to_nchw(static_cast<const bf16*>(in), y, batch, C, H, W, reinterpret_cast<cudaStream_t>(stream));
@@ -638,5 +674,16 @@ int idf_mmd_fwd_bwd(const float* x, const float* y, float* loss, float* grad_y, 
   if (e != cudaSuccess) return cuda_fail(e, "mmd launch");
   return IDF_OK;
 }
+
+int idf_mmd_fwd_bwd_ordered(const float* x, const float* y, float* loss, float* grad_y, int32_t B, int32_t D, float* ws,
+                            uint32_t* tickets, idf_stream_t stream) {
+  if (x == nullptr || y == nullptr || loss == nullptr || ws == nullptr || tickets == nullptr || B <= 0 || D <= 0 || D > 4096)
+    return fail(IDF_ERR_ARG, "bad mmd arguments");
+  cudaError_t e = launch_mmd_ordered(x, y, loss, grad_y, B, D, ws, tickets, reinterpret_cast<cudaStream_t>(stream));
+  if (e != cudaSuccess) return cuda_fail(e, "mmd (ordered) launch");
+  return IDF_OK;
+}
+
+int64_t idf_mmd_ws_floats(int32_t B) { return B > 0 ? B : 0; }
 
 }  // extern "C"

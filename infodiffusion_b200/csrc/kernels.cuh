@@ -72,8 +72,10 @@ struct alignas(64) WgradKernelParams {
   int32_t n_kb, kb_per_slab;
   int32_t cout, cin, ntaps;
   float* dw;                        // fp32 [Cout, ntaps, Cin], accumulated with atomics
+  float* partials;                  // ordered variant: fp32 [slabs][Cout, ntaps, Cin], reduced into dw in slab order
 };
-cudaError_t launch_wgrad(const WgradKernelParams& p, int grid, cudaStream_t stream);
+// partials == nullptr or a single slab: one launch; otherwise the ordered kernel and the slab reduction
+cudaError_t launch_wgrad(const WgradKernelParams& p, int grid, int slabs, int num_sms, cudaStream_t stream);
 
 static_assert(sizeof(ConvKernelParams) <= 4000, "kernel parameters are limited to 4 KB");
 
@@ -155,6 +157,17 @@ cudaError_t launch_nchw_to_padflat(const float* x, bf16* out, int batch, int C, 
 cudaError_t launch_upsample2x_bwd(const bf16* dout, bf16* din, int batch, int H, int W, int C, int accumulate, cudaStream_t stream);
 cudaError_t launch_depth_to_space(const bf16* dph, bf16* din, int batch, int H, int W, int C, int accumulate, cudaStream_t stream);
 cudaError_t launch_colsum(const bf16* m, float* out, long long rows, int C, int num_sms, cudaStream_t stream);
+// ordered variants (torch's deterministic mode): partials in `ws`, combined in index order by the last-arriving CTA, which
+// takes a ticket from the caller-zeroed `tickets` and resets it to zero
+int64_t colsum_ws_floats(long long rows, int C, int num_sms);
+cudaError_t launch_colsum_ordered(const bf16* m, float* out, long long rows, int C, int num_sms, float* ws, unsigned* tickets,
+                                  cudaStream_t stream);
+int64_t gemm_f32_ws_floats(int M, int N, int K);
+cudaError_t launch_gemm_f32_ordered(const float* A, int64_t lda, int transA, const float* B, int64_t ldb, int transB, float* Cm,
+                                    int64_t ldc, int M, int N, int K, int accumulate, float* ws, unsigned* tickets,
+                                    cudaStream_t stream);
+cudaError_t launch_mmd_ordered(const float* x, const float* y, float* loss, float* grad_y, int B, int D, float* ws,
+                               unsigned* tickets, cudaStream_t stream);
 cudaError_t launch_padflat_to_nchw(const bf16* in, float* y, int batch, int C, int H, int W, cudaStream_t stream);
 cudaError_t launch_sampler_update(float* x, const float* eps, const float* noise, const float* coef,
                                   const int32_t* step_ptr, int64_t n, cudaStream_t stream);

@@ -256,9 +256,11 @@ cudaError_t launch_depth_to_space(const bf16* dph, bf16* din, int batch, int H, 
 
 // bias gradient: out[c] += sum_r m[r, c]   (m bf16 [rows, C], C % 8 == 0, C <= 2048).  Thread = one 16-byte
 // granule (8 channels) of every rpp-th row, four rows in flight; block partials combined in shared memory,
-// one atomicAdd per channel and block.
+// one atomicAdd per channel and block.  Ordered: the block partials go to ws[block][C] and the last-arriving block
+// adds them to out in block order.
+template <bool kOrdered>
 __global__ void __launch_bounds__(256) colsum_kernel(const bf16* __restrict__ m, float* __restrict__ out, long long rows,
-                                                     int C) {
+                                                     int C, float* __restrict__ ws, unsigned* __restrict__ tickets) {
   __shared__ float red[256][9];
   const int VPR = C >> 3, rpp = 256 / VPR;
   const int t = threadIdx.x, vl = t % VPR, rsub = t / VPR;
@@ -287,16 +289,46 @@ __global__ void __launch_bounds__(256) colsum_kernel(const bf16* __restrict__ m,
     const int cvl = ch >> 3, j = ch & 7;
     float sum = 0.f;
     for (int rs = 0; rs < rpp; ++rs) sum += red[rs * VPR + cvl][j];
-    atomicAdd(out + ch, sum);
+    if constexpr (kOrdered) ws[static_cast<long long>(blockIdx.x) * C + ch] = sum;
+    else atomicAdd(out + ch, sum);
+  }
+  if constexpr (kOrdered) {
+    __shared__ bool last;
+    __threadfence();
+    __syncthreads();
+    if (t == 0) last = atomicAdd(tickets, 1u) == gridDim.x - 1;
+    __syncthreads();
+    if (!last) return;
+    __threadfence();
+    for (int ch = t; ch < C; ch += 256) {
+      float sum = 0.f;
+      for (unsigned b = 0; b < gridDim.x; ++b) sum += __ldcg(ws + static_cast<long long>(b) * C + ch);
+      out[ch] += sum;
+    }
+    if (t == 0) *tickets = 0u;
   }
 }
-cudaError_t launch_colsum(const bf16* m, float* out, long long rows, int C, int num_sms, cudaStream_t stream) {
-  if (C % 8 || C > 2048 || C <= 0) return cudaErrorInvalidValue;
+static long long colsum_grid(long long rows, int C, int num_sms) {
   const int rpp = 256 / (C / 8);
   long long grid = (rows + 16ll * rpp - 1) / (16ll * rpp);          // >= 16 rows per thread
   if (grid > 4ll * num_sms) grid = 4ll * num_sms;
   if (grid < 1) grid = 1;
-  colsum_kernel<<<static_cast<unsigned>(grid), 256, 0, stream>>>(m, out, rows, C);
+  return grid;
+}
+cudaError_t launch_colsum(const bf16* m, float* out, long long rows, int C, int num_sms, cudaStream_t stream) {
+  if (C % 8 || C > 2048 || C <= 0) return cudaErrorInvalidValue;
+  colsum_kernel<false><<<static_cast<unsigned>(colsum_grid(rows, C, num_sms)), 256, 0, stream>>>(m, out, rows, C, nullptr,
+                                                                                                nullptr);
+  return cudaGetLastError();
+}
+int64_t colsum_ws_floats(long long rows, int C, int num_sms) {
+  if (C % 8 || C > 2048 || C <= 0) return 0;
+  return colsum_grid(rows, C, num_sms) * C;
+}
+cudaError_t launch_colsum_ordered(const bf16* m, float* out, long long rows, int C, int num_sms, float* ws, unsigned* tickets,
+                                  cudaStream_t stream) {
+  if (C % 8 || C > 2048 || C <= 0 || ws == nullptr || tickets == nullptr) return cudaErrorInvalidValue;
+  colsum_kernel<true><<<static_cast<unsigned>(colsum_grid(rows, C, num_sms)), 256, 0, stream>>>(m, out, rows, C, ws, tickets);
   return cudaGetLastError();
 }
 
@@ -449,10 +481,11 @@ cudaError_t launch_linear_f32(const float* x, int64_t ldx, const float* w, const
 // accumulators per thread, K in chunks of 16 staged k-major; fixed fp32 FMA order over k (deterministic).  These GEMMs
 // are tiny (M = batch <= 1024, N, K <= 8192) and weight-bandwidth bound: tensor cores would not help (fp32 operands).
 // ----------------------------------------------------------------------------------------------
+template <bool kOrdered>
 __global__ void __launch_bounds__(256) gemm_f32_kernel(const float* __restrict__ A, long long lda, int transA,
                                                        const float* __restrict__ B, long long ldb, int transB,
                                                        float* __restrict__ Cm, long long ldc, int M, int N, int K,
-                                                       int accumulate) {
+                                                       int accumulate, float* __restrict__ ws, unsigned* __restrict__ tickets) {
   __shared__ __align__(16) float as[16][68];
   __shared__ __align__(16) float bs[16][68];
   const int m0 = blockIdx.y * 64, n0 = blockIdx.x * 64;
@@ -461,6 +494,8 @@ __global__ void __launch_bounds__(256) gemm_f32_kernel(const float* __restrict__
   float acc[4][4] = {};
   // split-K: blockIdx.z owns the k range [kb, ke); partial tiles are combined with atomicAdd (C pre-zeroed by the
   // launcher).  Used when M x N alone gives too few CTAs (dX of a [batch, 4992] x [4992, 256] Linear: 4 tiles, K = 4992).
+  // Ordered: each split stores its 64x64 partial tile to ws[tile][split]; the last split to arrive at a tile sums them
+  // in split order.
   const int kchunk = ((K + gridDim.z - 1) / gridDim.z + 15) / 16 * 16;
   const int kb = blockIdx.z * kchunk, ke = min(K, kb + kchunk);
   for (int k0 = kb; k0 < ke; k0 += 16) {
@@ -489,6 +524,33 @@ __global__ void __launch_bounds__(256) gemm_f32_kernel(const float* __restrict__
     }
     __syncthreads();
   }
+  if constexpr (kOrdered) {
+    if (gridDim.z > 1) {
+      const unsigned tile = blockIdx.y * gridDim.x + blockIdx.x;
+      float* part = ws + static_cast<long long>(tile) * gridDim.z * 4096;
+#pragma unroll
+      for (int i = 0; i < 4; ++i)
+        *reinterpret_cast<float4*>(part + blockIdx.z * 4096 + (tm + i) * 64 + tn) =
+            make_float4(acc[i][0], acc[i][1], acc[i][2], acc[i][3]);
+      __shared__ bool last;
+      __threadfence();
+      __syncthreads();
+      if (t == 0) last = atomicAdd(tickets + tile, 1u) == gridDim.z - 1;
+      __syncthreads();
+      if (!last) return;
+      __threadfence();
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        float4 v = __ldcg(reinterpret_cast<const float4*>(part + (tm + i) * 64 + tn));
+        for (unsigned z = 1; z < gridDim.z; ++z) {
+          const float4 u = __ldcg(reinterpret_cast<const float4*>(part + z * 4096 + (tm + i) * 64 + tn));
+          v.x += u.x; v.y += u.y; v.z += u.z; v.w += u.w;
+        }
+        acc[i][0] = v.x; acc[i][1] = v.y; acc[i][2] = v.z; acc[i][3] = v.w;
+      }
+      if (t == 0) tickets[tile] = 0u;
+    }
+  }
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
     const int m = m0 + tm + i;
@@ -498,23 +560,28 @@ __global__ void __launch_bounds__(256) gemm_f32_kernel(const float* __restrict__
       const int n = n0 + tn + j;
       if (n < N) {
         float* dst = Cm + static_cast<long long>(m) * ldc + n;
-        if (gridDim.z > 1) atomicAdd(dst, acc[i][j]);
+        if (!kOrdered && gridDim.z > 1) atomicAdd(dst, acc[i][j]);
         else *dst = accumulate ? *dst + acc[i][j] : acc[i][j];
       }
     }
   }
 }
 
-cudaError_t launch_gemm_f32(const float* A, int64_t lda, int transA, const float* B, int64_t ldb, int transB, float* Cm,
-                            int64_t ldc, int M, int N, int K, int accumulate, cudaStream_t stream) {
-  dim3 grid((N + 63) / 64, (M + 63) / 64, 1);
-  const int tiles = static_cast<int>(grid.x * grid.y);
+static int gemm_f32_splits(int M, int N, int K) {
+  const int tiles = ((N + 63) / 64) * ((M + 63) / 64);
   int splits = 1;
   if (tiles < 64 && K >= 512) {                       // too few tiles to fill the machine and a long K loop
     splits = 148 / tiles;
     if (splits > K / 128) splits = K / 128;
     if (splits < 1) splits = 1;
   }
+  return splits;
+}
+
+cudaError_t launch_gemm_f32(const float* A, int64_t lda, int transA, const float* B, int64_t ldb, int transB, float* Cm,
+                            int64_t ldc, int M, int N, int K, int accumulate, cudaStream_t stream) {
+  dim3 grid((N + 63) / 64, (M + 63) / 64, 1);
+  const int splits = gemm_f32_splits(M, N, K);
   if (splits > 1) {
     grid.z = splits;
     if (!accumulate) {                                // the partial tiles are added atomically
@@ -527,7 +594,22 @@ cudaError_t launch_gemm_f32(const float* A, int64_t lda, int transA, const float
       }
     }
   }
-  gemm_f32_kernel<<<grid, 256, 0, stream>>>(A, lda, transA, B, ldb, transB, Cm, ldc, M, N, K, accumulate);
+  gemm_f32_kernel<false><<<grid, 256, 0, stream>>>(A, lda, transA, B, ldb, transB, Cm, ldc, M, N, K, accumulate, nullptr,
+                                                   nullptr);
+  return cudaGetLastError();
+}
+
+int64_t gemm_f32_ws_floats(int M, int N, int K) {
+  const int splits = gemm_f32_splits(M, N, K);
+  return splits > 1 ? static_cast<int64_t>((N + 63) / 64) * ((M + 63) / 64) * splits * 4096 : 0;
+}
+
+cudaError_t launch_gemm_f32_ordered(const float* A, int64_t lda, int transA, const float* B, int64_t ldb, int transB, float* Cm,
+                                    int64_t ldc, int M, int N, int K, int accumulate, float* ws, unsigned* tickets,
+                                    cudaStream_t stream) {
+  dim3 grid((N + 63) / 64, (M + 63) / 64, gemm_f32_splits(M, N, K));
+  if (grid.z > 1 && (ws == nullptr || tickets == nullptr)) return cudaErrorInvalidValue;
+  gemm_f32_kernel<true><<<grid, 256, 0, stream>>>(A, lda, transA, B, ldb, transB, Cm, ldc, M, N, K, accumulate, ws, tickets);
   return cudaGetLastError();
 }
 
@@ -690,14 +772,17 @@ cudaError_t launch_gather_elems(const float* src, const int* idx, const int* idx
 // MMD (utils.py:74-90): loss = mean k(x,x) + mean k(y,y) - 2 mean k(x,y), k(u,v)=exp(-|u-v|^2/D^2)
 // One block per column index j: accumulates sum_i [k(x_i,x_j) + k(y_i,y_j) - 2 k(x_i,y_j)] and
 // d loss / d y_j.  The per-block partial is added to *loss with one atomicAdd (loss must be zeroed).
+// Ordered: every warp accumulates d loss / d y_j in a shared row of its own (the rows are summed in warp order), the
+// per-block partials go to ws[j], and the last-arriving block sums them in block order.
 // ----------------------------------------------------------------------------------------------
+template <bool kOrdered>
 __global__ void __launch_bounds__(128) mmd_kernel(const float* __restrict__ x, const float* __restrict__ y,
                                                   float* __restrict__ loss, float* __restrict__ grad_y, int B,
-                                                  int D) {
+                                                  int D, float* __restrict__ ws, unsigned* __restrict__ tickets) {
   extern __shared__ float sm[];
   float* xj = sm;            // [D]
   float* yj = sm + D;        // [D]
-  float* gacc = sm + 2 * D;  // [D]
+  float* gacc = sm + 2 * D;  // [D] ([4][D] ordered)
   __shared__ float red[4];
   const int j = blockIdx.x;
   const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
@@ -705,6 +790,7 @@ __global__ void __launch_bounds__(128) mmd_kernel(const float* __restrict__ x, c
     xj[d] = x[static_cast<long long>(j) * D + d];
     yj[d] = y[static_cast<long long>(j) * D + d];
     gacc[d] = 0.f;
+    if constexpr (kOrdered) gacc[D + d] = gacc[2 * D + d] = gacc[3 * D + d] = 0.f;
   }
   __syncthreads();
   const float inv_d2 = 1.0f / (static_cast<float>(D) * static_cast<float>(D));
@@ -736,22 +822,62 @@ __global__ void __launch_bounds__(128) mmd_kernel(const float* __restrict__ x, c
       const float cxy = 4.0f * kxy * inv_d2 * inv_b2;
       for (int d = lane; d < D; d += 32) {
         const float g = cy * (yj[d] - yi[d]) + cxy * (yj[d] - xi[d]);
-        atomicAdd(&gacc[d], g);
+        if constexpr (kOrdered) gacc[warp * D + d] += g;      // this lane owns element d of its warp's row
+        else atomicAdd(&gacc[d], g);
       }
     }
   }
   if (lane == 0) red[warp] = part;
   __syncthreads();
-  if (t == 0) atomicAdd(loss, (red[0] + red[1] + red[2] + red[3]) * inv_b2);
-  if (grad_y != nullptr)
-    for (int d = t; d < D; d += 128) grad_y[static_cast<long long>(j) * D + d] = gacc[d];
+  if constexpr (kOrdered) {
+    if (t == 0) ws[j] = (red[0] + red[1] + red[2] + red[3]) * inv_b2;
+    if (grad_y != nullptr)
+      for (int d = t; d < D; d += 128)
+        grad_y[static_cast<long long>(j) * D + d] = (gacc[d] + gacc[D + d]) + (gacc[2 * D + d] + gacc[3 * D + d]);
+    __shared__ bool last;
+    __threadfence();
+    __syncthreads();
+    if (t == 0) last = atomicAdd(tickets, 1u) == gridDim.x - 1;
+    __syncthreads();
+    if (!last) return;
+    __threadfence();
+    float s = 0.f;                                          // fixed order: thread t sums blocks t, t + 128, ...
+    for (int b = t; b < B; b += 128) s += __ldcg(ws + b);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    __syncthreads();
+    if (lane == 0) red[warp] = s;
+    __syncthreads();
+    if (t == 0) {
+      *loss = (red[0] + red[1]) + (red[2] + red[3]);
+      *tickets = 0u;
+    }
+  } else {
+    if (t == 0) atomicAdd(loss, (red[0] + red[1] + red[2] + red[3]) * inv_b2);
+    if (grad_y != nullptr)
+      for (int d = t; d < D; d += 128) grad_y[static_cast<long long>(j) * D + d] = gacc[d];
+  }
 }
 
 cudaError_t launch_mmd(const float* x, const float* y, float* loss, float* grad_y, int B, int D,
                        cudaStream_t stream) {
   cudaError_t e = cudaMemsetAsync(loss, 0, sizeof(float), stream);
   if (e != cudaSuccess) return e;
-  mmd_kernel<<<B, 128, 3 * D * sizeof(float), stream>>>(x, y, loss, grad_y, B, D);
+  mmd_kernel<false><<<B, 128, 3 * D * sizeof(float), stream>>>(x, y, loss, grad_y, B, D, nullptr, nullptr);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_mmd_ordered(const float* x, const float* y, float* loss, float* grad_y, int B, int D, float* ws,
+                               unsigned* tickets, cudaStream_t stream) {
+  if (ws == nullptr || tickets == nullptr) return cudaErrorInvalidValue;
+  const int smem = 6 * D * static_cast<int>(sizeof(float));
+  static bool attr_set = false;
+  if (!attr_set) {
+    cudaError_t e = cudaFuncSetAttribute(mmd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 6 * 4096 * 4);
+    if (e != cudaSuccess) return e;
+    attr_set = true;
+  }
+  mmd_kernel<true><<<B, 128, smem, stream>>>(x, y, loss, grad_y, B, D, ws, tickets);
   return cudaGetLastError();
 }
 

@@ -10,7 +10,9 @@
 //
 // Work unit = (128-wide co tile, <=128-wide ci chunk, cluster of <=3 taps, slab of K blocks): accumulators
 // (<= 3 x 128 fp32 columns) stay in TMEM for the whole slab, then are added to the global fp32 dW with
-// red.global.add (split-K across slabs; summation order across slabs is not deterministic).
+// red.global.add (split-K across slabs; summation order across slabs is not deterministic).  The ordered variant
+// (torch's deterministic mode) stores each slab's tile into its own dW-shaped slice of a partials buffer instead, and
+// wgrad_reduce_kernel adds the slices to dW in slab order.
 #include "kernels.cuh"
 
 namespace idf {
@@ -29,6 +31,7 @@ __device__ __forceinline__ uint64_t umma_desc_mn(uint32_t smem_addr, uint32_t lb
   return d;
 }
 
+template <bool kOrdered>
 __global__ void __launch_bounds__(192, 1) wgrad_kernel(const __grid_constant__ WgradKernelParams p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -132,7 +135,16 @@ __global__ void __launch_bounds__(192, 1) wgrad_kernel(const __grid_constant__ W
           tmem_ld_32x32(tmem + lane_addr + static_cast<uint32_t>(t * ci_n + c), v);
           tmem_ld_wait();
           if (co < p.cout) {
-            float* dst = p.dw + (static_cast<int64_t>(co) * p.ntaps + tap) * p.cin + ci0 + c;
+            const int64_t e = (static_cast<int64_t>(co) * p.ntaps + tap) * p.cin + ci0 + c;
+            if constexpr (kOrdered) {
+              float4* dst = reinterpret_cast<float4*>(p.partials + static_cast<int64_t>(slab) * p.cout * p.ntaps * p.cin + e);
+#pragma unroll
+              for (int j = 0; j < 8; ++j)
+                dst[j] = make_float4(__uint_as_float(v[4 * j]), __uint_as_float(v[4 * j + 1]), __uint_as_float(v[4 * j + 2]),
+                                     __uint_as_float(v[4 * j + 3]));
+              continue;
+            }
+            float* dst = p.dw + e;
 #pragma unroll
             for (int j = 0; j < 8; ++j)      // 16-byte vector reductions: 8 instead of 32 atomics per lane and chunk
               asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst + 4 * j), "f"(__uint_as_float(v[4 * j])),
@@ -152,15 +164,44 @@ __global__ void __launch_bounds__(192, 1) wgrad_kernel(const __grid_constant__ W
   }
 }
 
-cudaError_t launch_wgrad(const WgradKernelParams& p, int grid, cudaStream_t stream) {
-  constexpr uint32_t SMEM = kWgStages * (2 * kWgKB * 128 + 2 * (kWgKB + kWgHalo) * 128) + 128 + 1024;
-  static bool attr_set = false;
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(SMEM));
-    if (e != cudaSuccess) return e;
-    attr_set = true;
+// dW[e] += partials[0][e] + partials[1][e] + ... (slab order), one float4 of dW per thread
+__global__ void __launch_bounds__(256) wgrad_reduce_kernel(const float4* __restrict__ partials, float4* __restrict__ dw,
+                                                           long long n4, int slabs) {
+  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < n4;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    float4 s = __ldg(partials + i);
+    for (int k = 1; k < slabs; ++k) {
+      const float4 v = __ldg(partials + k * n4 + i);
+      s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
+    }
+    float4 d = dw[i];
+    d.x += s.x; d.y += s.y; d.z += s.z; d.w += s.w;
+    dw[i] = d;
   }
-  wgrad_kernel<<<grid, 192, SMEM, stream>>>(p);
+}
+
+cudaError_t launch_wgrad(const WgradKernelParams& p, int grid, int slabs, int num_sms, cudaStream_t stream) {
+  constexpr uint32_t SMEM = kWgStages * (2 * kWgKB * 128 + 2 * (kWgKB + kWgHalo) * 128) + 128 + 1024;
+  const bool ordered = p.partials != nullptr && slabs > 1;     // a single slab adds each element once: already ordered
+  static bool attr_set[2] = {false, false};
+  if (!attr_set[ordered]) {
+    cudaError_t e = cudaFuncSetAttribute(ordered ? wgrad_kernel<true> : wgrad_kernel<false>,
+                                         cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(SMEM));
+    if (e != cudaSuccess) return e;
+    attr_set[ordered] = true;
+  }
+  if (!ordered) {
+    wgrad_kernel<false><<<grid, 192, SMEM, stream>>>(p);
+    return cudaGetLastError();
+  }
+  wgrad_kernel<true><<<grid, 192, SMEM, stream>>>(p);
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return e;
+  const long long n4 = static_cast<long long>(p.cout) * p.ntaps * p.cin / 4;
+  long long blocks = (n4 + 255) / 256;
+  if (blocks > 8ll * num_sms) blocks = 8ll * num_sms;
+  wgrad_reduce_kernel<<<static_cast<unsigned>(blocks), 256, 0, stream>>>(reinterpret_cast<const float4*>(p.partials),
+                                                                         reinterpret_cast<float4*>(p.dw), n4, slabs);
   return cudaGetLastError();
 }
 

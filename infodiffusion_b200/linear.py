@@ -5,6 +5,9 @@ The small fully-connected layers of the path -- TimeEmbedding and the per-block 
 (models.py:147-163, 223-234) -- stay in fp32 like the reference.  In training they sit inside torch's autograd graph;
 this Function keeps them off cuBLAS: y = x W^T + b, dX = dY W, dW = dY^T X, db = 1^T dY are all launches of
 libidf_b200.so.  Elementwise glue around them (SiLU, LayerNorm, dropout) remains ordinary torch ops.
+
+While torch.are_deterministic_algorithms_enabled(), the split-K GEMMs combine their partial tiles in split order
+(idf_gemm_f32_ordered) instead of with atomics, so forward and backward are bitwise reproducible.
 """
 from __future__ import annotations
 
@@ -17,6 +20,17 @@ from . import _lib
 
 def _stream(t: torch.Tensor) -> int:
     return torch.cuda.current_stream(t.device).cuda_stream
+
+
+def _gemm(lib, A, lda, tA, B, ldb, tB, Cm, ldc, M, N, K, acc, st) -> None:
+    """Cm[M,N] (+)= op(A) . op(B) on idf_gemm_f32, or on its ordered variant in torch's deterministic mode."""
+    if not torch.are_deterministic_algorithms_enabled():
+        _lib.check(lib.idf_gemm_f32(A, lda, tA, B, ldb, tB, Cm, ldc, M, N, K, acc, st))
+        return
+    n = int(lib.idf_gemm_f32_ws_floats(M, N, K))
+    ws = torch.empty(max(n, 4), dtype=torch.float32, device="cuda")
+    tickets = torch.zeros(64, dtype=torch.int32, device="cuda")
+    _lib.check(lib.idf_gemm_f32_ordered(A, lda, tA, B, ldb, tB, Cm, ldc, M, N, K, acc, ws.data_ptr(), tickets.data_ptr(), st))
 
 
 class _LinearFn(torch.autograd.Function):
@@ -34,7 +48,7 @@ class _LinearFn(torch.autograd.Function):
             # few output tiles and a long reduction (the encoder's fc_a: [B, 4096] -> a_dim): split-K GEMM accumulated on
             # top of the bias (atomic partial sums -- training only; the inference plans keep the deterministic kernel)
             y = (bb if bb is not None else torch.zeros(N, device=x.device)).expand(M, N).contiguous()
-            _lib.check(lib.idf_gemm_f32(x2.data_ptr(), K, 0, w.data_ptr(), K, 1, y.data_ptr(), N, M, N, K, 1, _stream(x)))
+            _gemm(lib, x2.data_ptr(), K, 0, w.data_ptr(), K, 1, y.data_ptr(), N, M, N, K, 1, _stream(x))
         else:
             y = torch.empty(M, N, dtype=torch.float32, device=x.device)
             _lib.check(lib.idf_linear_f32(x2.data_ptr(), K, w.data_ptr(), None if bb is None else bb.data_ptr(), y.data_ptr(), N,
@@ -57,17 +71,17 @@ class _LinearFn(torch.autograd.Function):
         n = 0
         if ctx.needs_input_grad[0]:                  # dX[M,K] = dY[M,N] . W[N,K]
             dx = torch.empty(M, K, dtype=torch.float32, device=dy2.device)
-            _lib.check(lib.idf_gemm_f32(dy2.data_ptr(), N, 0, w.data_ptr(), K, 0, dx.data_ptr(), K, M, K, N, 0, st))
+            _gemm(lib, dy2.data_ptr(), N, 0, w.data_ptr(), K, 0, dx.data_ptr(), K, M, K, N, 0, st)
             dx = dx.view(ctx.xshape)
             n += 1
         if ctx.needs_input_grad[1]:                  # dW[N,K] = dY^T[N,M] . X[M,K]
             dw = torch.empty(N, K, dtype=torch.float32, device=dy2.device)
-            _lib.check(lib.idf_gemm_f32(dy2.data_ptr(), N, 1, x2.data_ptr(), K, 0, dw.data_ptr(), K, N, K, M, 0, st))
+            _gemm(lib, dy2.data_ptr(), N, 1, x2.data_ptr(), K, 0, dw.data_ptr(), K, N, K, M, 0, st)
             n += 1
         if ctx.has_bias and ctx.needs_input_grad[2]:  # db[N] = 1^T[1,M] . dY[M,N]
             ones = torch.ones(1, M, dtype=torch.float32, device=dy2.device)
             db = torch.empty(N, dtype=torch.float32, device=dy2.device)
-            _lib.check(lib.idf_gemm_f32(ones.data_ptr(), M, 0, dy2.data_ptr(), N, 0, db.data_ptr(), N, 1, N, M, 0, st))
+            _gemm(lib, ones.data_ptr(), M, 0, dy2.data_ptr(), N, 0, db.data_ptr(), N, 1, N, M, 0, st)
             n += 1
         _lib.count_launch(n)
         return dx, dw, db

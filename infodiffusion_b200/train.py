@@ -14,6 +14,12 @@ Gradient conventions
   * attention backward       = recomputed with torch matmuls for now (1 % of the FLOPs; kernel is a next step);
   * the small MLPs (time embedding, fc_a, temb/aemb projections, encoder fc heads) and the loss arithmetic stay
     in torch autograd: this module exposes the conv stacks as autograd Functions with (x, mod_t, mod_z) inputs.
+
+Deterministic mode: a plan built while torch.are_deterministic_algorithms_enabled() is an ORDERED plan.  Its split-K
+weight gradients, bias gradients and GroupNorm-affine gradients use the library's ordered variants, whose partials are
+combined in a fixed index order, so the step is bitwise reproducible on one GPU model.  The plan owns their workspaces:
+one scratch shared by the side-stream ops (weight / bias gradients run in stream order there) and one for the
+main-stream AdaGN backward, each with its own ticket counter.
 """
 from __future__ import annotations
 
@@ -80,6 +86,12 @@ class BwdState:
         self.late: List[Callable[[], None]] = []        # pointer fix-ups once the fp32 arena exists
         self.side: set = set()       # indices of ops that nothing later in the list depends on (weight / bias gradients)
         self.side_stream: Optional[torch.cuda.Stream] = None
+        self.ordered = bool(getattr(plan, "ordered", False))
+        self.side_ws_floats = 0      # ordered: largest colsum workspace (the wgrad partials are sized once the plans exist)
+        self.main_ws_floats = 0      # ordered: largest AdaGN dgamma / dbeta workspace
+        self.side_ws: Optional[torch.Tensor] = None
+        self.main_ws: Optional[torch.Tensor] = None
+        self.tickets: Optional[torch.Tensor] = None   # [0]: side-stream ops, [1]: main-stream ops; zero between launches
 
     def __del__(self):
         try:
@@ -166,13 +178,19 @@ def _wgrad(plan, st: BwdState, dout, x, x_rows: int, cin: int, cout: int, tap_of
     st.wplans.append((d, h, get))           # created once the arena is allocated (needs the dw pointer)
     st.side.add(len(st.ops))                 # leaf of the backward graph: runs on the side stream
     st.ops.append(lambda: (_lib.check(plan.lib.idf_wgrad_run(h, torch.cuda.current_stream(plan.device).cuda_stream)),
-                           _lib.count_launch()))
+                           _lib.count_launch(2 if d.partials else 1)))       # ordered split-K: + the slab reduction
     return get
 
 
 def _bias_grad(plan, st: BwdState, dout, cout: int):
     get = st.arena((cout,))
     st.side.add(len(st.ops))
+    if st.ordered:
+        st.side_ws_floats = max(st.side_ws_floats, int(plan.lib.idf_colsum_ws_floats(dout.rows, cout)))
+        st.ops.append(lambda: (_lib.check(plan.lib.idf_colsum_bf16_ordered(
+            dout.t.data_ptr(), get().data_ptr(), dout.rows, cout, st.side_ws.data_ptr(), st.tickets.data_ptr(),
+            torch.cuda.current_stream(plan.device).cuda_stream)), _lib.count_launch()))
+        return get
     st.ops.append(lambda: (_lib.check(plan.lib.idf_colsum_bf16(dout.t.data_ptr(), get().data_ptr(), dout.rows, cout,
                                                                torch.cuda.current_stream(plan.device).cuda_stream)),
                            _lib.count_launch()))
@@ -345,6 +363,10 @@ def bwd_adagn(plan, a, src0, src1, out, gn: nn.GroupNorm, gamma: torch.Tensor, b
     if a.mod_z:
         b.d_mod_z = plan.d_mod_z.data_ptr() + 4 * mod_cols
     st.late.append(lambda: (setattr(b, "dgamma", gget().data_ptr()), setattr(b, "dbeta", bget().data_ptr())))
+    if st.ordered:
+        st.main_ws_floats = max(st.main_ws_floats, plan.B * Cc * 2)
+        st.late.append(lambda: (setattr(b, "dparam_ws", st.main_ws.data_ptr()),
+                                setattr(b, "dparam_ticket", st.tickets.data_ptr() + 4)))
     st.kernel(plan.lib.idf_adagn_silu_bwd, C.byref(b))
     st.param_grads.append((gn.weight, gget))
     st.param_grads.append((gn.bias, bget))
@@ -379,11 +401,23 @@ def finalize_backward(plan) -> BwdState:
     for emit in reversed(plan.tape):
         emit()
     st.flat = torch.zeros(max(st.flat_size, 4), dtype=torch.float32, device=plan.device)
-    for fix in st.late:
-        fix()
     for d, h, get in st.wplans:
         d.dw = get().data_ptr()
         _lib.check(plan.lib.idf_wgrad_plan_create(C.byref(d), C.byref(h)))
+    if st.ordered:
+        # the split-K partials share the side-stream scratch; their size is known once the plans exist, and the
+        # pointer is part of the plan, so the multi-slab plans are created again with it
+        part = [int(plan.lib.idf_wgrad_plan_partials_floats(h)) for _, h, _ in st.wplans]
+        st.side_ws = torch.zeros(max([st.side_ws_floats, 4] + part), dtype=torch.float32, device=plan.device)
+        st.main_ws = torch.zeros(max(st.main_ws_floats, 4), dtype=torch.float32, device=plan.device)
+        st.tickets = torch.zeros(2, dtype=torch.int32, device=plan.device)
+        for (d, h, _), n in zip(st.wplans, part):
+            if n:
+                _lib.check(plan.lib.idf_wgrad_plan_destroy(h))
+                d.partials = st.side_ws.data_ptr()
+                _lib.check(plan.lib.idf_wgrad_plan_create(C.byref(d), C.byref(h)))
+    for fix in st.late:
+        fix()
     _build_grad_maps(plan, st)
     st._final = True
     return st
@@ -613,9 +647,11 @@ def backbone_train_forward(net, x_t: torch.Tensor, t: torch.Tensor, a: torch.Ten
     from .engine import BackbonePlan, conditioned_blocks, modulation_weights
     B = x_t.shape[0]
     plans = net._plans()
-    key = ("train", B, x_t.device.index, float(dropout_p))
+    ordered = torch.are_deterministic_algorithms_enabled()
+    key = ("train", B, x_t.device.index, float(dropout_p), ordered)
     if key not in plans:
         plans[key] = BackbonePlan(net, B, x_t.device, mode="train", dropout_p=dropout_p)
+        plans[key].ordered = ordered
     plan = plans[key]
     # modulation rows through torch autograd (tiny GEMMs): temb -> all blocks' temb_proj, a -> fc_a -> aemb_proj
     from . import linear as L                    # fp32 Linears with autograd on the library's own kernels (no cuBLAS)
@@ -639,9 +675,11 @@ def encoder_train_forward(net, x: torch.Tensor, seed: int, dropout_p: float):
     from .engine import EncoderPlan
     B = x.shape[0]
     plans = net._plans()
-    key = ("train_enc", B, x.device.index, float(dropout_p))
+    ordered = torch.are_deterministic_algorithms_enabled()
+    key = ("train_enc", B, x.device.index, float(dropout_p), ordered)
     if key not in plans:
         plans[key] = EncoderPlan(net, B, x.device, training=True, dropout_p=dropout_p)
+        plans[key].ordered = ordered
     plan = plans[key]
     params = stack_params(net)
     fmap = _ConvStackFn.apply(plan, x, None, None, seed, *params)

@@ -22,7 +22,13 @@ class _MMD(torch.autograd.Function):
         loss = torch.empty((), dtype=torch.float32, device=y.device)
         grad = torch.empty_like(yc)
         stream = torch.cuda.current_stream(y.device).cuda_stream
-        _lib.check(lib.idf_mmd_fwd_bwd(x.data_ptr(), yc.data_ptr(), loss.data_ptr(), grad.data_ptr(), B, D, stream))
+        if torch.are_deterministic_algorithms_enabled():          # partials summed in a fixed order, no atomics
+            ws = torch.empty(int(lib.idf_mmd_ws_floats(B)), dtype=torch.float32, device=y.device)
+            tickets = torch.zeros(1, dtype=torch.int32, device=y.device)
+            _lib.check(lib.idf_mmd_fwd_bwd_ordered(x.data_ptr(), yc.data_ptr(), loss.data_ptr(), grad.data_ptr(), B, D,
+                                                   ws.data_ptr(), tickets.data_ptr(), stream))
+        else:
+            _lib.check(lib.idf_mmd_fwd_bwd(x.data_ptr(), yc.data_ptr(), loss.data_ptr(), grad.data_ptr(), B, D, stream))
         _lib.count_launch()
         ctx.save_for_backward(grad)
         return loss

@@ -83,6 +83,9 @@ def parse_args(argv=None):
                    help='eval_fid without --is_latent: skip the vanilla model / two-phase sampler (the reference requires it)')
     p.add_argument('--allow_random_init', action='store_true',
                    help='evaluate the seeded random initialisation when the checkpoint is missing (the reference raises)')
+    p.add_argument('--deterministic_training', action='store_true',
+                   help='train / train_latent_ddim: torch.use_deterministic_algorithms(True), so the seed pins the run '
+                        '(bitwise reproducible on one GPU model; the gradient reductions run in a fixed order)')
     return p.parse_args(argv)
 
 
@@ -243,6 +246,8 @@ def _batches(x, batch_size, rank, world, seed):
 def train(args):
     rank, world = _world()
     seed_everything(args.r_seed)
+    if args.deterministic_training:
+        torch.use_deterministic_algorithms(True)
     device = torch.device("cuda", torch.cuda.current_device())
     shape = get_dataset_config(args)
     x, _ = load_images(args, shape)
@@ -255,6 +260,8 @@ def train(args):
 def train_latent_ddim(args):
     rank, world = _world()
     seed_everything(args.r_seed)
+    if args.deterministic_training:
+        torch.use_deterministic_algorithms(True)
     device = torch.device("cuda", torch.cuda.current_device())
     z = torch.from_numpy(np.load("{}_{}_latent.npz".format(args.model, generate_exp_string(args).replace(".", "_")))["all_a"]).float()
     model = Diff(args, device, (1, args.a_dim, args.a_dim))
