@@ -205,6 +205,8 @@ typedef struct {
   int32_t stats_planes0, stats_planes1;
   int32_t stats_rows0, stats_rows1;
 } idf_adagn_args;
+/* C = c0 + c1 <= 1024 with C % 32 == 0 and c0, c1 multiples of 8.  Without statistics for every source (the two-sweep
+ * variant, which computes them itself) C <= 256; a wider call returns IDF_ERR_CUDA and writes nothing. */
 int idf_adagn_silu_fwd(const idf_adagn_args* args, idf_stream_t stream);
 /* Coefficients only: coef_out[n][c] = (A, B) with AdaGN(x)[n, c, :, :] = A*x + B (before the activation), from the
  * producers' window records (stats0 / stats1 required).  Feeds idf_conv_desc.xf_coef; out / src pointers of
@@ -235,7 +237,12 @@ int64_t idf_adagn_bwd_ws_floats(int32_t batch, int32_t C);
 int idf_adagn_silu_bwd(const idf_adagn_bwd_args* args, idf_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
- * Fused single-head self attention (QK^T -> softmax -> PV on tcgen05), S = H*W tokens, d = 128.
+ * Fused single-head self attention (QK^T -> softmax -> PV), S = H*W tokens, one of three kernels by shape:
+ *   d = 128 with S in {64, 256}: tcgen05 (P rounded to bf16 before the PV product);
+ *   otherwise S <= 64 with S*d <= 8192: a small-map kernel, plain fp32 FMAs, one CTA per sample;
+ *   otherwise d % 8 == 0, d <= 1024 and S <= 1024: a CUDA-core kernel, fp32, one CTA per (sample, 16 queries)
+ *     (the vanilla Diff model's heads of 256 and 512 channels).
+ * Other shapes return IDF_ERR_CUDA with a message naming these.
  * Replaces torch.bmm / F.softmax / permutes at modules.py:152-161.
  * qkv: bf16 pad-flat [rows, 3*d] (q | k | v), out: bf16 pad-flat [rows, d]; scale = d^-0.5.
  * ------------------------------------------------------------------------------------------ */

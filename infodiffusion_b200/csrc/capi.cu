@@ -403,7 +403,7 @@ int idf_wgrad_run(const idf_wgrad_plan* plan, idf_stream_t stream) {
 int idf_adagn_coef(const idf_adagn_args* a, float* coef_out, idf_stream_t stream) {
   if (a == nullptr || coef_out == nullptr) return fail(IDF_ERR_ARG, "null argument");
   cudaError_t e = launch_adagn_coef(*a, coef_out, reinterpret_cast<cudaStream_t>(stream));
-  if (e != cudaSuccess) return cuda_fail(e, "adagn_coef launch (needs stats0/stats1, C <= 256, C % 32 == 0)");
+  if (e != cudaSuccess) return cuda_fail(e, "adagn_coef launch (needs stats0/stats1, C <= 1024, C % 32 == 0)");
   return IDF_OK;
 }
 
@@ -437,7 +437,9 @@ int idf_attn_fwd(const void* qkv, void* out, int32_t batch, int32_t H, int32_t W
     else                                       // wide heads (vanilla Diff model, d = 256 / 512): CUDA-core kernel
       e = launch_attn_generic(static_cast<const bf16*>(qkv), static_cast<bf16*>(out), batch, H, W, d, scale,
                               reinterpret_cast<cudaStream_t>(stream));
-    if (e != cudaSuccess) return cuda_fail(e, "attention launch (tensor-core kernel: d=128 with H*W in {64,256}; otherwise d % 8 == 0, H*W <= 1024)");
+    if (e != cudaSuccess)
+      return cuda_fail(e, "attention launch (supported: d = 128 with H*W in {64, 256}; H*W <= 64 with H*W*d <= 8192; "
+                          "or d % 8 == 0, d <= 1024, H*W <= 1024)");
     return IDF_OK;
   }
   CUtensorMap tm;   // TMA boxes per image row
