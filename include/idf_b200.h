@@ -360,6 +360,14 @@ int idf_sampler_update(float* x, const float* eps, const float* noise, const flo
                        int64_t n, idf_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Sampled latent of the encoder, models.py:515:  out = mu + noise * exp(0.5 * log_var), elementwise over n fp32
+ * values.  Each operation is rounded on its own, as torch's composite computes it on the GPU (same bits).  Any n,
+ * any 4-byte alignment (float4 loads when all four pointers are 16-byte aligned).
+ * ------------------------------------------------------------------------------------------ */
+int idf_reparameterize_f32(const float* mu, const float* log_var, const float* noise, float* out, int64_t n,
+                           idf_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------
  * MMD prior loss (utils.py:74-90), fused pairwise Gaussian-kernel reduction.
  *   loss = mean k(x,x) + mean k(y,y) - 2 mean k(x,y),  k(u,v) = exp(-|u-v|^2 / D^2)
  * x: prior samples [B,D], y: latents [B,D]; grad_y (optional) = d loss / d y.

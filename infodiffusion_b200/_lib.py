@@ -163,6 +163,7 @@ SIGNATURES = {
     "idf_colsum_ws_floats": (C.c_int64, [C.c_int64, C.c_int32]),
     "idf_sampler_update": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
                                      C.c_void_p]),
+    "idf_reparameterize_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "idf_mmd_fwd_bwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32,
                                   C.c_void_p]),
     "idf_mmd_fwd_bwd_ordered": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32,

@@ -668,6 +668,15 @@ int idf_sampler_update(float* x, const float* eps, const float* noise, const flo
   return IDF_OK;
 }
 
+int idf_reparameterize_f32(const float* mu, const float* log_var, const float* noise, float* out, int64_t n,
+                           idf_stream_t stream) {
+  if (mu == nullptr || log_var == nullptr || noise == nullptr || out == nullptr || n < 0)
+    return fail(IDF_ERR_ARG, "bad reparameterize arguments");
+  cudaError_t e = launch_reparameterize(mu, log_var, noise, out, n, reinterpret_cast<cudaStream_t>(stream));
+  if (e != cudaSuccess) return cuda_fail(e, "reparameterize launch");
+  return IDF_OK;
+}
+
 int idf_mmd_fwd_bwd(const float* x, const float* y, float* loss, float* grad_y, int32_t B, int32_t D,
                     idf_stream_t stream) {
   if (x == nullptr || y == nullptr || loss == nullptr || B <= 0 || D <= 0 || D > 4096)

@@ -171,6 +171,8 @@ cudaError_t launch_mmd_ordered(const float* x, const float* y, float* loss, floa
 cudaError_t launch_padflat_to_nchw(const bf16* in, float* y, int batch, int C, int H, int W, cudaStream_t stream);
 cudaError_t launch_sampler_update(float* x, const float* eps, const float* noise, const float* coef,
                                   const int32_t* step_ptr, int64_t n, cudaStream_t stream);
+cudaError_t launch_reparameterize(const float* mu, const float* log_var, const float* noise, float* out, int64_t n,
+                                  cudaStream_t stream);
 cudaError_t launch_mmd(const float* x, const float* y, float* loss, float* grad_y, int B, int D, cudaStream_t stream);
 
 }  // namespace idf

@@ -369,6 +369,45 @@ cudaError_t launch_sampler_update(float* x, const float* eps, const float* noise
 }
 
 // ----------------------------------------------------------------------------------------------
+// sampled latent a_q = mu + noise * exp(0.5 * log_var) (float4 vectorised).  Every operation is rounded on its own,
+// in torch's order, so the result is the torch composite's bit for bit: the intrinsics keep the compiler from
+// contracting the product and the sum into one FMA, and expf is the same libdevice routine torch's exp calls.
+// ----------------------------------------------------------------------------------------------
+__device__ __forceinline__ float reparameterize1(float mu, float log_var, float noise) {
+  return __fadd_rn(mu, __fmul_rn(noise, expf(__fmul_rn(0.5f, log_var))));
+}
+
+__global__ void reparameterize_kernel(const float* __restrict__ mu, const float* __restrict__ log_var,
+                                      const float* __restrict__ noise, float* __restrict__ out, long long n4,
+                                      long long n) {
+  const long long stride = static_cast<long long>(gridDim.x) * blockDim.x;
+  const long long tid = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
+  for (long long i = tid; i < n4; i += stride) {
+    const float4 m = __ldg(reinterpret_cast<const float4*>(mu) + i);
+    const float4 l = __ldg(reinterpret_cast<const float4*>(log_var) + i);
+    const float4 z = __ldg(reinterpret_cast<const float4*>(noise) + i);
+    reinterpret_cast<float4*>(out)[i] = make_float4(reparameterize1(m.x, l.x, z.x), reparameterize1(m.y, l.y, z.y),
+                                                    reparameterize1(m.z, l.z, z.z), reparameterize1(m.w, l.w, z.w));
+  }
+  // scalar tail: n not a multiple of 4, or every element when a pointer is not 16-byte aligned (n4 = 0)
+  for (long long i = n4 * 4 + tid; i < n; i += stride) out[i] = reparameterize1(mu[i], log_var[i], noise[i]);
+}
+
+cudaError_t launch_reparameterize(const float* mu, const float* log_var, const float* noise, float* out, int64_t n,
+                                  cudaStream_t stream) {
+  const bool aligned =
+      ((reinterpret_cast<uintptr_t>(mu) | reinterpret_cast<uintptr_t>(log_var) | reinterpret_cast<uintptr_t>(noise) |
+        reinterpret_cast<uintptr_t>(out)) & 15) == 0;
+  const long long n4 = aligned ? n / 4 : 0;
+  const long long items = n4 > n - 4 * n4 ? n4 : n - 4 * n4;
+  long long blocks = (items + 255) / 256;
+  if (blocks > 148 * 8) blocks = 148 * 8;
+  if (blocks < 1) blocks = 1;
+  reparameterize_kernel<<<static_cast<unsigned>(blocks), 256, 0, stream>>>(mu, log_var, noise, out, n4, n);
+  return cudaGetLastError();
+}
+
+// ----------------------------------------------------------------------------------------------
 // small fp32 linear: y[m,n] = sum_k act(x[m,k]) w[n,k] + b[n]; 16x64 output tile, K in chunks of 32
 // ----------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) linear_f32_kernel(const float* __restrict__ x, long long ldx,

@@ -813,10 +813,12 @@ class ModulationTables(Plan):
 # ------------------------------------------------------------------------------------------------
 class EncoderPlan(Plan):
     """(a, mu, log_var) = Encoder(x) for a fixed batch (reference models.py:488-518).  With training=True only
-    the conv stack runs here (x -> 1-channel map, tape recorded); fc_a / fc_mu / fc_var stay in torch autograd."""
+    the conv stack runs here (x -> 1-channel map, tape recorded); fc_a / fc_mu / fc_var stay in torch autograd.
+    Given `latent_noise` [B, a_dim] (filled by the caller before each run), the plan also writes the sampled latent
+    a_q = mu + latent_noise * exp(0.5 * log_var) (models.py:515) into self.a_q."""
 
     def __init__(self, net, batch: int, device, ws: Optional[Workspace] = None, x_in: Optional[torch.Tensor] = None,
-                 training: bool = False, dropout_p: float = 0.0):
+                 training: bool = False, dropout_p: float = 0.0, latent_noise: Optional[torch.Tensor] = None):
         super().__init__(batch, device, ws, training=training)
         Cimg, H, W = net.shape
         assert H == W and H in (32, 64)
@@ -841,6 +843,15 @@ class EncoderPlan(Plan):
             self.linear(flat, self.f32(net.fc_a.weight), self.f32(net.fc_a.bias), self.a, silu_in=False)
             self.linear(self.a, self.f32(net.fc_mu.weight), self.f32(net.fc_mu.bias), self.mu, silu_in=False)
             self.linear(self.a, self.f32(net.fc_var.weight), self.f32(net.fc_var.bias), self.log_var, silu_in=False)
+        self.latent_noise = latent_noise
+        self.a_q = None
+        if latent_noise is not None:
+            assert not training, "the training path samples a_q in torch autograd"
+            assert latent_noise.shape == (B, net.a_dim) and latent_noise.is_contiguous()
+            self.a_q = torch.zeros(B, net.a_dim, **f32)
+            self._emit("reparameterize", self.lib.idf_reparameterize_f32,
+                       (self.mu.data_ptr(), self.log_var.data_ptr(), latent_noise.data_ptr(), self.a_q.data_ptr(),
+                        B * net.a_dim))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -879,13 +890,13 @@ def encoder_forward(net, x: torch.Tensor):
     key = ("enc", B, x.device.index)
     plans = net._plans()
     if key not in plans:
-        plans[key] = EncoderPlan(net, B, x.device)
+        plans[key] = EncoderPlan(net, B, x.device,
+                                 latent_noise=torch.zeros(B, net.a_dim, dtype=torch.float32, device=x.device))
     p: EncoderPlan = plans[key]
     p.x_in.copy_(x)
+    p.latent_noise.copy_(torch.randn_like(p.mu))                     # reference models.py:515
     p.run()
-    a, mu, log_var = p.a.clone(), p.mu.clone(), p.log_var.clone()
-    a_q = mu + torch.randn_like(mu) * torch.exp(0.5 * log_var)      # reference models.py:515
-    return a, a_q, mu, log_var
+    return p.a.clone(), p.a_q.clone(), p.mu.clone(), p.log_var.clone()
 
 
 # ------------------------------------------------------------------------------------------------

@@ -5,8 +5,9 @@ diffusion_fn, device, shape)`` with ``.sampling(sampling_number, xT, a)`` and
 ``.reverse_sampling(x0, a)``.  The loop body is different: one step is a single CUDA-graph replay of
 the whole UNet with the x_{t-1} update fused into the output convolution's epilogue; per-step values
 come from device tables indexed by a device-resident step counter, so the host does nothing per
-step except (for stochastic steps) drawing that step's noise with torch's generator, in the
-reference's order, so identical seeds give identical noise.
+step except (for stochastic steps, and for the sampled latent of a KLD model's re-encoding reverse
+steps) drawing that step's noise with torch's generator, in the reference's order, so identical
+seeds give identical noise.
 """
 from __future__ import annotations
 
@@ -109,6 +110,10 @@ class _FusedSampler:
         self.tables = ModulationTables(net, dev, self.pack, T)
         self.tables.run()
         self.mod_z = torch.zeros(batch, self.pack.ncol, **f32)
+        # a KLD model conditions the re-encoded step on a_q = mu + noise * exp(0.5 * log_var) (models.py:515, 714-721):
+        # one full-batch noise buffer, refilled before every step, so chunked plans read the same values
+        sampled = with_encoder and model._uses_sampled_latent()
+        self.latent_noise = torch.zeros(batch, model.encoder.a_dim, **f32) if sampled else None
         chunk = batch if chunk is None else min(chunk, batch)
         assert batch % chunk == 0, "chunk must divide the batch"
         # lanes: micro-batches on different lanes run on different streams (own workspace each), so the small
@@ -127,11 +132,10 @@ class _FusedSampler:
             if with_encoder:
                 # bug-compatible reverse DDIM: re-encode the current x_t every step (sampling.py:84,
                 # models.py:709-710) and derive this chunk's z-modulation rows from the fresh latent
-                if model.kld_weight != 0:
-                    raise NotImplementedError("re-encoding reverse DDIM with a sampled latent (kld_weight != 0)")
-                ep = EncoderPlan(model.encoder, chunk, dev, ws=self.ws, x_in=self.x[sl])
+                ep = EncoderPlan(model.encoder, chunk, dev, ws=self.ws, x_in=self.x[sl],
+                                 latent_noise=self.latent_noise[sl] if sampled else None)
                 zp = Plan(chunk, dev, ws=self.ws)
-                zp._emit_latent_mlp(net, self.pack, ep.a, self.mod_z[sl])
+                zp._emit_latent_mlp(net, self.pack, ep.a_q if sampled else ep.a, self.mod_z[sl])
                 self.plans += [ep, zp]
             bp = BackbonePlan(net, chunk, dev, mode="sampler", ws=self.ws, x_io=self.x[sl],
                               noise=None if self.noise is None else self.noise[sl], coef=self.coef, step=self.step,
@@ -192,6 +196,9 @@ class DiffusionProcess():
         # noise_fn(idx, out) fills `out` with the step's N(0,1) noise; the default draws from torch's CUDA
         # generator exactly where the reference calls torch.randn_like (parity tests inject fixed tensors)
         self.noise_fn = lambda idx, out: out.normal_()
+        # latent_noise_fn(idx, out) fills `out` [B, a_dim] with the N(0,1) draw of the encoder's sampled latent before
+        # every re-encoding reverse step of a KLD model: the reference's one randn_like(mu) per model call (models.py:515)
+        self.latent_noise_fn = lambda idx, out: out.normal_()
         self._samplers = {}
 
     # ------------------------------------------------------------------------------------------
@@ -231,6 +238,8 @@ class DiffusionProcess():
                 # ddpm: drawn BEFORE the model call (sampling.py:29); ddim: the reference draws it after the model
                 # call (sampling.py:56) -- the model call consumes no random numbers, so the stream is identical
                 self.noise_fn(idx, s.noise)
+            if s.latent_noise is not None:
+                self.latent_noise_fn(idx, s.latent_noise)
             s.run_step(idx, use_graph=self.use_graph)
             yield idx, s
 
@@ -266,7 +275,9 @@ class DiffusionProcess():
     def reverse_sampling(self, x0, a=None, trace=None):
         """x0 -> xT by deterministic reverse DDIM (reference sampling.py:81-87).  The reference drops
         ``a`` and re-encodes x_t at every step (SURVEY H5a); that is the default here too.  Set
-        ``args.reverse_uses_given_latent = True`` to honour the caller's ``a`` instead."""
+        ``args.reverse_uses_given_latent = True`` to honour the caller's ``a`` instead.  A KLD model
+        (kld_weight != 0) conditions each re-encoded step on the sampled latent a_q, whose noise
+        ``latent_noise_fn`` draws before the step (models.py:515, 714-721)."""
         if not self.honor_latent_in_reverse:
             a = None
         return self._run("reverse", x0, a, trace)

@@ -18,8 +18,8 @@ What differs, on purpose:
     batch from the same seed, so the written images do not depend on the number of GPUs (checked by
     tools/check_run_py_multigpu.sh: 2 GPUs vs 1 GPU differ by at most one uint8 level in 0.01 % of the pixels).
 The analysis modes latent_quality / disentangle / interpolate (run.py:310-341, 371-414, 444-481) are thin callers of
-the encoder, reverse DDIM and the sampler and are built; the VAE baseline, plot_latent (matplotlib) and save_original_img
-are not.
+the encoder, reverse DDIM and the sampler and are built, for MMD and KLD (--kld_weight) models alike; the VAE baseline,
+plot_latent (matplotlib) and save_original_img are not.
 """
 from __future__ import annotations
 
