@@ -79,6 +79,21 @@ class _EngineNet(nn.Module):
         self.invalidate_plans()
         return out
 
+    def _differentiable(self, *inputs) -> bool:
+        """The routing rule of every forward: autograd through the kernels' backward when grad mode is on and either
+        the module is in train mode or a tensor input requires grad.  Every other call keeps the fused inference plan,
+        including an eval() call whose inputs need no gradient (parameters that require grad do not count, or every
+        such call would run on a training plan)."""
+        return torch.is_grad_enabled() and (self.training or any(torch.is_tensor(v) and v.requires_grad for v in inputs))
+
+    def _dropout(self):
+        """(seed, p) of the differentiable forward.  train(): the hash-dropout seed comes from torch's CPU generator, so
+        it follows torch.manual_seed.  eval(): dropout is off and nothing is drawn, so the call leaves torch's
+        generators where the inference call leaves them."""
+        if not self.training:
+            return 0, 0.0
+        return int(torch.empty((), dtype=torch.int64).random_().item()), self.dropout_p
+
 
 class AuxiliaryUNet(_EngineNet):
     """eps-network conditioned on timestep t and auxiliary latent a (reference models.py:237-326)."""
@@ -108,11 +123,11 @@ class AuxiliaryUNet(_EngineNet):
 
     def forward(self, x, t, a):
         """x [B,C,H,W] fp32, t int64 [B], a [B,a_dim] -> eps [B,C,H,W] fp32 (reference models.py:296).
-        eval(): inference plan.  train(): dropout on and autograd through the kernels' backward."""
-        if self.training and torch.is_grad_enabled():
+        train() with grad: dropout on and autograd through the kernels' backward.  eval() with grad and x or a
+        requiring grad: the same path with dropout off.  Otherwise: the inference plan."""
+        if self._differentiable(x, a):
             from .train import backbone_train_forward
-            seed = int(torch.empty((), dtype=torch.int64).random_().item())   # CPU generator: follows torch.manual_seed
-            return backbone_train_forward(self, x, t, a, seed, self.dropout_p)
+            return backbone_train_forward(self, x, t, a, *self._dropout())
         from .engine import backbone_forward
         return backbone_forward(self, x, t, a)
 
@@ -143,10 +158,9 @@ class UNet(_EngineNet):
 
     def forward(self, x, t):
         """x [B,C,H,W] fp32, t int64 [B] -> eps (reference models.py:62)."""
-        if self.training and torch.is_grad_enabled():
+        if self._differentiable(x):
             from .train import backbone_train_forward
-            seed = int(torch.empty((), dtype=torch.int64).random_().item())
-            return backbone_train_forward(self, x, t, None, seed, self.dropout_p)
+            return backbone_train_forward(self, x, t, None, *self._dropout())
         from .engine import backbone_forward
         return backbone_forward(self, x, t, None)
 
@@ -178,10 +192,9 @@ class BottleneckAuxUNet(_EngineNet):
         init.zeros_(self.tail[-1].bias)
 
     def forward(self, x, t, a):
-        if self.training and torch.is_grad_enabled():
+        if self._differentiable(x, a):
             from .train import backbone_train_forward
-            seed = int(torch.empty((), dtype=torch.int64).random_().item())
-            return backbone_train_forward(self, x, t, a, seed, self.dropout_p)
+            return backbone_train_forward(self, x, t, a, *self._dropout())
         from .engine import backbone_forward
         return backbone_forward(self, x, t, a)
 
@@ -213,10 +226,9 @@ class Encoder(_EngineNet):
         init.zeros_(self.tail[-1].bias)
 
     def forward(self, x):
-        if self.training and torch.is_grad_enabled():
+        if self._differentiable(x):
             from .train import encoder_train_forward
-            seed = int(torch.empty((), dtype=torch.int64).random_().item())   # CPU generator: follows torch.manual_seed
-            return encoder_train_forward(self, x, seed, self.dropout_p)
+            return encoder_train_forward(self, x, *self._dropout())
         from .engine import encoder_forward
         return encoder_forward(self, x)
 
@@ -283,9 +295,10 @@ class LatentUNet(_EngineNet):
 
     def forward(self, x, t):
         """x [B, D] fp32, t int64 [B] -> eps [B, D] (reference models.py:223).  eval(): fused kernels
-        (engine.LatentPlan); train() with grad: the same arithmetic as a torch autograd composite on the GPU."""
+        (engine.LatentPlan); train() with grad, or eval() with grad and x requiring grad: the same arithmetic as a torch
+        autograd composite on the GPU (its Dropouts are identities in eval())."""
         from .engine import latent_forward, latent_forward_autograd
-        if self.training and torch.is_grad_enabled():
+        if self._differentiable(x):
             return latent_forward_autograd(self, x, t)
         return latent_forward(self, x, t)
 
@@ -335,7 +348,7 @@ class InfoDiff(nn.Module):
     def loss_fn(self, args, x, idx=None, curr_epoch=0):
         """Training objective (reference models.py:632-696), prior='regular'.  In train() mode the returned
         scalar carries an autograd graph whose heavy nodes are the sm_100a backward kernels
-        (infodiffusion_b200.train); in eval() mode it is the forward value only."""
+        (infodiffusion_b200.train); in eval() mode it is the forward value only, unless x requires grad."""
         output, epsilon, a, mu, log_var = self.forward(x, idx=idx, get_target=True)
         loss = (output - epsilon).square().mean()
         x_0 = torch.sqrt(1 / self.alphas[0]) * (x - self.betas[0] / torch.sqrt(1 - self.alpha_bars[0]) * output)

@@ -10,6 +10,8 @@ Gradient conventions
   * data gradient of a conv  = the forward implicit-GEMM kernel over dY with negated taps / transposed weights;
   * weight gradient          = idf_wgrad (tcgen05, pixels as K), fp32, one flat buffer zeroed per step;
   * bias gradient            = column sums of dY;
+  * input gradient           = the head conv's data gradient into fp32 NCHW, one launch after the backward graph,
+    only when the network's input requires grad (bwd_head);
   * AdaGN                    = idf_adagn_silu_bwd -> dx and (S1, S2); gamma/beta/modulation grads in closed form;
   * attention backward       = recomputed with torch matmuls for now (1 % of the FLOPs; kernel is a next step);
   * the small MLPs (time embedding, fc_a, temb/aemb projections, encoder fc heads) and the loss arithmetic stay
@@ -31,8 +33,8 @@ import torch
 import torch.nn as nn
 
 from . import _lib
-from ._lib import AdaGNBwdArgs, WgradDesc
-from .layout import pv, tap_offsets3x3, taps_stride2
+from ._lib import EPI_F32_NCHW, AdaGNBwdArgs, WgradDesc
+from .layout import pad_rows, pv, tap_offsets3x3, taps_stride2
 
 BF16 = torch.bfloat16
 
@@ -258,13 +260,34 @@ def bwd_conv1x1_stack(plan, src, convs: Sequence[nn.Conv2d], out, residual) -> N
 
 
 def bwd_head(plan, patches, conv: nn.Conv2d, out, Cimg: int) -> None:
+    """head conv (im2col + K=64 GEMM): weight and bias gradients in the backward list.  The input gradient is a
+    Cimg <- cout 3x3 conv over dY (negated taps, transposed weights, fp32 NCHW out: the tail's forward shape) whose
+    conv plan is kept on the training plan as `dx_op`; _ConvStackFn.backward launches it only when the input
+    requires grad, so a step without input gradient keeps its launch list."""
     st = _state(plan)
     dout = st.grad(out)
-    cout = out.C
+    cout, H = out.C, out.H
     get = _wgrad(plan, st, dout, patches, patches.t.shape[0], 64, cout, [0])
     st.param_grads.append((conv.weight, lambda: get()[:, 0, :9 * Cimg].view(cout, 9, Cimg).permute(0, 2, 1)
                            .reshape(cout, Cimg, 3, 3)))
     st.param_grads.append((conv.bias, _bias_grad(plan, st, dout, cout)))
+    kb = [(0, c0, -off) for off in tap_offsets3x3(H, H) for c0 in range(0, cout, 64)]
+    # packed with the plan's other recipes, so the re-pack before every forward keeps it on the current parameters
+    wp = plan.weight(lambda: pad_rows(pv(conv.weight).permute(1, 2, 3, 0).reshape(Cimg, 9 * cout), 16))
+    zero_bias = torch.zeros(wp.shape[0], dtype=torch.float32, device=plan.device)
+    plan.d_x = torch.zeros(plan.B, Cimg, H, H, dtype=torch.float32, device=plan.device)
+    plan.keep.append(zero_bias)
+    plan.conv([dout], kb, wp, zero_bias, H, Cimg, 16, epilogue=EPI_F32_NCHW, out_f32=plan.d_x)
+    plan.dx_op = plan.ops.pop()
+    plan.meta.pop()
+
+
+def run_input_grad(plan) -> torch.Tensor:
+    """d_x of the plan's input from the head output's gradient the last backward left (see bwd_head)."""
+    fn, args = plan.dx_op
+    _lib.check(fn(*args, torch.cuda.current_stream(plan.device).cuda_stream))
+    _lib.count_launch()
+    return plan.d_x.clone()
 
 
 def bwd_tail(plan, ta, tconv: nn.Conv2d, out_f32: torch.Tensor, cout: int) -> None:
@@ -628,7 +651,8 @@ class _ConvStackFn(torch.autograd.Function):
         grads = fused_param_grads(plan)            # same order as ctx.params (= plan.pindex.params)
         dmt = plan.d_mod_t.clone() if ctx.has_mod else None
         dmz = plan.d_mod_z.clone() if ctx.has_mod else None
-        return (None, None, dmt, dmz, None, *grads)
+        dx = run_input_grad(plan) if ctx.needs_input_grad[1] else None
+        return (None, dx, dmt, dmz, None, *grads)
 
 
 def stack_params(net) -> List[nn.Parameter]:
@@ -644,7 +668,8 @@ def stack_params(net) -> List[nn.Parameter]:
 def backbone_train_forward(net, x_t: torch.Tensor, t: torch.Tensor, a: torch.Tensor, seed: int,
                            dropout_p: float) -> torch.Tensor:
     """eps = AuxiliaryUNet(x_t, t, a) with autograd through the sm_100a kernels (reference models.py:296-326)."""
-    from .engine import BackbonePlan, conditioned_blocks, modulation_weights
+    from .engine import BackbonePlan, _require_cuda, conditioned_blocks, modulation_weights
+    _require_cuda(x_t, "x")
     B = x_t.shape[0]
     plans = net._plans()
     ordered = torch.are_deterministic_algorithms_enabled()
@@ -672,7 +697,8 @@ def backbone_train_forward(net, x_t: torch.Tensor, t: torch.Tensor, a: torch.Ten
 
 def encoder_train_forward(net, x: torch.Tensor, seed: int, dropout_p: float):
     """(a, a_q, mu, log_var) = Encoder(x) with autograd (reference models.py:488-518)."""
-    from .engine import EncoderPlan
+    from .engine import EncoderPlan, _require_cuda
+    _require_cuda(x, "x")
     B = x.shape[0]
     plans = net._plans()
     ordered = torch.are_deterministic_algorithms_enabled()
