@@ -109,11 +109,15 @@ typedef struct {
   /* optional (IDF_EPI_BF16): GroupNorm partial sums of the stored (bf16-rounded) output, fp32
    * [2][ceil(rows/128)*4][cout][2] (capacity; the item form below fills a prefix).  Records cover UNITS of
    * idf_conv_plan_stats_unit(plan) rows:
-   *   unit = 32   one record per 32-row window k = row/32 (windows never span 128-row tiles);
+   *   unit = 32   one record per 32-row window k = row/32 (windows never span 128-row tiles), split at the window's
+   *               LAST image boundary b: A[k][c] = (sum, sumsq) over the rows before b (image (b-1)/R, R = (H+1)*(W+1)),
+   *               B[k][c] = the same over the rows from b on (image b/R); no boundary: A over all rows.  With R < 32
+   *               a window can touch three images; the rows before an earlier boundary are then pad rows, which needs
+   *               31 - R <= W + 2 (H = W >= 4).  Smaller grids (H = W <= 3) return IDF_ERR_ARG when stats_out is set;
    *   unit = 128*MT (chosen when an image has at least that many pad-flat rows): 4 records per work item of MT
-   *                 tiles, k = item*4 + q, q = lane quarter (rows 32q..32q+31 of each of the item's tiles).
-   *   A[k][c] = (sum, sumsq) over the record's rows in the image the UNIT starts in,
-   *   B[k][c] = the same over its rows in the following image (only written if the unit straddles).
+   *                 tiles, k = item*4 + q, q = lane quarter (rows 32q..32q+31 of each of the item's tiles);
+   *                 A[k][c] over the record's rows in the image the UNIT starts in, B[k][c] over its rows in the
+   *                 following image (only written if the unit straddles).
    * Consumed by idf_adagn_silu_fwd / idf_adagn_coef (stats0 / stats1 with stats_unit0 / stats_unit1).   */
   float* stats_out;
   /* optional: AdaGN (+SiLU) of the CONSUMED activation fused into the A-operand path (inference): k-blocks with
@@ -190,7 +194,8 @@ typedef struct {
   const int32_t* step_ptr;
   int32_t apply_silu;
   /* optional: per-tile partial sums written by the producing convolution (idf_conv_desc.stats_out).
-   * When given for every source the kernel is a single streaming sweep (no statistics pass).     */
+   * When given for every source the kernel is a single streaming sweep (no statistics pass).  Records over a grid
+   * that idf_conv_plan_create rejects for stats_out (H = W <= 3) return IDF_ERR_ARG.             */
   const float* stats0; const float* stats1;
   /* training only: inverted dropout applied after SiLU (nn.Dropout at modules.py:221,227,280,286,342).
    * keep-mask = hash(*dropout_seed, dropout_layer, element index) >= p; 0 disables.               */
@@ -213,7 +218,8 @@ int idf_adagn_silu_fwd(const idf_adagn_args* args, idf_stream_t stream);
  * `args` are not dereferenced. */
 int idf_adagn_coef(const idf_adagn_args* args, float* coef_out, idf_stream_t stream);
 
-/* Backward of idf_adagn_silu_fwd (streaming variant: stats0/stats1 required).
+/* Backward of idf_adagn_silu_fwd (streaming variant: stats0/stats1 required).  Without save_coef the statistics are
+ * read from 32-row window records of this map (stats_unit 32, no up2 planes; others return IDF_ERR_ARG).
  *   dx0 / dx1 : gradient w.r.t. the sources (bf16 pad-flat; added to the buffer if acc0 / acc1)
  *   sums      : fp32 [batch, C, 2] = (sum_hw dv, sum_hw dv * xhat) with dv = dL/d(pre-activation) -- every
  *               parameter / modulation gradient of the op is a closed form of these (see models.py mirror)

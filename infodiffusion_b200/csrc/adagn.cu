@@ -38,6 +38,7 @@ struct AdaGNParams {
   int c0, c1, C;
   int Hp, Wp, H, W;
   int rows_per_img;
+  int batch;
   int chunk_rows;      // rows per CTA (last CTA of the cluster may have fewer)
   const float* gamma;
   const float* beta;
@@ -306,8 +307,18 @@ __device__ __forceinline__ void fold_coefficients(const AdaGNParams& p, int n, C
     const long long rw = static_cast<long long>(P) * cs;    // record row width
     const float2* stA = reinterpret_cast<const float2*>(first ? p.stats0 : p.stats1) + (first ? ch : ch - p.c0);
     const float2* stB = stA + (first ? p.bwin0 : p.bwin1) * rw;
+    // record of the first unit (B when it starts in image n-1) and of the last window; the records between lie inside
+    // image n (A).  32-row windows follow window_record_of: at R < 32 either end may also hold no rows of image n (-1).
+    int rec_first = first_straddles ? 1 : 0, rec_last = 0;
+    if (S == 1) {
+      const int last_row = p.batch * Rs - 1;
+      rec_first = window_record_of(w_first, n, Rs, last_row);
+      rec_last = window_record_of(w_last, n, Rs, last_row);
+    }
     auto part = [&](int w) -> float2 {
-      const float2* st = ((w < w_bend && first_straddles) ? stB : stA) + static_cast<long long>(w) * rw;
+      const int rec = w < w_bend ? rec_first : (w == w_last ? rec_last : 0);
+      if (rec < 0) return make_float2(0.f, 0.f);
+      const float2* st = (rec ? stB : stA) + static_cast<long long>(w) * rw;
       float2 v = __ldg(st);
       for (int pl = 1; pl < P; ++pl) {                      // parity planes of an up2 producer (fixed order)
         const float2 o = __ldg(st + static_cast<long long>(pl) * cs);
@@ -518,6 +529,7 @@ static cudaError_t fill_params(const idf_adagn_args& a, int c1, AdaGNParams& p) 
   p.C = p.c0 + p.c1;
   p.H = a.H; p.W = a.W; p.Hp = a.H + 1; p.Wp = a.W + 1;
   p.rows_per_img = p.Hp * p.Wp;
+  p.batch = a.batch;
   p.gamma = a.gamma; p.beta = a.beta; p.eps = a.eps;
   p.mod_t = a.mod_t; p.mod_t_step_stride = a.mod_t_step_stride; p.mod_t_batch_stride = a.mod_t_batch_stride;
   p.mod_z = a.mod_z; p.mod_z_step_stride = a.mod_z_step_stride; p.mod_z_batch_stride = a.mod_z_batch_stride;

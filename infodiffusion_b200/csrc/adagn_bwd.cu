@@ -22,7 +22,7 @@ constexpr int kBSlices = 16;   // max row slices per sample (the launcher uses f
 
 struct AdaGNBwdParams {
   const bf16* src0; const bf16* src1;
-  int c0, c1, C, Hp, Wp, H, W, R;
+  int c0, c1, C, Hp, Wp, H, W, R, batch;
   const float* gamma; const float* beta; float eps;
   const float* mod_t; long long mod_t_step_stride, mod_t_batch_stride;
   const float* mod_z; long long mod_z_step_stride, mod_z_batch_stride;
@@ -70,7 +70,7 @@ __device__ void bwd_prologue(const AdaGNBwdParams& p, int n, BwdShared<kMaxC>& s
     return;
   }
   const int w_first = (n * R) / 32, w_last = ((n + 1) * R - 1) / 32;
-  const bool first_straddles = (w_first * 32) < n * R;
+  const int last_row = p.batch * R - 1;
   const int nsub = (kBT / C) > 0 ? (kBT / C) : 1;
   for (int idx = t; idx < C * nsub; idx += kBT) {
     const int ch = idx % C, sub = idx / C;
@@ -78,9 +78,10 @@ __device__ void bwd_prologue(const AdaGNBwdParams& p, int n, BwdShared<kMaxC>& s
     const int cs = first ? p.c0 : p.c1;
     const float2* stA = reinterpret_cast<const float2*>(first ? p.stats0 : p.stats1) + (first ? ch : ch - p.c0);
     const float2* stB = stA + p.stats_b_windows * cs;
-    auto part = [&](int w) -> float2 {
-      const float2* st = (w == w_first && first_straddles) ? stB : stA;
-      return __ldg(st + static_cast<long long>(w) * cs);
+    auto part = [&](int w) -> float2 {       // the window's record that holds image n's rows (window_record_of)
+      const int rec = window_record_of(w, n, R, last_row);
+      if (rec < 0) return make_float2(0.f, 0.f);
+      return __ldg((rec ? stB : stA) + static_cast<long long>(w) * cs);
     };
     float sx = 0.f, sq = 0.f;
     int w = w_first + sub;
@@ -364,7 +365,7 @@ cudaError_t launch_adagn_bwd(const idf_adagn_bwd_args& b, int num_sms, cudaStrea
   AdaGNBwdParams p;
   p.src0 = static_cast<const bf16*>(a.src0); p.src1 = static_cast<const bf16*>(a.src1);
   p.c0 = a.c0; p.c1 = a.src1 ? a.c1 : 0; p.C = p.c0 + p.c1;
-  p.H = a.H; p.W = a.W; p.Hp = a.H + 1; p.Wp = a.W + 1; p.R = p.Hp * p.Wp;
+  p.H = a.H; p.W = a.W; p.Hp = a.H + 1; p.Wp = a.W + 1; p.R = p.Hp * p.Wp; p.batch = a.batch;
   p.gamma = a.gamma; p.beta = a.beta; p.eps = a.eps;
   p.mod_t = a.mod_t; p.mod_t_step_stride = a.mod_t_step_stride; p.mod_t_batch_stride = a.mod_t_batch_stride;
   p.mod_z = a.mod_z; p.mod_z_step_stride = a.mod_z_step_stride; p.mod_z_batch_stride = a.mod_z_batch_stride;

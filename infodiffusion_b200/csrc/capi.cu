@@ -263,6 +263,11 @@ int idf_conv_plan_create(const idf_conv_desc* d, idf_conv_plan** out_plan) {
                   static_cast<int64_t>(p.Hp) * p.Wp >= static_cast<int64_t>(mt) * kBM) ? 1 : 0;
   pl->stats_unit = p.stats_item ? mt * kBM : 32;
   if (p.stats != nullptr && d->out_ld != d->cout) { delete pl; return fail(IDF_ERR_ARG, "stats_out needs out_ld == cout"); }
+  if (p.stats != nullptr && !window_records_exact(d->H, d->W)) {
+    delete pl;
+    return fail(IDF_ERR_ARG, "stats_out: 32-row GroupNorm records cannot keep the images of a %dx%d grid apart "
+                "(needs (H+1)*(W+1) >= 32 or 31 - (H+1)*(W+1) <= W+2)", d->H, d->W);
+  }
   for (int i = 0; i < d->n_src; ++i) {
     rc = encode_2d(&p.tmA[i], d->src[i], d->src_rows[i], d->src_ld[i], kBM);
     if (rc != IDF_OK) { delete pl; return rc; }
@@ -400,8 +405,24 @@ int idf_wgrad_run(const idf_wgrad_plan* plan, idf_stream_t stream) {
   return IDF_OK;
 }
 
+// The producers' 32-row window records of an AdaGN's sources (over this map, or over the half-resolution input grid of
+// an up2 producer) must keep the images apart; otherwise the statistics have to come from the AdaGN kernel itself.
+static int check_records(const idf_adagn_args* a) {
+  const float* st[2] = {a->stats0, a->stats1};
+  const int planes[2] = {a->stats_planes0, a->stats_planes1};
+  for (int i = 0; i < 2; ++i) {
+    const int H = planes[i] > 1 ? a->H / 2 : a->H, W = planes[i] > 1 ? a->W / 2 : a->W;
+    if (st[i] != nullptr && !window_records_exact(H, W))
+      return fail(IDF_ERR_ARG, "stats%d: 32-row GroupNorm records cannot keep the images of a %dx%d grid apart "
+                  "(needs (H+1)*(W+1) >= 32 or 31 - (H+1)*(W+1) <= W+2); pass no statistics", i, H, W);
+  }
+  return IDF_OK;
+}
+
 int idf_adagn_coef(const idf_adagn_args* a, float* coef_out, idf_stream_t stream) {
   if (a == nullptr || coef_out == nullptr) return fail(IDF_ERR_ARG, "null argument");
+  const int rc = check_records(a);
+  if (rc != IDF_OK) return rc;
   cudaError_t e = launch_adagn_coef(*a, coef_out, reinterpret_cast<cudaStream_t>(stream));
   if (e != cudaSuccess) return cuda_fail(e, "adagn_coef launch (needs stats0/stats1, C <= 1024, C % 32 == 0)");
   return IDF_OK;
@@ -409,6 +430,8 @@ int idf_adagn_coef(const idf_adagn_args* a, float* coef_out, idf_stream_t stream
 
 int idf_adagn_silu_fwd(const idf_adagn_args* a, idf_stream_t stream) {
   if (a == nullptr || a->src0 == nullptr || a->out == nullptr) return fail(IDF_ERR_ARG, "null argument");
+  const int rc = check_records(a);
+  if (rc != IDF_OK) return rc;
   cudaError_t e = launch_adagn(*a, reinterpret_cast<cudaStream_t>(stream));
   if (e != cudaSuccess) return cuda_fail(e, "adagn launch");
   return IDF_OK;
@@ -418,6 +441,14 @@ int64_t idf_adagn_bwd_ws_floats(int32_t batch, int32_t C) { return adagn_bwd_ws_
 
 int idf_adagn_silu_bwd(const idf_adagn_bwd_args* b, idf_stream_t stream) {
   if (b == nullptr) return fail(IDF_ERR_ARG, "null argument");
+  if (b->f.save_coef == nullptr) {           // the statistics come from the records
+    const idf_adagn_args& f = b->f;
+    if (f.stats_unit0 > 32 || f.stats_unit1 > 32 || f.stats_planes0 > 1 || f.stats_planes1 > 1)
+      return fail(IDF_ERR_ARG, "adagn backward: without save_coef the statistics must be 32-row window records of this map "
+                  "(stats_unit 32, no up2 planes)");
+    const int rc = check_records(&f);
+    if (rc != IDF_OK) return rc;
+  }
   cudaError_t e = launch_adagn_bwd(*b, g_num_sms, reinterpret_cast<cudaStream_t>(stream));
   if (e != cudaSuccess) return cuda_fail(e, "adagn backward launch (needs stats0/stats1, dy, dx, sums, ws; C <= 1024, C % 32 == 0)");
   return IDF_OK;

@@ -181,8 +181,9 @@ __device__ __forceinline__ void epilogue_drain_chunk(const ConvKernelParams& p, 
 // GroupNorm partial sums of one staged (bf16-rounded) 32 x 32 tile, taken by a statistics warp (all 32 lanes), so the
 // drain warps only move data: column sums written per tile and lane quarter (no cross-warp exchange, fixed summation
 // order => deterministic):
-//   statsA[(tile*4 + q)][col] = (sum, sumsq) over the window's rows in the image of its first row,
-//   statsB[(tile*4 + q)][col] = the same over the rows that already belong to the next image
+//   statsA[(tile*4 + q)][col] = (sum, sumsq) over the window's rows before its last image boundary (all of them when
+//                               it has none),
+//   statsB[(tile*4 + q)][col] = the same over the rows from that boundary on
 //                               (written only when the 32-row window straddles an image boundary).
 __device__ __forceinline__ void epilogue_stats_chunk(const ConvKernelParams& p, uint32_t stage, int col0, int n_a, int tile,
                                                      int q, int lane, uint64_t* staged, uint64_t* sdone, uint32_t use) {
@@ -869,9 +870,12 @@ __global__ void __launch_bounds__(conv_threads(XF), 1) conv_halo_kernel(const __
         for (int m = 0; m < MT; ++m) {
           const int tile = ms * MT + m;
           const int64_t wr0 = static_cast<int64_t>(tile) * kBM + q * 32;
-          const int img_w = __float2int_rd((static_cast<float>(wr0) + 0.5f) * inv_R);
-          const int64_t next_img_row = static_cast<int64_t>(img_w + 1) * R;
-          const int n_a = static_cast<int>((next_img_row - wr0 < 32) ? (next_img_row - wr0) : 32);
+          // split at the window's LAST image boundary: with R < 32 a window can touch three images, and the rows before
+          // an earlier boundary are then pad rows (zeros; the plan rejects geometries where they are not)
+          const int64_t wr_last = (wr0 + 31 < p.rows) ? wr0 + 31 : p.rows - 1;
+          const int img_l = __float2int_rd((static_cast<float>(wr_last) + 0.5f) * inv_R);
+          const int64_t last_bnd = static_cast<int64_t>(img_l) * R;
+          const int n_a = last_bnd > wr0 ? static_cast<int>(last_bnd - wr0) : 32;
 #pragma unroll 1
           for (int c = 0; c < CHUNKS; ++c, k += (c & 1) ? 0u : 1u) {     // chunk c belongs to drain warp (c & 1) * 4 + q
             const uint32_t sl = 2u * ((c & 1) * 4 + q) + (k & 1u);

@@ -12,6 +12,26 @@ constexpr int kBK = 64;   // K elements per k-block == one 128-byte swizzle row
 
 constexpr int kMaxGroups = 40;   // halo loads per work item: (source, 64-channel slice, tap cluster); 1024 + 1024 channels = 32
 
+// GroupNorm window records (conv epilogue, unit = 32 rows): a window w (rows 32w .. 32w+31 of a pad-flat map with R rows
+// per image) is split at its LAST image boundary b: record A = rows before b, record B = rows from b on; A belongs to
+// image (b-1)/R, B to image b/R (no boundary: A alone, image of the window).  With R < 32 a window may hold rows of
+// three images; the two records keep every image apart only if the rows before an earlier boundary are pad rows --
+// an image ends in W + 2 of them (column W of row H-1, then row H), so that needs 31 - R <= W + 2.
+__host__ __device__ __forceinline__ bool window_records_exact(int H, int W) {
+  const int R = (H + 1) * (W + 1);
+  return R >= 32 || 31 - R <= W + 2;
+}
+// Which record of window w holds rows of image n: 0 = A, 1 = B, -1 = neither.  last_row = batch * R - 1.
+__device__ __forceinline__ int window_record_of(int w, int n, int R, int last_row) {
+  const int lo = 32 * w;
+  const int hi = min(lo + 31, last_row);
+  const int b0 = n * R, b1 = b0 + R, b2 = b1 + R;   // boundaries at the start of images n, n+1, n+2
+  if (lo < b0 && b0 <= hi && b1 > hi) return 1;     // last boundary of the window starts image n
+  if (lo < b1 && b1 <= hi && b2 > hi) return 0;     // last boundary starts image n+1: A holds image n's rows
+  if (lo >= b0 && b1 > hi) return 0;                // no boundary, the window lies in image n
+  return -1;
+}
+
 struct alignas(64) ConvKernelParams {
   CUtensorMap tmA[IDF_CONV_MAX_SRC];    // box {64, 128 rows}
   CUtensorMap tmAx[IDF_CONV_MAX_SRC];   // box {64, extra_rows[src]} -- tail of the halo

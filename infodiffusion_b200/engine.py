@@ -34,7 +34,7 @@ import torch.nn as nn
 from . import _lib
 from ._lib import EPI_BF16, EPI_F32_NCHW, EPI_SAMPLER, AdaGNArgs, ConvDesc
 from .layout import (ParamIndex, pack_conv1x1, pack_conv3x3, pack_conv3x3_up2, pad_cols as _pad_cols, pad_rows as _pad_rows,
-                     probing, pv, tap_offsets3x3, taps_stride2, taps_up2)
+                     probing, pv, tap_offsets3x3, taps_stride2, taps_up2, window_records_exact)
 from .modules import AttnBlock, AuxResBlock, DownSample, ResBlock, UpSample, timestep_embedding
 
 BF16 = torch.bfloat16
@@ -319,6 +319,7 @@ class Plan:
         if out is not None:
             assert out.H == (2 * H if up2 else H) and out.C == cout
             d.out, d.out_ld = out.t.data_ptr(), out.C
+            want_stats = want_stats and window_records_exact(H, H)     # records over the GEMM grid (up2: the input)
             if want_stats:
                 # (an up2 plan writes records over the input grid's tiles, 4 parity planes wide)
                 tiles_in = (self.B * (H + 1) * (H + 1) + 127) // 128

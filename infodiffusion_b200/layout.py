@@ -43,6 +43,31 @@ def taps_stride2(cin: int, Ho: int, Wo: int, phase_rows: int, src: int = 0) -> L
     return kb
 
 
+def stride2_phase_dgrad(cout: int, Ho: int, Wo: int, src: int = 0) -> List[Tuple[int, List[Tuple[int, int]], List[KBlock]]]:
+    """Data gradient of the stride-2 conv above, one implicit GEMM per space-to-depth phase (py, px): the taps (ky, kx)
+    that read that phase and their K-blocks over dY (negated row offsets, K ordered (tap, cout)).  Returns
+    [(phase = py*2 + px, taps, k-blocks)]; the weights of phase p are cat([W[:, :, ky, kx]^T for (ky, kx) in taps], 1)."""
+    sel = {0: (1, -1), 1: (0, 0), 2: (1, 0)}
+    out = []
+    for py in (0, 1):
+        for px in (0, 1):
+            taps = [(ky, kx) for ky in range(3) for kx in range(3) if sel[ky][0] == py and sel[kx][0] == px]
+            kb: List[KBlock] = []
+            for ky, kx in taps:
+                off = sel[ky][1] * (Wo + 1) + sel[kx][1]
+                kb += [(src, c0, -off) for c0 in range(0, cout, 64)]
+            out.append((py * 2 + px, taps, kb))
+    return out
+
+
+def window_records_exact(H: int, W: int) -> bool:
+    """Whether the conv epilogue's 32-row GroupNorm records (idf_conv_desc.stats_out) keep the images of an H x W
+    pad-flat grid apart (mirror of window_records_exact in csrc/kernels.cuh): false for H = W <= 3, where
+    idf_conv_plan_create rejects stats_out."""
+    R = (H + 1) * (W + 1)
+    return R >= 32 or 31 - R <= W + 2
+
+
 def taps1x1(cin: int, src: int = 0) -> List[KBlock]:
     return [(src, c0, 0) for c0 in range(0, cin, 64)]
 

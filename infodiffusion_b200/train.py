@@ -34,7 +34,7 @@ import torch.nn as nn
 
 from . import _lib
 from ._lib import EPI_F32_NCHW, AdaGNBwdArgs, WgradDesc
-from .layout import pad_rows, pv, tap_offsets3x3, taps_stride2
+from .layout import pad_rows, pv, stride2_phase_dgrad, tap_offsets3x3, taps_stride2
 
 BF16 = torch.bfloat16
 
@@ -325,22 +325,14 @@ def bwd_downsample(plan, src, ph, conv: nn.Conv2d, out) -> None:
     rows_o = out.rows
     dph_t = torch.zeros_like(ph.t)
     st.keep.append(dph_t)
-    sel = {0: (1, -1), 1: (0, 0), 2: (1, 0)}
     w = conv.weight
-    for py in (0, 1):
-        for px in (0, 1):
-            taps = [(ky, kx) for ky in range(3) for kx in range(3) if sel[ky][0] == py and sel[kx][0] == px]
-            kb = []
-            for ky, kx in taps:
-                off = sel[ky][1] * (Ho + 1) + sel[kx][1]
-                kb += [(0, c0, -off) for c0 in range(0, cout, 64)]
-            phase = py * 2 + px
-            tgt = Act(dph_t[phase * rows_o:(phase + 1) * rows_o], Ho, Cc, 1, rows_o)
-            st.keep.append(tgt)
-            st.grads[id(tgt)] = tgt              # the phase slice IS the gradient buffer of this pseudo-activation
-            st.written[id(tgt)] = False
-            _dgrad(plan, st, dout, tgt, kb,
-                   lambda taps=taps: torch.cat([pv(w)[:, :, ky, kx].t() for ky, kx in taps], dim=1), Cc)
+    for phase, taps, kb in stride2_phase_dgrad(cout, Ho, Ho):
+        tgt = Act(dph_t[phase * rows_o:(phase + 1) * rows_o], Ho, Cc, 1, rows_o)
+        st.keep.append(tgt)
+        st.grads[id(tgt)] = tgt              # the phase slice IS the gradient buffer of this pseudo-activation
+        st.written[id(tgt)] = False
+        _dgrad(plan, st, dout, tgt, kb,
+               lambda taps=taps: torch.cat([pv(w)[:, :, ky, kx].t() for ky, kx in taps], dim=1), Cc)
     g = st.grad(src)
     st.kernel(plan.lib.idf_depth_to_space, dph_t.data_ptr(), g.t.data_ptr(), plan.B, src.H, src.H, Cc,
               1 if st.is_written(src) else 0)
