@@ -26,6 +26,7 @@ Fusions relative to the reference's one-op-per-kernel execution (modules.py / mo
 from __future__ import annotations
 
 import ctypes as C
+from dataclasses import dataclass
 from typing import Dict, List, Optional, Sequence, Tuple
 
 import torch
@@ -126,6 +127,46 @@ class Workspace:
 
 
 # ------------------------------------------------------------------------------------------------
+# op records and their runner
+# ------------------------------------------------------------------------------------------------
+@dataclass
+class Op:
+    """One launch of a plan: `fn(*args, stream)` is a library call that launches `kernels` kernels; with kernels = 0
+    it is a torch op, `fn(*args)` on the current stream.  `side`: a leaf of the backward graph (weight / bias
+    gradient) that may run on the side stream."""
+    tag: str
+    fn: object
+    args: tuple
+    kernels: int = 1
+    flops: int = 0
+    bytes: int = 0
+    side: bool = False
+
+
+def run_ops(ops: Sequence[Op], device, side: Optional[torch.cuda.Stream] = None) -> None:
+    """Enqueue `ops` in order on the current stream, check every return code and count the declared kernels.  With a
+    `side` stream, each op marked `side` runs there after everything enqueued before it; the side stream is joined
+    at the end."""
+    main = torch.cuda.current_stream(device)
+    stream, side_stream = main.cuda_stream, side.cuda_stream if side is not None else None
+    if side is not None:
+        side.wait_stream(main)
+    n = 0
+    for op in ops:
+        if not op.kernels:
+            op.fn(*op.args)
+        elif op.side and side is not None:
+            side.wait_stream(main)
+            _lib.check(op.fn(*op.args, side_stream))
+        else:
+            _lib.check(op.fn(*op.args, stream))
+        n += op.kernels
+    if side is not None:
+        main.wait_stream(side)
+    _lib.count_launch(n)
+
+
+# ------------------------------------------------------------------------------------------------
 # plan builder
 # ------------------------------------------------------------------------------------------------
 class _GatherArena:
@@ -170,7 +211,8 @@ class _GatherArena:
 class Plan:
     """Ordered list of kernel launches + everything they reference."""
 
-    def __init__(self, batch: int, device, ws: Optional[Workspace] = None, training: bool = False):
+    def __init__(self, batch: int, device, ws: Optional[Workspace] = None, training: bool = False,
+                 ordered: bool = False):
         self.lib = _lib.load()
         _lib.check(self.lib.idf_init())
         self.B = batch
@@ -184,13 +226,16 @@ class Plan:
         self.fuse_adagn = FUSE_ADAGN and not training
         self.ws = ws if ws is not None else Workspace(batch, device, recycle=not training)
         self.tape: List = []         # training: backward emitters, one per forward composite, replayed in reverse
+        self.bwd = None              # training: the backward op lists (infodiffusion_b200.train.BwdState)
+        if training:
+            from .train import BwdState
+            self.bwd = BwdState(self, ordered)
         self.pindex: Optional[ParamIndex] = None   # training: flat parameter layout the packing gathers read
         self.recipes: List = []      # training: (packed tensor, recipe) pairs (kept for verification)
         self.dropout_p = 0.0
         self.dropout_seed = None     # device int64 scalar
         self._drop_layers = 0
-        self.ops: List = []          # (callable, args tuple); last arg slot is the stream
-        self.meta: List[dict] = []   # per op: kernel class, algorithmic flops / bytes
+        self.ops: List[Op] = []
         self.keep: List = []         # tensors / ctypes structs that must outlive the plan
         self.conv_plans: List[int] = []
         self.flops = 0               # algorithmic conv/attention FLOPs of one run
@@ -204,11 +249,14 @@ class Plan:
         except Exception:
             pass
 
-    def _emit(self, tag: str, fn, args: tuple, flops: int = 0, nbytes: int = 0) -> None:
-        self.ops.append((fn, args))
-        self.meta.append(dict(tag=tag, flops=flops, bytes=nbytes))
-        self.flops += flops
-        self.adagn_bytes += nbytes if tag == "adagn" else 0
+    def _emit(self, tag: str, fn, args: tuple, flops: int = 0, nbytes: int = 0, emit: bool = True) -> Op:
+        """Record one launch; with emit=False the record is only returned (backward ops, kept outside this plan)."""
+        op = Op(tag, fn, args, flops=flops, bytes=nbytes)
+        if emit:
+            self.ops.append(op)
+            self.flops += flops
+            self.adagn_bytes += nbytes if tag == "adagn" else 0
+        return op
 
     # ---- execution -----------------------------------------------------------------------------
     def run_timed(self, run_ahead_ms: float = 8.0) -> List[Tuple[str, float, int, int]]:
@@ -221,20 +269,14 @@ class Plan:
         if run_ahead_ms > 0:
             torch.cuda._sleep(int(run_ahead_ms * 1.9e6))          # cycles at ~1.9 GHz
         evs[0].record(st)
-        for i, (fn, args) in enumerate(self.ops):
-            _lib.check(fn(*args, st.cuda_stream))
+        for i, op in enumerate(self.ops):
+            run_ops([op], self.device)
             evs[i + 1].record(st)
         st.synchronize()
-        _lib.count_launch(len(self.ops))
-        return [(m["tag"], evs[i].elapsed_time(evs[i + 1]), m["flops"], m["bytes"]) for i, m in enumerate(self.meta)]
+        return [(op.tag, evs[i].elapsed_time(evs[i + 1]), op.flops, op.bytes) for i, op in enumerate(self.ops)]
 
-    def run(self, stream: Optional[int] = None) -> None:
-        if stream is None:
-            stream = torch.cuda.current_stream(self.device).cuda_stream
-        check = _lib.check
-        for fn, args in self.ops:
-            check(fn(*args, stream))
-        _lib.count_launch(len(self.ops))
+    def run(self) -> None:
+        run_ops(self.ops, self.device)
 
     # ---- op emitters ---------------------------------------------------------------------------
     def weight(self, m) -> torch.Tensor:
@@ -275,28 +317,24 @@ class Plan:
         self._arena_bf16 = _GatherArena(BF16, int(2.3 * total) + (4 << 20), self.device)
         self._arena_f32 = _GatherArena(torch.float32, 1 << 20, self.device)
 
-    def refresh_weights(self) -> None:
+    def refresh_ops(self) -> List[Op]:
         """flat_params <- parameters (one multi-tensor copy), then one gather launch per arena chunk."""
-        if self.pindex is None:
-            return
-        with torch.no_grad():
-            torch._foreach_copy_(self._flat_views, [p.detach() for p in self.pindex.params])
-        stream = torch.cuda.current_stream(self.device).cuda_stream
-        n = 0
+        ops = [Op("param_copy", torch._foreach_copy_, (self._flat_views, [p.detach() for p in self.pindex.params]),
+                  kernels=0)]
         for arena in (self._arena_bf16, self._arena_f32):
             for buf, idx, idx2, used in arena.chunks():
-                _lib.check(self.lib.idf_gather_elems(self.flat_params.data_ptr(), idx.data_ptr(),
-                                                     idx2.data_ptr() if idx2 is not None else None, buf.data_ptr(),
-                                                     used, 1 if arena.dtype == BF16 else 0, 0, stream))
-                n += 1
-        _lib.count_launch(n)
+                ops.append(Op("repack", self.lib.idf_gather_elems,
+                              (self.flat_params.data_ptr(), idx.data_ptr(), idx2.data_ptr() if idx2 is not None else None,
+                               buf.data_ptr(), used, 1 if arena.dtype == BF16 else 0, 0)))
+        return ops
 
     def conv(self, srcs: Sequence[Act], kblocks: Sequence[Tuple[int, int, int]], wp: torch.Tensor,
              bias: torch.Tensor, H: int, cout: int, block_n: int, out: Optional[Act] = None,
              residual: Optional[Act] = None, epilogue: int = EPI_BF16, out_f32=None, x_io=None, noise=None,
              coef=None, step=None, real_macs_per_row: Optional[int] = None, want_stats: bool = True,
-             xf: Optional[Tuple[torch.Tensor, bool, Sequence[int]]] = None, up2: bool = False) -> None:
-        """`xf` = (coefficients [B, Ctot, 2], silu?, per-k-block channel base or -1): fused AdaGN on the A operand."""
+             xf: Optional[Tuple[torch.Tensor, bool, Sequence[int]]] = None, up2: bool = False, emit: bool = True) -> Op:
+        """`xf` = (coefficients [B, Ctot, 2], silu?, per-k-block channel base or -1): fused AdaGN on the A operand.
+        Returns the launch record (appended to this plan unless emit=False)."""
         d = ConvDesc()
         d.n_src = len(srcs)
         for i, s in enumerate(srcs):
@@ -346,10 +384,10 @@ class Plan:
         macs = real_macs_per_row if real_macs_per_row is not None else 64 * len(kblocks) * cout
         # conv_igemm_xf: the launches that also apply a fused AdaGN (+SiLU) to their A operand -- they replace a
         # stand-alone AdaGN pass and are accounted separately from the plain implicit GEMMs
-        self._emit("conv_igemm_xf" if xf is not None else "conv_igemm", self.lib.idf_conv_run, (h,),
-                   flops=2 * self.B * H * H * macs,
-                   nbytes=(2 * 2 * self.B * H * H * 64 * len({(si, c0) for (si, c0, _), v in zip(kblocks, xf[2]) if v >= 0})
-                           if xf is not None else 0))       # HBM bytes of the AdaGN pass this launch replaces
+        return self._emit("conv_igemm_xf" if xf is not None else "conv_igemm", self.lib.idf_conv_run, (h,),
+                          flops=2 * self.B * H * H * macs,
+                          nbytes=(2 * 2 * self.B * H * H * 64 * len({(si, c0) for (si, c0, _), v in zip(kblocks, xf[2]) if v >= 0})
+                                  if xf is not None else 0), emit=emit)   # HBM bytes of the AdaGN pass this launch replaces
 
     def norm(self, src0: Act, src1: Optional[Act], gn: nn.GroupNorm, silu: bool, mod_t=None, mod_z=None, step=None,
              dropout: bool = False, mod_cols: Optional[int] = None):
@@ -732,8 +770,8 @@ class BackbonePlan(Plan):
                  coef: Optional[torch.Tensor] = None, step: Optional[torch.Tensor] = None,
                  mod_t_table: Optional[torch.Tensor] = None, mod_z: Optional[torch.Tensor] = None,
                  eps_out: Optional[torch.Tensor] = None, pack: Optional[ModulationPack] = None,
-                 dropout_p: float = 0.0):
-        super().__init__(batch, device, ws, training=(mode == "train"))
+                 dropout_p: float = 0.0, ordered: bool = False):
+        super().__init__(batch, device, ws, training=(mode == "train"), ordered=ordered)
         assert mode in ("eps", "sampler", "train")
         self.mode = mode
         Cimg, H, W = net.shape
@@ -819,8 +857,9 @@ class EncoderPlan(Plan):
     a_q = mu + latent_noise * exp(0.5 * log_var) (models.py:515) into self.a_q."""
 
     def __init__(self, net, batch: int, device, ws: Optional[Workspace] = None, x_in: Optional[torch.Tensor] = None,
-                 training: bool = False, dropout_p: float = 0.0, latent_noise: Optional[torch.Tensor] = None):
-        super().__init__(batch, device, ws, training=training)
+                 training: bool = False, dropout_p: float = 0.0, latent_noise: Optional[torch.Tensor] = None,
+                 ordered: bool = False):
+        super().__init__(batch, device, ws, training=training, ordered=ordered)
         Cimg, H, W = net.shape
         assert H == W and H in (32, 64)
         B = batch

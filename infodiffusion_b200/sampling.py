@@ -145,7 +145,7 @@ class _FusedSampler:
             self.lane_plans[lane] += self.plans[n_before:]
         self.ws = self.lane_ws[0]
         self.graph: Optional[torch.cuda.CUDAGraph] = None
-        self.n_launch = sum(len(p.ops) for p in self.plans)
+        self.n_launch = sum(op.kernels for p in self.plans for op in p.ops)
 
     def set_latent(self, a: torch.Tensor) -> None:
         self.tables.latent_rows(a.contiguous().float(), self.mod_z)
@@ -404,7 +404,7 @@ class LatentDiffusionProcess():
         if s.graph is None:
             s.graph = _capture_step(s.plan.run, s.x, s.step, idx)
         s.graph.replay()
-        _lib.count_launch(len(s.plan.ops))
+        _lib.count_launch(sum(op.kernels for op in s.plan.ops))
 
     def _iter(self, kind: str, x: torch.Tensor):
         T = len(self.alpha_bars)

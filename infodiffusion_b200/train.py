@@ -34,6 +34,8 @@ import torch.nn as nn
 
 from . import _lib
 from ._lib import EPI_F32_NCHW, AdaGNBwdArgs, WgradDesc
+from .engine import (Act, BackbonePlan, EncoderPlan, Op, _require_cuda, conditioned_blocks, modulation_weights,
+                     run_ops)
 from .layout import pad_rows, pv, stride2_phase_dgrad, tap_offsets3x3, taps_stride2
 
 BF16 = torch.bfloat16
@@ -73,9 +75,10 @@ class Part:
 
 
 class BwdState:
-    def __init__(self, plan):
+    def __init__(self, plan, ordered: bool):
         self.plan = plan
-        self.ops: List[Callable[[], None]] = []          # executed in order by run_backward
+        self.ops: List[Op] = []          # run in order by run_backward; callable args are resolved by finalize_backward
+        self.gathers: List[Op] = []      # arena -> parameter-shaped gradients, after the side stream has joined
         self.grads: Dict[int, object] = {}               # id(Act) -> gradient Act
         self.written: Dict[int, bool] = {}
         self.flat_chunks: List[Tuple[int, int]] = []     # (offset, numel) of fp32 grad buffers in the flat arena
@@ -84,11 +87,10 @@ class BwdState:
         self.views: List = []                            # (name, offset, shape) resolved after allocation
         self.param_grads: List[Tuple[nn.Parameter, Callable[[], torch.Tensor]]] = []
         self.keep: List = []
-        self.wplans: List = []
-        self.late: List[Callable[[], None]] = []        # pointer fix-ups once the fp32 arena exists
-        self.side: set = set()       # indices of ops that nothing later in the list depends on (weight / bias gradients)
-        self.side_stream: Optional[torch.cuda.Stream] = None
-        self.ordered = bool(getattr(plan, "ordered", False))
+        self.wplans: List = []                           # (desc, handle, arena getter, op)
+        self.side_stream = torch.cuda.Stream(plan.device)
+        self.ordered = ordered
+        self.final = False
         self.side_ws_floats = 0      # ordered: largest colsum workspace (the wgrad partials are sized once the plans exist)
         self.main_ws_floats = 0      # ordered: largest AdaGN dgamma / dbeta workspace
         self.side_ws: Optional[torch.Tensor] = None
@@ -97,7 +99,7 @@ class BwdState:
 
     def __del__(self):
         try:
-            for _, h, _ in self.wplans:
+            for _, h, _, _ in self.wplans:
                 if h:
                     self.plan.lib.idf_wgrad_plan_destroy(h)
         except Exception:
@@ -116,7 +118,6 @@ class BwdState:
     def grad(self, act):
         g = self.grads.get(id(act))
         if g is None:
-            from .engine import Act
             t = torch.zeros_like(act.t)
             g = Act(t, act.H, act.C, act.phases, act.rows)
             self.grads[id(act)] = g
@@ -130,19 +131,9 @@ class BwdState:
     def mark(self, act) -> None:
         self.written[id(act)] = True
 
-    def kernel(self, fn, *args) -> None:
-        dev = self.plan.device
-
-        def run():
-            _lib.check(fn(*args, torch.cuda.current_stream(dev).cuda_stream))
-            _lib.count_launch()
-        self.ops.append(run)
-
-
-def _state(plan) -> BwdState:
-    if not hasattr(plan, "_bwd"):
-        plan._bwd = BwdState(plan)
-    return plan._bwd
+    def op(self, tag: str, fn, *args, kernels: int = 1, side: bool = False) -> Op:
+        self.ops.append(Op(tag, fn, args, kernels, side=side))
+        return self.ops[-1]
 
 
 # ------------------------------------------------------------------------------------------------
@@ -152,17 +143,11 @@ def _dgrad(plan, st: BwdState, dout, target, kblocks, wrecipe, cin: int) -> None
     """grad(target) (+)= implicit GEMM over dout with the given (negated-tap) K-blocks and [cin, K] weights."""
     g = st.grad(target)
     acc = st.is_written(target)
-    # emit into a scratch op list, then move the launch into the backward list
-    n0 = len(plan.ops)
     wp = plan.weight(wrecipe)
     zero_bias = torch.zeros(wp.shape[0], dtype=torch.float32, device=plan.device)
     plan.keep.append(zero_bias)
-    plan.conv([dout], kblocks, wp, zero_bias, target.H, cin, plan._bn(cin), out=g, residual=g if acc else None,
-              want_stats=False)
-    fn, args = plan.ops.pop()
-    plan.meta.pop()
-    assert len(plan.ops) == n0
-    st.kernel(fn, *args)
+    st.ops.append(plan.conv([dout], kblocks, wp, zero_bias, target.H, cin, plan._bn(cin), out=g,
+                            residual=g if acc else None, want_stats=False, emit=False))
     st.mark(target)
 
 
@@ -175,27 +160,21 @@ def _wgrad(plan, st: BwdState, dout, x, x_rows: int, cin: int, cout: int, tap_of
     d.n_taps = len(tap_off)
     for i, o in enumerate(tap_off):
         d.tap_off[i] = o
-    h = C.c_void_p()
+    h = C.c_void_p()                         # created once the arena is allocated (needs the dw pointer)
     st.keep.append(d)
-    st.wplans.append((d, h, get))           # created once the arena is allocated (needs the dw pointer)
-    st.side.add(len(st.ops))                 # leaf of the backward graph: runs on the side stream
-    st.ops.append(lambda: (_lib.check(plan.lib.idf_wgrad_run(h, torch.cuda.current_stream(plan.device).cuda_stream)),
-                           _lib.count_launch(2 if d.partials else 1)))       # ordered split-K: + the slab reduction
+    st.wplans.append((d, h, get, st.op("wgrad", plan.lib.idf_wgrad_run, h, side=True)))
     return get
 
 
 def _bias_grad(plan, st: BwdState, dout, cout: int):
     get = st.arena((cout,))
-    st.side.add(len(st.ops))
+    args = (dout.t.data_ptr(), lambda: get().data_ptr(), dout.rows, cout)
     if st.ordered:
         st.side_ws_floats = max(st.side_ws_floats, int(plan.lib.idf_colsum_ws_floats(dout.rows, cout)))
-        st.ops.append(lambda: (_lib.check(plan.lib.idf_colsum_bf16_ordered(
-            dout.t.data_ptr(), get().data_ptr(), dout.rows, cout, st.side_ws.data_ptr(), st.tickets.data_ptr(),
-            torch.cuda.current_stream(plan.device).cuda_stream)), _lib.count_launch()))
-        return get
-    st.ops.append(lambda: (_lib.check(plan.lib.idf_colsum_bf16(dout.t.data_ptr(), get().data_ptr(), dout.rows, cout,
-                                                               torch.cuda.current_stream(plan.device).cuda_stream)),
-                           _lib.count_launch()))
+        st.op("colsum", plan.lib.idf_colsum_bf16_ordered, *args, lambda: st.side_ws.data_ptr(),
+              lambda: st.tickets.data_ptr(), side=True)
+    else:
+        st.op("colsum", plan.lib.idf_colsum_bf16, *args, side=True)
     return get
 
 
@@ -203,15 +182,15 @@ def _add_into(plan, st: BwdState, src, target) -> None:
     """grad(target) (+)= src  (identity / residual paths), plain torch elementwise on bf16 buffers."""
     g = st.grad(target)
     if st.is_written(target):
-        st.ops.append(lambda: g.t.add_(src.t))
+        st.op("add", g.t.add_, src.t, kernels=0)
     else:
-        st.ops.append(lambda: g.t.copy_(src.t))
+        st.op("copy", g.t.copy_, src.t, kernels=0)
     st.mark(target)
 
 
 def bwd_conv(plan, parts: Sequence[Part], biases: Sequence[nn.Parameter], out, residual) -> None:
     """conv3x3 (+ fused 1x1 shortcut parts) (+ identity residual)."""
-    st = _state(plan)
+    st = plan.bwd
     dout = st.grad(out)
     H, cout = out.H, out.C
     offs = tap_offsets3x3(H, H)
@@ -242,7 +221,7 @@ def bwd_conv(plan, parts: Sequence[Part], biases: Sequence[nn.Parameter], out, r
 
 def bwd_conv1x1_stack(plan, src, convs: Sequence[nn.Conv2d], out, residual) -> None:
     """1x1 conv(s) stacked along N (qkv / proj)."""
-    st = _state(plan)
+    st = plan.bwd
     dout = st.grad(out)
     cout, cin = out.C, src.C
     kb = [(0, c0, 0) for c0 in range(0, cout, 64)]
@@ -264,7 +243,7 @@ def bwd_head(plan, patches, conv: nn.Conv2d, out, Cimg: int) -> None:
     Cimg <- cout 3x3 conv over dY (negated taps, transposed weights, fp32 NCHW out: the tail's forward shape) whose
     conv plan is kept on the training plan as `dx_op`; _ConvStackFn.backward launches it only when the input
     requires grad, so a step without input gradient keeps its launch list."""
-    st = _state(plan)
+    st = plan.bwd
     dout = st.grad(out)
     cout, H = out.C, out.H
     get = _wgrad(plan, st, dout, patches, patches.t.shape[0], 64, cout, [0])
@@ -277,30 +256,26 @@ def bwd_head(plan, patches, conv: nn.Conv2d, out, Cimg: int) -> None:
     zero_bias = torch.zeros(wp.shape[0], dtype=torch.float32, device=plan.device)
     plan.d_x = torch.zeros(plan.B, Cimg, H, H, dtype=torch.float32, device=plan.device)
     plan.keep.append(zero_bias)
-    plan.conv([dout], kb, wp, zero_bias, H, Cimg, 16, epilogue=EPI_F32_NCHW, out_f32=plan.d_x)
-    plan.dx_op = plan.ops.pop()
-    plan.meta.pop()
+    plan.dx_op = plan.conv([dout], kb, wp, zero_bias, H, Cimg, 16, epilogue=EPI_F32_NCHW, out_f32=plan.d_x, emit=False)
 
 
 def run_input_grad(plan) -> torch.Tensor:
     """d_x of the plan's input from the head output's gradient the last backward left (see bwd_head)."""
-    fn, args = plan.dx_op
-    _lib.check(fn(*args, torch.cuda.current_stream(plan.device).cuda_stream))
-    _lib.count_launch()
+    run_ops([plan.dx_op], plan.device)
     return plan.d_x.clone()
 
 
 def bwd_tail(plan, ta, tconv: nn.Conv2d, out_f32: torch.Tensor, cout: int) -> None:
     """tail conv (fp32 NCHW output): dY arrives as fp32 NCHW in plan.d_out, is re-laid out to a 64-channel
     pad-flat bf16 matrix (channels >= cout zero) and then treated like any other conv gradient."""
-    st = _state(plan)
-    from .engine import Act
+    st = plan.bwd
     H, cin = ta.H, ta.C
     rows = ta.rows
     dpf = Act(torch.zeros(rows, 64, dtype=BF16, device=plan.device), H, 64, 1, rows)
     st.keep.append(dpf)
     plan.d_out = torch.zeros_like(out_f32)
-    st.kernel(plan.lib.idf_nchw_to_padflat_ld, plan.d_out.data_ptr(), dpf.t.data_ptr(), plan.B, cout, H, H, 64)
+    st.op("nchw_to_padflat", plan.lib.idf_nchw_to_padflat_ld, plan.d_out.data_ptr(), dpf.t.data_ptr(), plan.B, cout, H, H,
+          64)
     offs = tap_offsets3x3(H, H)
     kb = [(0, 0, -off) for off in offs]
 
@@ -318,8 +293,7 @@ def bwd_tail(plan, ta, tconv: nn.Conv2d, out_f32: torch.Tensor, cout: int) -> No
 
 def bwd_downsample(plan, src, ph, conv: nn.Conv2d, out) -> None:
     """stride-2 conv over space-to-depth phases: one data-gradient GEMM per phase, then depth-to-space."""
-    st = _state(plan)
-    from .engine import Act
+    st = plan.bwd
     dout = st.grad(out)
     Ho, Cc, cout = out.H, src.C, out.C
     rows_o = out.rows
@@ -334,8 +308,8 @@ def bwd_downsample(plan, src, ph, conv: nn.Conv2d, out) -> None:
         _dgrad(plan, st, dout, tgt, kb,
                lambda taps=taps: torch.cat([pv(w)[:, :, ky, kx].t() for ky, kx in taps], dim=1), Cc)
     g = st.grad(src)
-    st.kernel(plan.lib.idf_depth_to_space, dph_t.data_ptr(), g.t.data_ptr(), plan.B, src.H, src.H, Cc,
-              1 if st.is_written(src) else 0)
+    st.op("depth_to_space", plan.lib.idf_depth_to_space, dph_t.data_ptr(), g.t.data_ptr(), plan.B, src.H, src.H, Cc,
+          1 if st.is_written(src) else 0)
     st.mark(src)
     offs = [o for (_, _, o) in taps_stride2(64, Ho, Ho, rows_o)]      # one offset per tap (cin = 64 -> one chunk)
     get = _wgrad(plan, st, dout, ph, ph.t.shape[0], Cc, cout, offs)
@@ -344,17 +318,17 @@ def bwd_downsample(plan, src, ph, conv: nn.Conv2d, out) -> None:
 
 
 def bwd_upsample(plan, src, up) -> None:
-    st = _state(plan)
+    st = plan.bwd
     dup = st.grad(up)
     g = st.grad(src)
-    st.kernel(plan.lib.idf_upsample2x_bwd, dup.t.data_ptr(), g.t.data_ptr(), plan.B, src.H, src.H, src.C,
-              1 if st.is_written(src) else 0)
+    st.op("upsample2x_bwd", plan.lib.idf_upsample2x_bwd, dup.t.data_ptr(), g.t.data_ptr(), plan.B, src.H, src.H, src.C,
+          1 if st.is_written(src) else 0)
     st.mark(src)
 
 
 def bwd_adagn(plan, a, src0, src1, out, gn: nn.GroupNorm, gamma: torch.Tensor, beta: torch.Tensor,
               mod_cols: Optional[int]) -> None:
-    st = _state(plan)
+    st = plan.bwd
     dy = st.grad(out)
     Cc = out.C
     b = AdaGNBwdArgs()
@@ -377,12 +351,15 @@ def bwd_adagn(plan, a, src0, src1, out, gn: nn.GroupNorm, gamma: torch.Tensor, b
         b.d_mod_t = plan.d_mod_t.data_ptr() + 4 * mod_cols
     if a.mod_z:
         b.d_mod_z = plan.d_mod_z.data_ptr() + 4 * mod_cols
-    st.late.append(lambda: (setattr(b, "dgamma", gget().data_ptr()), setattr(b, "dbeta", bget().data_ptr())))
     if st.ordered:
         st.main_ws_floats = max(st.main_ws_floats, plan.B * Cc * 2)
-        st.late.append(lambda: (setattr(b, "dparam_ws", st.main_ws.data_ptr()),
-                                setattr(b, "dparam_ticket", st.tickets.data_ptr() + 4)))
-    st.kernel(plan.lib.idf_adagn_silu_bwd, C.byref(b))
+
+    def args():
+        b.dgamma, b.dbeta = gget().data_ptr(), bget().data_ptr()
+        if st.ordered:
+            b.dparam_ws, b.dparam_ticket = st.main_ws.data_ptr(), st.tickets.data_ptr() + 4
+        return C.byref(b)
+    st.op("adagn_bwd", plan.lib.idf_adagn_silu_bwd, args, kernels=2)       # statistics, then apply
     st.param_grads.append((gn.weight, gget))
     st.param_grads.append((gn.bias, bget))
 
@@ -390,51 +367,59 @@ def bwd_adagn(plan, a, src0, src1, out, gn: nn.GroupNorm, gamma: torch.Tensor, b
 def bwd_attention(plan, qkv, out, d: int) -> None:
     """Softmax attention backward (reference modules.py:145-164 under autograd) on the tcgen05 kernels of
     csrc/attention_bwd.cu: P and dS are recomputed from the saved q | k | v, then dQ = dS K, dK = dS^T Q, dV = P^T dO."""
-    st = _state(plan)
+    st = plan.bwd
     dout = st.grad(out)
     gq = st.grad(qkv)
     H = qkv.H
     ws = torch.empty(int(plan.lib.idf_attn_bwd_ws_bytes(plan.B, H, H)), dtype=torch.uint8, device=plan.device)
     plan.keep.append(ws)
-    args = (qkv.t.data_ptr(), dout.t.data_ptr(), gq.t.data_ptr(), ws.data_ptr(), plan.B, H, H, d, float(d) ** -0.5)
-
-    def run():
-        _lib.check(plan.lib.idf_attn_bwd(*args, torch.cuda.current_stream(plan.device).cuda_stream))
-        _lib.count_launch(2)
-    st.ops.append(run)
+    st.op("attention_bwd", plan.lib.idf_attn_bwd, qkv.t.data_ptr(), dout.t.data_ptr(), gq.t.data_ptr(), ws.data_ptr(),
+          plan.B, H, H, d, float(d) ** -0.5, kernels=_attn_bwd_kernels(H * H, d))
     st.mark(qkv)
+
+
+def _attn_bwd_kernels(S: int, d: int) -> int:
+    """Kernels idf_attn_bwd launches: scores, then gradients on the tcgen05 path (d in {128, 256, 512} with S = H*W in
+    {64, 256}); one small-map kernel otherwise."""
+    return 2 if d in (128, 256, 512) and S in (64, 256) else 1
 
 
 # ------------------------------------------------------------------------------------------------
 # finalisation and execution
 # ------------------------------------------------------------------------------------------------
 def finalize_backward(plan) -> BwdState:
-    """Replay the tape in reverse, allocate the fp32 gradient arena and create the wgrad plans."""
-    st = _state(plan)
-    if getattr(st, "_final", False):
+    """Replay the tape in reverse, allocate the fp32 gradient arena, create the wgrad plans and resolve the op
+    arguments that point into them."""
+    st = plan.bwd
+    if st.final:
         return st
     for emit in reversed(plan.tape):
         emit()
     st.flat = torch.zeros(max(st.flat_size, 4), dtype=torch.float32, device=plan.device)
-    for d, h, get in st.wplans:
+    for d, h, get, _ in st.wplans:
         d.dw = get().data_ptr()
         _lib.check(plan.lib.idf_wgrad_plan_create(C.byref(d), C.byref(h)))
     if st.ordered:
         # the split-K partials share the side-stream scratch; their size is known once the plans exist, and the
         # pointer is part of the plan, so the multi-slab plans are created again with it
-        part = [int(plan.lib.idf_wgrad_plan_partials_floats(h)) for _, h, _ in st.wplans]
+        part = [int(plan.lib.idf_wgrad_plan_partials_floats(h)) for _, h, _, _ in st.wplans]
         st.side_ws = torch.zeros(max([st.side_ws_floats, 4] + part), dtype=torch.float32, device=plan.device)
         st.main_ws = torch.zeros(max(st.main_ws_floats, 4), dtype=torch.float32, device=plan.device)
         st.tickets = torch.zeros(2, dtype=torch.int32, device=plan.device)
-        for (d, h, _), n in zip(st.wplans, part):
+        for (d, h, _, op), n in zip(st.wplans, part):
             if n:
                 _lib.check(plan.lib.idf_wgrad_plan_destroy(h))
                 d.partials = st.side_ws.data_ptr()
                 _lib.check(plan.lib.idf_wgrad_plan_create(C.byref(d), C.byref(h)))
-    for fix in st.late:
-        fix()
+                op.kernels = 2                   # + the slab reduction
+    for op in st.ops:
+        op.args = tuple(a() if callable(a) else a for a in op.args)
+    st.ops.insert(0, Op("zero_grads", st.flat.zero_, (), kernels=0))
     _build_grad_maps(plan, st)
-    st._final = True
+    st.gathers = [Op("grad_gather", plan.lib.idf_gather_elems, (st.flat.data_ptr(), m.data_ptr(), None,
+                                                                 st.grad_flat.data_ptr(), m.numel(), 0, 1 if k else 0))
+                  for k, m in enumerate(st.grad_maps)]          # one per pass, the later passes accumulate
+    st.final = True
     return st
 
 
@@ -464,39 +449,18 @@ def _build_grad_maps(plan, st: BwdState) -> None:
 
 def run_backward(plan) -> None:
     st = finalize_backward(plan)
-    st.flat.zero_()
     # Weight and bias gradients are leaves: each needs only dY and the saved input of its layer, nothing on the
     # data-gradient chain waits for them.  They are forked onto a second stream (inside the captured graph: parallel
     # branches), where they fill the SMs that the small-batch chain kernels leave idle; joined before the gather.
-    main = torch.cuda.current_stream(plan.device)
-    if SIDE_STREAM and st.side:
-        if st.side_stream is None:
-            st.side_stream = torch.cuda.Stream(plan.device)
-        side = st.side_stream
-        side.wait_stream(main)
-        for i, op in enumerate(st.ops):
-            if i in st.side:
-                side.wait_stream(main)            # everything enqueued so far (dY of this layer) is a dependency
-                with torch.cuda.stream(side):
-                    op()
-            else:
-                op()
-        main.wait_stream(side)
-    else:
-        for op in st.ops:
-            op()
-    stream = torch.cuda.current_stream(plan.device).cuda_stream
-    for k, m in enumerate(st.grad_maps):         # parameter-shaped gradients, one gather launch per pass
-        _lib.check(plan.lib.idf_gather_elems(st.flat.data_ptr(), m.data_ptr(), None, st.grad_flat.data_ptr(),
-                                             m.numel(), 0, 1 if k else 0, stream))
-    _lib.count_launch(len(st.grad_maps))
+    run_ops(st.ops, plan.device, side=st.side_stream if SIDE_STREAM else None)
+    run_ops(st.gathers, plan.device)
 
 
 def fused_param_grads(plan) -> List[Optional[torch.Tensor]]:
     """Gradients of plan.pindex.params (None where the conv stack contributes nothing), as views of a fresh
     copy of the flat gradient buffer.  With a GradSync installed the flat buffer's all-reduce is started here,
     i.e. the backbone's gradients travel over NVLink while the encoder's backward kernels are still running."""
-    st = _state(plan)
+    st = plan.bwd
     flat = st.grad_flat.clone()
     views = plan.pindex.views(flat)
     if _grad_sync is not None:
@@ -565,7 +529,7 @@ def set_grad_sync(sync: Optional[GradSync]) -> None:
 
 def collect_param_grads(plan) -> Dict[nn.Parameter, torch.Tensor]:
     """Sum the contributions per parameter (a parameter can appear in several K segments)."""
-    st = _state(plan)
+    st = plan.bwd
     out: Dict[nn.Parameter, torch.Tensor] = {}
     for prm, get in st.param_grads:
         g = get()
@@ -584,27 +548,29 @@ SIDE_STREAM = True      # weight / bias gradient kernels on a second stream (par
 
 
 def _replay(plan, slot: str, body: Callable[[], None]) -> None:
-    """Run `body` (a fixed sequence of launches over static buffers: weight re-packing + forward plan, or
-    the backward op list incl. its few torch ops).  First call: eager (also sets kernel attributes); second
-    call: captured into a CUDA graph; afterwards a single graph replay -- the ~1000 launches of a step cost
-    one launch on the host."""
+    """Run `body` (op lists over static buffers: weight re-packing + forward plan, or the backward lists).  First
+    call: eager (also sets kernel attributes); second call: captured into a CUDA graph; afterwards a single graph
+    replay -- the ~1000 launches of a step cost one launch on the host.  The capture counts the kernels the graph
+    holds, the same declared sum as an eager run; every later replay adds that sum."""
     state = getattr(plan, slot, None)
-    if not USE_GRAPHS:
+    if not USE_GRAPHS or state is None:
         body()
-    elif state is None:
-        body()
-        setattr(plan, slot, "warm")
+        if USE_GRAPHS:
+            setattr(plan, slot, "warm")
     elif state == "warm":
         torch.cuda.synchronize(plan.device)
         g = torch.cuda.CUDAGraph()
+        n0 = _lib.launches()
         with torch.cuda.graph(g):
             body()
-        setattr(plan, slot, g)
+        setattr(plan, slot, (g, _lib.launches() - n0))
         g.replay()
-        _lib.count_launch(len(plan.ops) if slot == "_g_fwd" else len(_state(plan).ops))
     else:
-        state.replay()
-        _lib.count_launch(len(plan.ops) if slot == "_g_fwd" else len(_state(plan).ops))
+        g, n = state
+        g.replay()
+        _lib.count_launch(n)
+
+
 class _ConvStackFn(torch.autograd.Function):
     """out = plan(x, mod_t, mod_z); parameters are passed so that autograd routes their gradients."""
 
@@ -622,7 +588,7 @@ class _ConvStackFn(torch.autograd.Function):
             plan.mod_z.copy_(mod_z)
         if plan.dropout_seed is not None:
             plan.dropout_seed.fill_(int(seed))
-        _replay(plan, "_g_fwd", lambda: (plan.refresh_weights(), plan.run()))
+        _replay(plan, "_g_fwd", lambda: run_ops(plan.refresh_ops() + plan.ops, plan.device))
         ctx.plan = plan
         ctx.params = params
         ctx.has_mod = mod_t is not None
@@ -657,19 +623,22 @@ def stack_params(net) -> List[nn.Parameter]:
     return cached
 
 
+def _train_plan(net, x: torch.Tensor, kind: str, dropout_p: float, cls, **kw):
+    """The cached training plan of `net` for x's batch and device; a plan built in torch's deterministic mode is an
+    ordered plan and is cached apart."""
+    _require_cuda(x, "x")
+    ordered = torch.are_deterministic_algorithms_enabled()
+    key = (kind, x.shape[0], x.device.index, float(dropout_p), ordered)
+    plans = net._plans()
+    if key not in plans:
+        plans[key] = cls(net, x.shape[0], x.device, dropout_p=dropout_p, ordered=ordered, **kw)
+    return plans[key]
+
+
 def backbone_train_forward(net, x_t: torch.Tensor, t: torch.Tensor, a: torch.Tensor, seed: int,
                            dropout_p: float) -> torch.Tensor:
     """eps = AuxiliaryUNet(x_t, t, a) with autograd through the sm_100a kernels (reference models.py:296-326)."""
-    from .engine import BackbonePlan, _require_cuda, conditioned_blocks, modulation_weights
-    _require_cuda(x_t, "x")
-    B = x_t.shape[0]
-    plans = net._plans()
-    ordered = torch.are_deterministic_algorithms_enabled()
-    key = ("train", B, x_t.device.index, float(dropout_p), ordered)
-    if key not in plans:
-        plans[key] = BackbonePlan(net, B, x_t.device, mode="train", dropout_p=dropout_p)
-        plans[key].ordered = ordered
-    plan = plans[key]
+    plan = _train_plan(net, x_t, "train", dropout_p, BackbonePlan, mode="train")
     # modulation rows through torch autograd (tiny GEMMs): temb -> all blocks' temb_proj, a -> fc_a -> aemb_proj
     from . import linear as L                    # fp32 Linears with autograd on the library's own kernels (no cuBLAS)
     silu = torch.nn.functional.silu
@@ -689,16 +658,7 @@ def backbone_train_forward(net, x_t: torch.Tensor, t: torch.Tensor, a: torch.Ten
 
 def encoder_train_forward(net, x: torch.Tensor, seed: int, dropout_p: float):
     """(a, a_q, mu, log_var) = Encoder(x) with autograd (reference models.py:488-518)."""
-    from .engine import EncoderPlan, _require_cuda
-    _require_cuda(x, "x")
-    B = x.shape[0]
-    plans = net._plans()
-    ordered = torch.are_deterministic_algorithms_enabled()
-    key = ("train_enc", B, x.device.index, float(dropout_p), ordered)
-    if key not in plans:
-        plans[key] = EncoderPlan(net, B, x.device, training=True, dropout_p=dropout_p)
-        plans[key].ordered = ordered
-    plan = plans[key]
+    plan = _train_plan(net, x, "train_enc", dropout_p, EncoderPlan, training=True)
     params = stack_params(net)
     fmap = _ConvStackFn.apply(plan, x, None, None, seed, *params)
     from . import linear as L

@@ -314,7 +314,7 @@ def test_training_packing_and_gradient_gathers_are_exact(m1000):
             out = net(x, t, a)
             out.square().mean().backward()
         plan = next(p for k, p in net._plans().items() if k[0] == "train" and k[1] == B)
-        st = T._state(plan)
+        st = plan.bwd
         ref = T.collect_param_grads(plan)
         n = 0
         for prm, has in zip(plan.pindex.params, st.has_grad):
@@ -373,7 +373,7 @@ def test_fused_adagn_mode_matches_default(m10):
         f_eps = m.backbone(xd, td, ad)
         f_a = m.encoder(xd)[0]
         plan = next(iter(m.backbone._plans().values()))
-        assert any(mt["tag"] == "adagn_coef" for mt in plan.meta) and not any(mt["tag"] == "adagn" for mt in plan.meta)
+        assert any(op.tag == "adagn_coef" for op in plan.ops) and not any(op.tag == "adagn" for op in plan.ops)
         p1 = _proc(args, m, True)
         p1.noise_fn = lambda idx, out: out.copy_(step_noise(idx, shape))
         f_x0 = p1.sampling(2, xT=xT.to(DEV), a=ad)

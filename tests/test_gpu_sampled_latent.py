@@ -221,7 +221,7 @@ def test_mmd_reverse_path_is_unchanged():
     assert torch.equal(torch.cuda.get_rng_state(), state)
     s = p._sampler("reverse", B, with_encoder=True)
     assert s.latent_noise is None
-    assert all(mt["tag"] != "reparameterize" for pl in s.plans for mt in pl.meta)
+    assert all(op.tag != "reparameterize" for pl in s.plans for op in pl.ops)
     # the same step assembled from plans built without latent_noise
     net, dev = m.backbone, torch.device(DEV)
     x = x0.clone()
@@ -238,7 +238,7 @@ def test_mmd_reverse_path_is_unchanged():
     zp._emit_latent_mlp(net, pack, ep.a, mod_z)
     bp = BackbonePlan(net, B, dev, mode="sampler", ws=ws, x_io=x, coef=coef, step=step, mod_t_table=tables.table,
                       mod_z=mod_z, pack=pack)
-    assert s.n_launch == len(ep.ops) + len(zp.ops) + len(bp.ops)
+    assert s.n_launch == sum(op.kernels for pl in (ep, zp, bp) for op in pl.ops)
     for idx in range(1, T - 1):
         step.fill_(idx)
         for pl in (ep, zp, bp):

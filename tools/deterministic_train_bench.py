@@ -40,7 +40,6 @@ def main() -> None:
     a = ap.parse_args()
     from bench import make_args_ns
     from infodiffusion_b200 import _lib
-    from infodiffusion_b200 import train as T
     from infodiffusion_b200.models import InfoDiff
     from infodiffusion_b200.optim import ClipAdamW
     dev = torch.device("cuda", 0)
@@ -89,8 +88,8 @@ def main() -> None:
         ws = 0
         for net in (r["model"].backbone, r["model"].encoder):
             for key, plan in net._plans().items():
-                if str(key[0]).startswith("train") and hasattr(plan, "_bwd"):
-                    st = T._state(plan)
+                if str(key[0]).startswith("train") and plan.bwd is not None:
+                    st = plan.bwd
                     ws += sum(t.numel() * t.element_size() for t in (st.side_ws, st.main_ws, st.tickets) if t is not None)
         ms = sorted(r["ms"])
         result["deterministic" if det else "default"] = {
